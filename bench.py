@@ -63,7 +63,15 @@ def parse_args():
     ap.add_argument("--e2e-wide", action="store_true", help="same as --e2e-format 32")
     ap.add_argument("--call-kernel", type=int, default=13, help="include/amplisolve_b200.h as_set_call_kernel")
     ap.add_argument("--noise-kernel", type=int, default=1, help="include/amplisolve_b200.h as_set_noise_kernel")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy (float32 / float64, a "
+                         "seeded sample of the slots, at most 64 MB) for comparing two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA step's outputs: it does not apply to --impl reference")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -306,6 +314,57 @@ def bind_to_gpu_numa_node(index):
     return None
 
 
+DUMP_BYTES = 64_000_000   # the whole dump, .npy headers included
+
+
+def dump_outputs(path, out, view, calls, n_calls):
+    """Writes what the step returns to its caller as path/<name>.npy, so that two builds can be compared output for output:
+      per slot, at a sample of the slots (slots.npy): the noise model's thr, germ_val, germ_state, count and nrec, and thr_view
+      (the thresholds as the caller reads them);
+      calls_<field>.npy: the calls at those slots in the reference's row order (sample, slot, alt); n_calls.npy: all calls.
+    Every array is float32 or float64 (integers are exact in float64) and finite: a threshold the noise model leaves undefined
+    (NaN, printed "-1_-1" in the noise table) is written as -1, which no defined threshold (a ratio of counts) can be.  The
+    sample is a prefix of one seeded permutation of the slots, halved until the files, headers included, fit in 64 MB
+    (64,000,000 bytes): the same inputs give the same slots."""
+    import io
+
+    import torch
+
+    from amplisolve_b200 import CALL_DTYPE, calls_from_device
+    path.mkdir(parents=True, exist_ok=True)
+    per_slot = dict(out, thr_view=view)
+    all_calls = calls_from_device(calls, n_calls)
+    order = np.random.default_rng(WORKLOAD["seed"]).permutation(view.shape[0])
+    n = min(len(order), 1 << 18)
+    while True:
+        slots = np.sort(order[:n])
+        idx = torch.from_numpy(slots).to(view.device)
+        arrays = {"slots": slots.astype(np.float64)}
+        for name, t in per_slot.items():
+            a = t[idx].cpu().numpy()
+            if a.dtype == np.int32:   # uint32 counts held in int32 tensors
+                a = a.view(np.uint32)
+            arrays[name] = a.astype(np.float32 if a.dtype in (np.float32, np.uint8) else np.float64)
+        picked = all_calls[np.isin(all_calls["slot"], slots)]
+        for field in CALL_DTYPE.names:
+            arrays[f"calls_{field}"] = picked[field].astype(np.float64)
+        arrays["n_calls"] = np.array([len(all_calls)], np.float64)
+        arrays["thr"][np.isnan(arrays["thr"])] = -1.0
+        files = {}
+        for name, a in arrays.items():
+            buf = io.BytesIO()
+            np.save(buf, a)
+            files[name] = buf.getvalue()
+        if sum(len(b) for b in files.values()) <= DUMP_BYTES or n == 1:
+            break
+        n //= 2
+    bad = [name for name, a in arrays.items() if not np.isfinite(a).all()]
+    if bad:
+        raise RuntimeError(f"the step computed values that are not finite: {bad}")
+    for name, b in files.items():
+        (path / f"{name}.npy").write_bytes(b)
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -419,6 +478,8 @@ def run_ours(args):
     found = int(n_calls.item())
     if found > cap:
         raise RuntimeError(f"call list overflow in the benchmark: {found} > {cap}")
+    if args.dump_outputs:   # before the legs below reuse out, view and calls
+        dump_outputs(Path(args.dump_outputs) / (f"rank{rank}" if world > 1 else ""), out, view, calls, n_calls)
 
     # the only cross-GPU traffic of the job: one final gather of the compacted calls on rank 0 (outside the math path),
     # device to device: counts exchanged, exact-size NCCL sends into rank 0's buffer, one radix sort there

@@ -1,4 +1,6 @@
+import shutil
 import sys
+import tempfile
 from pathlib import Path
 
 import pytest
@@ -19,3 +21,14 @@ def ctx():
     c = Context(0)
     yield c
     c.close()
+
+
+@pytest.fixture
+def socket_path():
+    """A path for the resident service's UNIX socket.  sun_path holds at most 107 bytes, which a pytest tmp_path under a deep
+    TMPDIR or checkout exceeds, so the socket lives in a fresh directory of its own under /tmp."""
+    d = tempfile.mkdtemp(prefix="as_sock_", dir="/tmp")
+    try:
+        yield str(Path(d) / "as.sock")
+    finally:
+        shutil.rmtree(d, ignore_errors=True)

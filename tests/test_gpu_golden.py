@@ -83,14 +83,14 @@ def test_programs_end_to_end_byte_identical(name, tmp_path):
     assert len(dummy) == len(slots) and dummy[0] == f"{slots[0][0]}\t{slots[0][1]}\t.\t.\t.\t.\t.\t."
 
 
-def test_programs_through_the_resident_service(tmp_path):
+def test_programs_through_the_resident_service(tmp_path, socket_path):
     """amplisolve_b200_serve holds the CUDA context; the same programs, started with AS_SERVER, run inside it: outputs byte
     for byte those of the reference, twice in a row (every run gets and returns its own device memory), and the wait for
     CUDA is gone from the phases."""
     import os
     import re
     import signal
-    sock = str(tmp_path / "as.sock")
+    sock = socket_path
     srv = subprocess.Popen([str(BIN / "amplisolve_b200_serve"), f"socket={sock}"], cwd="/", stderr=subprocess.PIPE, text=True)
     try:
         assert "ready" in srv.stderr.readline()

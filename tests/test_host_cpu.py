@@ -190,7 +190,7 @@ def test_compute_counts_reads_the_container_and_fails_loudly_without_gpu(tmp_pat
         assert not (tmp_path / "o" / "ok.PILEUP.ASEQ").exists()
 
 
-def test_resident_service_runs_the_programs_for_its_clients(tmp_path):
+def test_resident_service_runs_the_programs_for_its_clients(tmp_path, socket_path):
     """amplisolve_b200_serve + AS_SERVER: argv, working directory, stdout / stderr and the exit status travel; the output is
     the one of a run in the program's own process; no service listening -> the program runs by itself.  (Default-error mode
     and usage errors need no GPU, so the plumbing is tested here; the GPU paths through the service in test_gpu_golden.py.)"""
@@ -202,7 +202,7 @@ def test_resident_service_runs_the_programs_for_its_clients(tmp_path):
     aseq_io.write_fasta(tmp_path, slots, list(case["ref_letters"]))
     args = [str(BIN / "AmpliSolveErrorEstimation"), "panel_design=panel.bed", "reference_genome=ref.fa", "germline_dir=not_available",
             "C_value=0.002", "coverage_cutoff=100", "default_error=0.02"]
-    sock = str(tmp_path / "as.sock")
+    sock = socket_path
     env = dict(os.environ, AS_SERVER=sock)
     # nobody listens: the program runs by itself
     r0 = subprocess.run(args + ["output_dir=alone"], cwd=tmp_path, capture_output=True, text=True, env=env)

@@ -6,7 +6,7 @@ from pathlib import Path
 import numpy as np
 import pytest
 
-from oracle import pyoracle, refrun
+from oracle import pyoracle
 from tests import golden_util as gu
 
 ROOT = Path(__file__).resolve().parent.parent
@@ -169,12 +169,18 @@ def test_live_reference_grids():
     assert np.array_equal(got.view(np.uint64), want[:40000].view(np.uint64))
 
 
-@needs_ref
-def test_screen_continued_fraction_branch_never_calls():
+def _reference_lib():
+    """The compiled reference (oracle/_ref), or None: it is built only where the original sources are at hand."""
+    path = ROOT / "oracle" / "_ref" / "libvc_ref_funcs.so"
+    return C.CDLL(str(path)) if path.exists() else None
+
+
+def test_screen_continued_fraction_branch_never_calls(grid):
     """SURVEY.md B.6(3), the screen both caller kernels rely on: whenever kf_gammaq takes the continued-fraction
     branch (m >= k and m > 1, VC:3728) the reference's Q stays below 5 -- including where the 99-step cap leaves
-    the fraction unconverged.  Checked against the compiled reference on a dense grid."""
-    L = C.CDLL(str(ROOT / "oracle" / "_ref" / "libvc_ref_funcs.so"))
+    the fraction unconverged.  Checked on a dense grid with the oracle's kf_gammaq, which equals the reference's bit for bit
+    on the continued-fraction points of the stored reference grid (tests/golden/vc_function_grid.npz) and, where the
+    compiled reference is present, on the whole dense grid."""
     rng = np.random.default_rng(7)
     ks = np.unique(np.concatenate([np.arange(1, 400), np.geomspace(400, 2_000_000, 1500).astype(np.int64),
                                    rng.integers(1, 200000, 3000)]))
@@ -184,64 +190,70 @@ def test_screen_continued_fraction_branch_never_calls():
     z = s * np.tile(ratios, len(ks))
     keep = (z >= s) & (z > 1.0)
     s, z = s[keep], z[keep]
-    out = np.empty(len(s))
-    L.ref_kf_gammaq_vec(s.ctypes.data_as(C.c_void_p), z.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p), C.c_long(len(s)))
+    kf = pyoracle.lib().aso_kf_gammaq
+    out = np.array([kf(a, b) for a, b in zip(s, z)])
+    cf = (grid["gq_z"] >= grid["gq_s"]) & (grid["gq_z"] > 1.0)
+    stored = np.array([kf(a, b) for a, b in zip(grid["gq_s"][cf], grid["gq_z"][cf])])
+    assert cf.sum() > 900 and np.array_equal(stored.view(np.uint64), grid["gq"][cf].view(np.uint64))
+    L = _reference_lib()
+    if L is not None:
+        want = np.empty(len(s))
+        L.ref_kf_gammaq_vec(s.ctypes.data_as(C.c_void_p), z.ctypes.data_as(C.c_void_p), want.ctypes.data_as(C.c_void_p),
+                            C.c_long(len(s)))
+        assert np.array_equal(out.view(np.uint64), want.view(np.uint64))
     p = 1.0 - out
     assert len(s) > 250000
     assert np.all(p > P_STAR), (s[p <= P_STAR][:5], z[p <= P_STAR][:5])
     assert p.min() > 0.49
 
 
-@needs_ref
-def test_toy_data_end_to_end_against_reference(tmp_path):
-    """BASELINE.json configs[0]: the whole of Toy_data through the compiled reference and through the oracle."""
-    from tests import aseq_io, synth
-    info = refrun.stage_toy(tmp_path)
-    noise_path, _ = refrun.run_ee_ref(tmp_path, "panel.bed", info["ref"], info["dup"], "N", "0.002", "100")
-    want = noise_path.read_text().splitlines()
-    slots = info["slots"]
-    where, pos_id, U = aseq_io.slot_index(slots)
-    P = len(slots)
-    names = sorted(p.name for p in (tmp_path / "N").glob("*.ASEQ"))
-    order = pyoracle.hash_iteration_order([f"N/{n}" for n in names])
-    normals = np.stack([aseq_io.read_aseq_dense(tmp_path / "N" / names[i], where, P)[0] for i in order])
-    rows, off = pyoracle.dense_to_rows(synth.to_oracle_layout(normals), pos_id)
-    nz = pyoracle.noise_estimate(rows, off, U, np.float32(0.002), 100)
-    case = {"slots": slots, "ref_letters": "".join(info["refmap"][k] for k in slots)}
-    lines = gu.noise_table_lines(case, nz["thr"][pos_id], nz["germ_val"][pos_id], nz["germ_present"][pos_id])
+def test_toy_data_end_to_end_against_reference():
+    """BASELINE.json configs[0]: the whole of Toy_data through the oracle, against the noise table the compiled reference
+    wrote for it (tests/golden/toy_full.npz)."""
+    case = gu.load("toy_full")
+    assert np.float32(case["c_value"]) == np.float32(0.002) and int(case["cutoff"]) == 100
+    nz = oracle_on_case(case)
+    pid = case["pos_id"]
+    lines = gu.noise_table_lines(case, nz["thr"][pid], nz["germ_val"][pid], nz["germ_present"][pid])
+    want = case["noise_table"].splitlines()
     assert lines == want
     assert len(want) == 41487
 
 
-@needs_ref
-def test_screen_critical_mean_never_calls():
+def test_screen_critical_mean_never_calls(grid):
     """The second exact screen of the caller (AS_MCRIT, scripts/critical_means.py): for k = 1..64 and every mean from the
-    table value m*(k)(1 + 1e-9) up to 3k, the compiled reference's Q stays below 5 -- on the series branch (m < k), at
+    table value m*(k)(1 + 1e-9) up to 3k, the reference's Q stays below 5 -- on the series branch (m < k), at
     m <= 1 (k = 1) and on the continued-fraction branch alike; a hair below m*(k) it reaches 5.  e = 2^-20 makes
-    m = depth * e exact."""
+    m = depth * e exact.  Checked with the oracle's Q, which equals the reference's bit for bit on the stored reference grid's
+    points with k = 1..64 (tests/golden/vc_function_grid.npz) and, where the compiled reference is present, on this grid."""
     import sys
     sys.path.insert(0, str(ROOT / "scripts"))
     from critical_means import critical_means
-    L = C.CDLL(str(ROOT / "oracle" / "_ref" / "libvc_ref_funcs.so"))
     mc = np.array(critical_means())
     ks, depths = [], []
     for k in range(1, 65):
         lo = int(np.ceil(mc[k - 1] * 2 ** 20))
-        grid = np.unique(np.concatenate([lo + np.arange(0, 200), np.geomspace(lo, 3 * k * 2 ** 20 + lo, 400).astype(np.int64)]))
-        ks.append(np.full(len(grid), k))
-        depths.append(grid)
+        grid_k = np.unique(np.concatenate([lo + np.arange(0, 200), np.geomspace(lo, 3 * k * 2 ** 20 + lo, 400).astype(np.int64)]))
+        ks.append(np.full(len(grid_k), k))
+        depths.append(grid_k)
     k = np.concatenate(ks).astype(np.int32)
     rd = np.concatenate(depths).astype(np.int32)
     err = np.full(len(k), 2.0 ** -20, np.float32)
-    q = np.empty(len(k), np.float64)
-    L.ref_poisson_q_vec(k.ctypes.data_as(C.c_void_p), rd.ctypes.data_as(C.c_void_p), err.ctypes.data_as(C.c_void_p),
-                        q.ctypes.data_as(C.c_void_p), C.c_long(len(k)))
-    assert len(k) > 30000 and (q < 5).all(), (k[q >= 5][:5], rd[q >= 5][:5])
-    # just below the critical mean the strand test passes: the table is tight, not merely safe
     kb = np.arange(1, 65, dtype=np.int32)
     rb = np.floor(mc / (1 + 1e-9) * (1 - 3e-6) * 2 ** 20).astype(np.int32)
-    qb = np.empty(64, np.float64)
     eb = np.full(64, 2.0 ** -20, np.float32)
-    L.ref_poisson_q_vec(kb.ctypes.data_as(C.c_void_p), rb.ctypes.data_as(C.c_void_p), eb.ctypes.data_as(C.c_void_p),
-                        qb.ctypes.data_as(C.c_void_p), C.c_long(64))
+    q = np.array([pyoracle.poisson_q(a, b, c) for a, b, c in zip(k, rd, err)])
+    qb = np.array([pyoracle.poisson_q(a, b, c) for a, b, c in zip(kb, rb, eb)])
+    small = (grid["q_k"] >= 1) & (grid["q_k"] <= 64)
+    stored = np.array([pyoracle.poisson_q(a, b, c) for a, b, c in zip(grid["q_k"][small], grid["q_rd"][small], grid["q_err"][small])])
+    assert small.sum() > 2000 and np.array_equal(stored.view(np.uint64), grid["q"][small].view(np.uint64))
+    L = _reference_lib()
+    if L is not None:
+        for kk, rr, ee, got in ((k, rd, err, q), (kb, rb, eb, qb)):
+            want = np.empty(len(kk), np.float64)
+            L.ref_poisson_q_vec(kk.ctypes.data_as(C.c_void_p), rr.ctypes.data_as(C.c_void_p), ee.ctypes.data_as(C.c_void_p),
+                                want.ctypes.data_as(C.c_void_p), C.c_long(len(kk)))
+            assert np.array_equal(got.view(np.uint64), want.view(np.uint64))
+    assert len(k) > 30000 and (q < 5).all(), (k[q >= 5][:5], rd[q >= 5][:5])
+    # just below the critical mean the strand test passes: the table is tight, not merely safe
     assert (qb >= 5).all()
