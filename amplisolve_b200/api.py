@@ -31,7 +31,7 @@ EXPORTS = [
     "as_noise_estimate_host16", "as_thresholds_caller_view_dev", "as_call_variants_dev", "as_call_variants_host",
     "as_call_variants_host16", "as_sort_calls_dev", "as_call_variants_sweep_dev", "as_noise_estimate_sweep_dev", "as_pack_counts", "as_noise_estimate_host_packed", "as_call_variants_host_packed", "as_poisson_test_host",
     "as_kf_gammaq_host", "as_synth_counts_dev", "as_synth_twin_links_dev", "as_hash_iteration_order", "as_fisher_test", "as_fisher_tests_host", "as_error_estimation_main",
-    "as_variant_calling_main", "as_pileup_begin", "as_pileup_add_host", "as_pileup_end_host", "as_compute_counts_main", "as_serve_main", "as_client_run", "as_process_is_resident",
+    "as_variant_calling_main", "as_pileup_begin", "as_pileup_add_host", "as_pileup_end_host", "as_pileup_end_wire", "as_pileup_set_host", "as_compute_counts_main", "as_serve_main", "as_client_run", "as_process_is_resident",
 ]
 
 
@@ -174,6 +174,8 @@ def lib():
     L.as_pileup_begin.argtypes = [vp, vp, i32, vp, i64]
     L.as_pileup_add_host.argtypes = [vp, vp, i64, vp, i64, vp, i32, i32, i32, C.c_uint32]
     L.as_pileup_end_host.argtypes = [vp, vp, vp]
+    L.as_pileup_end_wire.argtypes = [vp, vp, i64, i32, i32, i32, vp, vp, i64, C.POINTER(i64), C.POINTER(i64), vp]
+    L.as_pileup_set_host.argtypes = [vp, vp]
     for name in ("as_error_estimation_main", "as_variant_calling_main", "as_compute_counts_main"):
         if hasattr(L, name):
             getattr(L, name).argtypes = [C.c_int, C.POINTER(C.c_char_p)]
@@ -483,6 +485,36 @@ class Context:
         stats = np.zeros(2, np.uint64)
         _check(lib().as_pileup_end_host(self._h, counts.ctypes.data, stats.ctypes.data))
         return counts, (int(stats[0]), int(stats[1]))
+
+    def pileup_end_wire(self, slot_unique, mdc, fmt="packed", sample=0, wide_cap=None, counts=None):
+        """as_pileup_end_wire: ends the open pileup in the wire form of one sample of the programs' host tensor.  slot_unique
+        [P] = position (0..U-1) of every panel slot; a slot whose depth is below mdc is absent.  counts: uint32 [2][U][4]
+        put in place of the pileup's counts first (as_pileup_set_host; a pileup over positions 0..U-1 of one contig is opened
+        for them).  fmt "packed" -> wire uint32 [2][P], "16" -> uint16 [2][P][4].  Returns (wire, wide records sorted by slot,
+        present slots, (reads used, bases counted)).  More than wide_cap (default P) escaped records raise AmpliSolveError
+        with .code -5 and .n_wide = the true count; the pileup then stays open."""
+        slot_unique = np.ascontiguousarray(slot_unique, np.int32)
+        P = len(slot_unique)
+        if counts is not None:
+            counts = _np(counts, np.uint32)
+            U = counts.shape[1]
+            first = np.array([0, U], np.int64)
+            pos = np.arange(U, dtype=np.int32)
+            _check(lib().as_pileup_begin(self._h, first.ctypes.data, 1, pos.ctypes.data, U))
+            _check(lib().as_pileup_set_host(self._h, counts.ctypes.data))
+        f = {"packed": 1, "16": 2}[fmt]
+        wire = np.empty((2, P), np.uint32) if f == 1 else np.empty((2, P, 4), np.uint16)
+        cap = P if wide_cap is None else int(wide_cap)
+        wide = np.zeros(max(cap, 1), dtype=WIDE_DTYPE)
+        n, rows = C.c_int64(0), C.c_int64(0)
+        stats = np.zeros(2, np.uint64)
+        rc = lib().as_pileup_end_wire(self._h, slot_unique.ctypes.data, P, int(mdc), f, int(sample), wire.ctypes.data, wide.ctypes.data, cap,
+                                      C.byref(n), C.byref(rows), stats.ctypes.data)
+        if rc != 0:
+            err = AmpliSolveError(f"amplisolve_b200 error {rc}: {lib().as_last_error().decode(errors='replace')}")
+            err.code, err.n_wide = rc, int(n.value)
+            raise err
+        return wire, wide[:n.value], int(rows.value), (int(stats[0]), int(stats[1]))
 
     def synth_counts_dev(self, n_samples, P, *, seed, mean_depth, somatic_rate=0.0, sample_offset=0, slot_offset=0,
                          depth_sigma=0.5, germline_rate=1e-3, vaf=(0.01, 0.2), absent_rate=0.0, want_ref=True,

@@ -21,7 +21,7 @@ BIN = PKG / "bin"
 OBJ = PKG / "lib" / "obj"
 CU_SOURCES = ["as_kernels.cu", "as_noise_pattern.cu", "as_call_deferred.cu", "as_capi.cu", "as_sort.cu", "as_fisher.cu", "as_pileup.cu"]
 CXX_SOURCES = ["as_host.cpp", "as_bam.cpp", "as_serve.cpp"]  # as_bam.cpp inflates BGZF blocks with zlib (-lz)
-HEADERS = ["as_device.cuh", "as_noise.cuh", "as_pipeline.cuh", "as_call.cuh", "as_kernels.h", "as_wire.h",
+HEADERS = ["as_device.cuh", "as_noise.cuh", "as_pipeline.cuh", "as_call.cuh", "as_kernels.h", "as_wire.h", "as_bam.h",
            "../../include/amplisolve_b200.h"]
 # -cudart shared: the CUDA runtime is NOT linked into the product library (a static runtime would carry every runtime entry
 # point, used or not, into libamplisolve_b200.so); libcudart.so.12 comes from the toolkit (rpath) or from the process

@@ -9,7 +9,8 @@
 // are inflated on `threads` host threads (zlib, CRC checked), the record boundaries are indexed, and the records go to
 // the GPU (as_pileup_add_host), which walks the CIGARs and counts.  Rows are written in the order of the position file,
 // one row per line of it (a position listed twice -- overlapping amplicons -- gets two identical rows, which is what the
-// noise model's twin slots expect), and a position with fewer than mdc counted bases is left out.
+// noise model's twin slots expect), and a position with fewer than mdc counted bases is left out.  The reader (asbam::Reader,
+// as_bam.h) is shared with the two programs, which pile up a directory of BAM files themselves (as_host.cpp).
 #include <fcntl.h>
 #include <sys/mman.h>
 #include <sys/stat.h>
@@ -31,6 +32,7 @@
 #include <vector>
 
 #include "amplisolve_b200.h"
+#include "as_bam.h"
 
 namespace {
 
@@ -184,6 +186,7 @@ class Worker {
     std::thread th_;
 };
 
+
 double now_s() {
     timespec ts;
     clock_gettime(CLOCK_MONOTONIC, &ts);
@@ -191,6 +194,165 @@ double now_s() {
 }
 
 }  // namespace
+
+namespace asbam {
+
+struct Reader::Impl {
+    RawBuf bufs[2];  // carried bytes of the previous piece + the inflated blocks of this one (reused by every BAM)
+    std::vector<int64_t> offs[2];
+    Worker gpu;  // runs as_pileup_add_host of a piece while the next piece inflates
+};
+
+Reader::Reader() : impl_(new Impl()) {}
+Reader::~Reader() = default;
+
+int Reader::pileup(const std::string& bam, const std::map<std::string, int32_t>& contig_id, int threads, int mbq, int mrq,
+                   const std::function<as_ctx*()>& begin, uint64_t* n_records_out) {
+    RawBuf* bufs = impl_->bufs;
+    std::vector<int64_t>* offs = impl_->offs;
+    Worker& gpu = impl_->gpu;
+    const bool timing = getenv("AS_TIMING") != nullptr;
+    // ---- BAM container
+    Mapped f;
+    if (!f.open(bam)) { printf("Error from computeCounts: Cannot open file: %s\n", bam.c_str()); return 1; }
+    Block probe;
+    if (f.n < 28 || bgzf_block(f.p, f.n, 0, probe) == 0) { printf("Error from computeCounts: %s is not a BGZF (BAM) file\n", bam.c_str()); return 1; }
+
+    // Two piece buffers: while the GPU takes the records of one piece (upload + kernel, on a helper thread), the host
+    // threads inflate the next piece into the other buffer.
+    const size_t piece_budget = (size_t)(getenv("AS_BAM_PIECE_MB") ? atol(getenv("AS_BAM_PIECE_MB")) : 64) << 20;
+    std::string job_err;
+    int cur = 0;
+    std::vector<int32_t> ref_contig;
+    size_t file_off = 0, carried = 0;
+    bool header_done = false;
+    as_ctx* ctx = nullptr;  // set by begin(): the pileup has started
+    uint64_t n_records = 0, bytes_inflated = 0;
+    double t_inflate = 0, t_gpu = 0;
+    int32_t n_ref = 0;
+    // declared last, destroyed first: no job outlives what it reads on an early return
+    struct Drain { Worker& w; ~Drain() { w.wait(); } } drain{gpu};
+
+    while (file_off < f.n || carried > 0) {
+        // blocks of this piece
+        std::vector<Block> blocks;
+        size_t out_bytes = 0;
+        while (file_off < f.n && (blocks.empty() || out_bytes < piece_budget)) {
+            Block b;
+            const size_t len = bgzf_block(f.p, f.n, file_off, b);
+            if (len == 0) { printf("Error from computeCounts: corrupt BGZF block at byte %zu of %s\n", file_off, bam.c_str()); return 1; }
+            b.out_off = out_bytes;
+            out_bytes += b.isize;
+            blocks.push_back(b);
+            file_off += len;
+        }
+        if (blocks.empty() && carried > 0) { printf("Error from computeCounts: %s ends inside a record\n", bam.c_str()); return 1; }
+        RawBuf& buf = bufs[cur];  // no job reads it: the one that did was waited for before the carry-over
+        std::vector<int64_t>& rec_off = offs[cur];
+        if (!buf.ensure(carried, carried + out_bytes + 8)) { printf("Error from computeCounts: out of memory\n"); return 1; }
+        const double ti = now_s();
+        {
+            std::atomic<size_t> next{0};
+            std::atomic<bool> bad{false};
+            const int nt = (int)std::min<size_t>((size_t)threads, std::max<size_t>(1, blocks.size()));
+            std::vector<std::thread> th;
+            for (int t = 0; t < nt; ++t)
+                th.emplace_back([&]() {
+                    for (size_t i; (i = next.fetch_add(1)) < blocks.size();)
+                        if (!inflate_block(f.p, blocks[i], buf.data() + carried + blocks[i].out_off)) bad = true;
+                });
+            for (auto& t : th) t.join();
+            if (bad) { printf("Error from computeCounts: a BGZF block of %s does not inflate (or fails its CRC)\n", bam.c_str()); return 1; }
+        }
+        t_inflate += now_s() - ti;
+        bytes_inflated += out_bytes;
+        const size_t have = carried + out_bytes;
+        size_t off = 0;
+        if (!header_done) {
+            // magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
+            bool complete = false;
+            do {
+                if (have < 12) break;
+                if (memcmp(buf.data(), "BAM\1", 4) != 0) { printf("Error from computeCounts: %s is not a BAM file\n", bam.c_str()); return 1; }
+                size_t o = 8 + (size_t)le32(buf.data() + 4);
+                if (o + 4 > have) break;
+                n_ref = (int32_t)le32(buf.data() + o);
+                o += 4;
+                std::vector<int32_t> map;
+                bool ok = true;
+                for (int32_t r = 0; r < n_ref; ++r) {
+                    if (o + 4 > have) { ok = false; break; }
+                    const size_t l_name = le32(buf.data() + o);
+                    if (o + 4 + l_name + 4 > have) { ok = false; break; }
+                    std::string name((const char*)buf.data() + o + 4, l_name ? l_name - 1 : 0);
+                    auto it = contig_id.find(name);
+                    map.push_back(it == contig_id.end() ? -1 : it->second);
+                    o += 4 + l_name + 4;
+                }
+                if (!ok) break;
+                ref_contig = std::move(map);
+                off = o;
+                complete = true;
+            } while (false);
+            if (!complete) {
+                if (file_off >= f.n) { printf("Error from computeCounts: %s ends inside its header\n", bam.c_str()); return 1; }
+                carried = have;  // keep everything and read more blocks
+                continue;
+            }
+            header_done = true;
+            if (n_ref < 1) ref_contig.assign(1, -1), n_ref = 1;
+        }
+        // records of this piece
+        rec_off.clear();
+        const size_t first = off;
+        while (off + 4 <= have) {
+            const size_t bs = le32(buf.data() + off);
+            if (off + 4 + bs > have) break;
+            if (bs >= 32) rec_off.push_back((int64_t)(off - first));
+            off += 4 + bs;
+        }
+        n_records += rec_off.size();
+        if (!ctx && !(ctx = begin())) return 1;
+        // the other buffer's job (the previous piece) ran while this piece inflated; it must be over before the
+        // carried bytes are copied into that buffer
+        const double tg = now_s();
+        if (gpu.wait() != AS_OK) { printf("Error from computeCounts: %s\n", job_err.c_str()); return 1; }
+        t_gpu += now_s() - tg;
+        carried = have - off;
+        if (file_off >= f.n && carried > 0) { printf("Error from computeCounts: %s ends inside a record\n", bam.c_str()); return 1; }
+        if (carried > 0) {
+            if (!bufs[cur ^ 1].ensure(0, carried)) { printf("Error from computeCounts: out of memory\n"); return 1; }
+            memcpy(bufs[cur ^ 1].data(), buf.data() + off, carried);
+        }
+        if (!rec_off.empty()) {
+            const uint8_t* rec = buf.data() + first;
+            const int64_t n_bytes = (int64_t)(off - first), n_rec = (int64_t)rec_off.size();
+            const int64_t* ro = rec_off.data();
+            gpu.submit([&, rec, n_bytes, ro, n_rec]() {
+                const int rc = as_pileup_add_host(ctx, rec, n_bytes, ro, n_rec, ref_contig.data(), n_ref, mbq, mrq, 0x704u);
+                if (rc != AS_OK) job_err = as_last_error();
+                return rc;
+            });
+        }
+        cur ^= 1;
+    }
+    {
+        const double tg = now_s();
+        if (gpu.wait() != AS_OK) { printf("Error from computeCounts: %s\n", job_err.c_str()); return 1; }
+        t_gpu += now_s() - tg;
+    }
+    if (!header_done) { printf("Error from computeCounts: %s holds no BAM header\n", bam.c_str()); return 1; }
+    // a BAM without records: every count is zero, nothing to report -- still needs no CPU path: the GPU zeroes
+    if (!ctx && !(ctx = begin())) return 1;
+    if (timing) {
+        fprintf(stderr, "AS_TIMING inflate_busy %.6f (%.3g B/s)\n", t_inflate, t_inflate > 0 ? bytes_inflated / t_inflate : 0.0);
+        fprintf(stderr, "AS_TIMING pileup_gpu_wait %.6f\n", t_gpu);
+    }
+    if (n_records_out) *n_records_out = n_records;
+    return 0;
+}
+
+}  // namespace asbam
 
 extern "C" int as_compute_counts_main(int argc, char** argv) {
     std::string vcf, bam, out = ".";
@@ -286,160 +448,20 @@ extern "C" int as_compute_counts_main(int argc, char** argv) {
     lap("positions");
 
     const std::string bam_list = bam;
-    RawBuf bufs[2];                 // carried bytes of the previous piece + the inflated blocks of this one (reused by every BAM)
-    std::vector<int64_t> offs[2];
-    Worker gpu;  // runs as_pileup_add_host of a piece while the next piece inflates
+    asbam::Reader reader;
     auto one_bam = [&](const std::string& bam) -> int {
-        // ---- BAM container
-        Mapped f;
-        if (!f.open(bam)) { printf("Error from computeCounts: Cannot open file: %s\n", bam.c_str()); return 1; }
-        Block probe;
-        if (f.n < 28 || bgzf_block(f.p, f.n, 0, probe) == 0) { printf("Error from computeCounts: %s is not a BGZF (BAM) file\n", bam.c_str()); return 1; }
-
-        // Two piece buffers: while the GPU takes the records of one piece (upload + kernel, on a helper thread), the host
-        // threads inflate the next piece into the other buffer.
-        const size_t piece_budget = (size_t)(getenv("AS_BAM_PIECE_MB") ? atol(getenv("AS_BAM_PIECE_MB")) : 64) << 20;
-        std::string job_err;
-        int cur = 0;
-        std::vector<int32_t> ref_contig;
-        size_t file_off = 0, carried = 0;
-        bool header_done = false, started = false;
-        uint64_t n_records = 0, bytes_inflated = 0;
-        double t_inflate = 0, t_gpu = 0;
-        int32_t n_ref = 0;
-        // declared last, destroyed first: no job outlives what it reads on an early return
-        struct Drain { Worker& w; ~Drain() { w.wait(); } } drain{gpu};
-
-        while (file_off < f.n || carried > 0) {
-            // blocks of this piece
-            std::vector<Block> blocks;
-            size_t out_bytes = 0;
-            while (file_off < f.n && (blocks.empty() || out_bytes < piece_budget)) {
-                Block b;
-                const size_t len = bgzf_block(f.p, f.n, file_off, b);
-                if (len == 0) { printf("Error from computeCounts: corrupt BGZF block at byte %zu of %s\n", file_off, bam.c_str()); return 1; }
-                b.out_off = out_bytes;
-                out_bytes += b.isize;
-                blocks.push_back(b);
-                file_off += len;
-            }
-            if (blocks.empty() && carried > 0) { printf("Error from computeCounts: %s ends inside a record\n", bam.c_str()); return 1; }
-            RawBuf& buf = bufs[cur];  // no job reads it: the one that did was waited for before the carry-over
-            std::vector<int64_t>& rec_off = offs[cur];
-            if (!buf.ensure(carried, carried + out_bytes + 8)) { printf("Error from computeCounts: out of memory\n"); return 1; }
-            const double ti = now_s();
-            {
-                std::atomic<size_t> next{0};
-                std::atomic<bool> bad{false};
-                const int nt = (int)std::min<size_t>((size_t)threads, std::max<size_t>(1, blocks.size()));
-                std::vector<std::thread> th;
-                for (int t = 0; t < nt; ++t)
-                    th.emplace_back([&]() {
-                        for (size_t i; (i = next.fetch_add(1)) < blocks.size();)
-                            if (!inflate_block(f.p, blocks[i], buf.data() + carried + blocks[i].out_off)) bad = true;
-                    });
-                for (auto& t : th) t.join();
-                if (bad) { printf("Error from computeCounts: a BGZF block of %s does not inflate (or fails its CRC)\n", bam.c_str()); return 1; }
-            }
-            t_inflate += now_s() - ti;
-            bytes_inflated += out_bytes;
-            const size_t have = carried + out_bytes;
-            size_t off = 0;
-            if (!header_done) {
-                // magic, l_text, text, n_ref, (l_name, name, l_ref) * n_ref
-                bool complete = false;
-                do {
-                    if (have < 12) break;
-                    if (memcmp(buf.data(), "BAM\1", 4) != 0) { printf("Error from computeCounts: %s is not a BAM file\n", bam.c_str()); return 1; }
-                    size_t o = 8 + (size_t)le32(buf.data() + 4);
-                    if (o + 4 > have) break;
-                    n_ref = (int32_t)le32(buf.data() + o);
-                    o += 4;
-                    std::vector<int32_t> map;
-                    bool ok = true;
-                    for (int32_t r = 0; r < n_ref; ++r) {
-                        if (o + 4 > have) { ok = false; break; }
-                        const size_t l_name = le32(buf.data() + o);
-                        if (o + 4 + l_name + 4 > have) { ok = false; break; }
-                        std::string name((const char*)buf.data() + o + 4, l_name ? l_name - 1 : 0);
-                        auto it = contig_id.find(name);
-                        map.push_back(it == contig_id.end() ? -1 : it->second);
-                        o += 4 + l_name + 4;
-                    }
-                    if (!ok) break;
-                    ref_contig = std::move(map);
-                    off = o;
-                    complete = true;
-                } while (false);
-                if (!complete) {
-                    if (file_off >= f.n) { printf("Error from computeCounts: %s ends inside its header\n", bam.c_str()); return 1; }
-                    carried = have;  // keep everything and read more blocks
-                    continue;
-                }
-                header_done = true;
-                if (n_ref < 1) ref_contig.assign(1, -1), n_ref = 1;
-            }
-            // records of this piece
-            rec_off.clear();
-            const size_t first = off;
-            while (off + 4 <= have) {
-                const size_t bs = le32(buf.data() + off);
-                if (off + 4 + bs > have) break;
-                if (bs >= 32) rec_off.push_back((int64_t)(off - first));
-                off += 4 + bs;
-            }
-            n_records += rec_off.size();
-            if (!started) {
-                if (starter.joinable()) starter.join();
-                if (ctx_rc != AS_OK || !ctx) { printf("Error from computeCounts: %s\n", ctx_err.c_str()); return 1; }
-                lap("cuda_context_wait");
-                if (as_pileup_begin(ctx, contig_first.data(), n_contig, slot_pos.data(), P) != AS_OK) {
-                    printf("Error from computeCounts: %s\n", as_last_error());
-                    return 1;
-                }
-                started = true;
-            }
-            // the other buffer's job (the previous piece) ran while this piece inflated; it must be over before the
-            // carried bytes are copied into that buffer
-            const double tg = now_s();
-            if (gpu.wait() != AS_OK) { printf("Error from computeCounts: %s\n", job_err.c_str()); return 1; }
-            t_gpu += now_s() - tg;
-            carried = have - off;
-            if (file_off >= f.n && carried > 0) { printf("Error from computeCounts: %s ends inside a record\n", bam.c_str()); return 1; }
-            if (carried > 0) {
-                if (!bufs[cur ^ 1].ensure(0, carried)) { printf("Error from computeCounts: out of memory\n"); return 1; }
-                memcpy(bufs[cur ^ 1].data(), buf.data() + off, carried);
-            }
-            if (!rec_off.empty()) {
-                const uint8_t* rec = buf.data() + first;
-                const int64_t n_bytes = (int64_t)(off - first), n_rec = (int64_t)rec_off.size();
-                const int64_t* ro = rec_off.data();
-                gpu.submit([&, rec, n_bytes, ro, n_rec]() {
-                    const int rc = as_pileup_add_host(ctx, rec, n_bytes, ro, n_rec, ref_contig.data(), n_ref, mbq, mrq, 0x704u);
-                    if (rc != AS_OK) job_err = as_last_error();
-                    return rc;
-                });
-            }
-            cur ^= 1;
-        }
-        {
-            const double tg = now_s();
-            if (gpu.wait() != AS_OK) { printf("Error from computeCounts: %s\n", job_err.c_str()); return 1; }
-            t_gpu += now_s() - tg;
-        }
-        if (!header_done) { printf("Error from computeCounts: %s holds no BAM header\n", bam.c_str()); return 1; }
-        if (!started) {  // a BAM without records: every count is zero, nothing to report -- still needs no CPU path: the GPU zeroes
+        uint64_t n_records = 0;
+        const int rrc = reader.pileup(bam, contig_id, threads, mbq, mrq, [&]() -> as_ctx* {
             if (starter.joinable()) starter.join();
-            if (ctx_rc != AS_OK || !ctx) { printf("Error from computeCounts: %s\n", ctx_err.c_str()); return 1; }
+            if (ctx_rc != AS_OK || !ctx) { printf("Error from computeCounts: %s\n", ctx_err.c_str()); return nullptr; }
+            lap("cuda_context_wait");
             if (as_pileup_begin(ctx, contig_first.data(), n_contig, slot_pos.data(), P) != AS_OK) {
                 printf("Error from computeCounts: %s\n", as_last_error());
-                return 1;
+                return nullptr;
             }
-        }
-        if (timing) {
-            fprintf(stderr, "AS_TIMING inflate_busy %.6f (%.3g B/s)\n", t_inflate, t_inflate > 0 ? bytes_inflated / t_inflate : 0.0);
-            fprintf(stderr, "AS_TIMING pileup_gpu_wait %.6f\n", t_gpu);
-        }
+            return ctx;
+        }, &n_records);
+        if (rrc != 0) return rrc;
         std::vector<uint32_t> counts((size_t)P * 8);
         uint64_t stats[2] = {0, 0};
         if (as_pileup_end_host(ctx, counts.data(), stats) != AS_OK) { printf("Error from computeCounts: %s\n", as_last_error()); return 1; }

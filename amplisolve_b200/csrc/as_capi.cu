@@ -106,6 +106,7 @@ struct as_ctx {
     int64_t lg_n = 0;
     PinnedGrow h_links, h_small;                                              // _host pipelines, host side
     DevBuf pile_first, pile_pos, pile_counts, pile_rec, pile_off, pile_ref, pile_stats;  // as_pileup_*
+    DevBuf pile_slots, pile_wire, pile_wide;                                            // as_pileup_end_wire
     int64_t pile_P = -1;
     int32_t pile_contigs = 0;
     double pile_kernel_ms = 0, pile_h2d_ms = 0;  // AS_TIMING only
@@ -216,7 +217,7 @@ void as_destroy(as_ctx* c) {
     c->heads.release(); c->nheads.release(); c->misc.release(); c->calls.release(); c->sortbuf.release();
     c->h_links.release(); c->h_small.release(); c->lgtab.release(); c->defer.release();
     c->pile_first.release(); c->pile_pos.release(); c->pile_counts.release(); c->pile_rec.release(); c->pile_off.release();
-    c->pile_ref.release(); c->pile_stats.release();
+    c->pile_ref.release(); c->pile_stats.release(); c->pile_slots.release(); c->pile_wire.release(); c->pile_wide.release();
     for (int i = 0; i < 2; ++i) {
         c->tile[i].release(); c->tile16[i].release(); c->wide[i].release(); c->out[i].release(); c->aux[i].release();
         if (c->ev_up[i]) cudaEventDestroy(c->ev_up[i]);
@@ -1148,6 +1149,74 @@ int as_pileup_end_host(as_ctx* c, uint32_t* counts, uint64_t* stats_out) {
         fprintf(stderr, "AS_TIMING capi.pileup.h2d %.6f\nAS_TIMING capi.pileup.kernel %.6f\n", 1e-3 * c->pile_h2d_ms, 1e-3 * c->pile_kernel_ms);
         c->pile_h2d_ms = c->pile_kernel_ms = 0;
     }
+    c->pile_P = -1;
+    return AS_OK;
+}
+
+int as_pileup_set_host(as_ctx* c, const uint32_t* counts) {
+    if (!c || !counts) return fail(AS_EINVAL, "bad argument");
+    if (c->subs.size() > 1) c = c->subs[0];
+    if (c->pile_P < 1) return fail(AS_EINVAL, "as_pileup_begin has not been called");
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->exec_stream;
+    CU(cudaMemcpyAsync(c->pile_counts.p, counts, sizeof(uint32_t) * 8 * (size_t)c->pile_P, cudaMemcpyHostToDevice, st));
+    CU(cudaStreamSynchronize(st));
+    return AS_OK;
+}
+
+// The pileup of one sample -> its slice of a host wire tensor (pileup_encode_kernel), the escaped records sorted by slot.
+int as_pileup_end_wire(as_ctx* c, const int32_t* slot_unique, int64_t P, int32_t mdc, int32_t fmt, int32_t sample, void* wire,
+                       as_wide_record* wide, int64_t wide_cap, int64_t* n_wide, int64_t* rows_out, uint64_t* stats_out) {
+    if (!c || !slot_unique || !wire || !n_wide || P < 1 || P > 0x7fffffffll || (fmt != 1 && fmt != 2) || wide_cap < 0 ||
+        (wide_cap > 0 && !wide))
+        return fail(AS_EINVAL, "bad argument");
+    if (c->subs.size() > 1) c = c->subs[0];
+    const int64_t U = c->pile_P;
+    if (U < 1) return fail(AS_EINVAL, "as_pileup_begin has not been called");
+    for (int64_t s = 0; s < P; ++s)
+        if (slot_unique[s] < 0 || slot_unique[s] >= U)
+            return fail(AS_EINVAL, "slot_unique[%lld] = %d is not a position of the pileup (0..%lld)", (long long)s, slot_unique[s], (long long)U - 1);
+    CU(cudaSetDevice(c->device));
+    const size_t wire_bytes = (size_t)P * 2 * (fmt == 1 ? 4 : 8);
+    const int64_t keep = std::min<int64_t>(wide_cap, P);  // no more than P records can escape
+    CU(c->pile_slots.need(sizeof(int32_t) * (size_t)P));
+    CU(c->pile_wire.need(wire_bytes));
+    CU(c->pile_wide.need(sizeof(as_wide_record) * (size_t)std::max<int64_t>(1, keep)));
+    CU(c->misc.need(32));
+    cudaStream_t st = c->exec_stream;
+    const bool timing = getenv("AS_TIMING") != nullptr;
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    if (timing) for (auto& e : ev) CU(cudaEventCreate(&e));
+    CU(cudaMemcpyAsync(c->pile_slots.p, slot_unique, sizeof(int32_t) * (size_t)P, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(c->misc.p, 0, 16, st));
+    if (timing) CU(cudaEventRecord(ev[0], st));
+    CU(as_launch_pileup_encode(fmt, (const uint32_t*)c->pile_counts.p, U, (const int32_t*)c->pile_slots.p, P, mdc, sample, c->pile_wire.p,
+                               (as_wide_record*)c->pile_wide.p, keep, (unsigned long long*)c->misc.p, st));
+    c->launches += 1;
+    if (timing) CU(cudaEventRecord(ev[1], st));
+    unsigned long long h[4] = {0ull, 0ull, 0ull, 0ull};  // escaped, present; reads used, bases counted
+    CU(cudaMemcpyAsync(wire, c->pile_wire.p, wire_bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h, c->misc.p, 16, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h + 2, c->pile_stats.p, 16, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    const int64_t n = (int64_t)h[0];
+    if (n > 0 && n <= keep) {
+        CU(cudaMemcpyAsync(wide, c->pile_wide.p, sizeof(as_wide_record) * (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        std::sort(wide, wide + n, [](const as_wide_record& x, const as_wide_record& y) { return x.slot < y.slot; });
+    }
+    if (timing) {
+        float ms = 0;
+        CU(cudaEventElapsedTime(&ms, ev[0], ev[1]));
+        for (auto& e : ev) cudaEventDestroy(e);
+        fprintf(stderr, "AS_TIMING capi.pileup.h2d %.6f\nAS_TIMING capi.pileup.kernel %.6f\nAS_TIMING capi.pileup.encode %.6f\n",
+                1e-3 * c->pile_h2d_ms, 1e-3 * c->pile_kernel_ms, 1e-3 * ms);
+        c->pile_h2d_ms = c->pile_kernel_ms = 0;
+    }
+    *n_wide = n;
+    if (rows_out) *rows_out = (int64_t)h[1];
+    if (stats_out) { stats_out[0] = h[2]; stats_out[1] = h[3]; }
+    if (n > wide_cap) return fail(AS_EOVERFLOW, "%lld records escape the wire format, capacity %lld", (long long)n, (long long)wide_cap);
     c->pile_P = -1;
     return AS_OK;
 }

@@ -38,6 +38,7 @@
 #endif
 
 #include "../../include/amplisolve_b200.h"
+#include "as_bam.h"
 #include "as_factorials.h"
 #include "as_wire.h"
 
@@ -241,15 +242,49 @@ bool annotate_reference(const std::string& fasta, Panel& panel, std::string& err
 // ---------------------------------------------------------------------------------------------------
 struct CountFile { std::string path, sample; };
 
-bool list_count_files(const std::string& dir, std::vector<CountFile>& files, std::vector<std::string>& listed) {
+inline bool ends_with(const std::string& n, const char* tail) {
+    const size_t k = strlen(tail);
+    return n.size() >= k && n.compare(n.size() - k, k, tail) == 0;
+}
+
+// A count directory is read as BAM input when it holds *.bam files and no *.ASEQ file (names starting with '.' do not
+// count, as for `ls <dir>/*.ASEQ`); a directory with an ASEQ file is read as ASEQ text whatever else it holds.
+bool bam_input_dir(const std::string& dir) {
     DIR* d = opendir(dir.c_str());
     if (!d) return false;
-    std::vector<std::string> names;
+    bool aseq = false, bam = false;
+    while (dirent* en = readdir(d)) {
+        const std::string n = en->d_name;
+        if (n[0] == '.') continue;
+        aseq = aseq || ends_with(n, ".ASEQ");
+        bam = bam || ends_with(n, ".bam");
+    }
+    closedir(d);
+    return bam && !aseq;
+}
+
+// *bam_mode (when not NULL): the directory holds BAM input (bam_input_dir).  A BAM file <name>.bam takes the place its computeCounts output
+// <name>.PILEUP.ASEQ would take: the same sort and the same hash keys give the same sample order and names, only the path
+// (and the list file) names the BAM.
+bool list_count_files(const std::string& dir, std::vector<CountFile>& files, std::vector<std::string>& listed, bool* bam_mode = nullptr) {
+    DIR* d = opendir(dir.c_str());
+    if (!d) return false;
+    std::vector<std::string> names, bams;
     while (dirent* en = readdir(d)) {
         const std::string n = en->d_name;
         if (n.size() >= 5 && n.compare(n.size() - 5, 5, ".ASEQ") == 0 && n[0] != '.') names.push_back(n);
+        if (ends_with(n, ".bam") && n[0] != '.') bams.push_back(n);
     }
     closedir(d);
+    const bool bam = bam_mode && names.empty() && !bams.empty();
+    if (bam_mode) *bam_mode = bam;
+    std::map<std::string, std::string> bam_of;  // "<dir>/<name>.PILEUP.ASEQ" -> "<dir>/<name>.bam"
+    if (bam) {
+        for (const std::string& b : bams) {
+            names.push_back(b.substr(0, b.size() - 4) + ".PILEUP.ASEQ");
+            bam_of[dir + "/" + names.back()] = dir + "/" + b;
+        }
+    }
     setlocale(LC_COLLATE, "");
     std::sort(names.begin(), names.end(), [](const std::string& a, const std::string& b) {
         const int c = strcoll(a.c_str(), b.c_str());
@@ -258,12 +293,12 @@ bool list_count_files(const std::string& dir, std::vector<CountFile>& files, std
     std::unordered_map<std::string, std::string> hash;  // exactly the container of EE:832 / VC:615
     for (const std::string& n : names) {
         const std::string path = dir + "/" + n;
-        listed.push_back(path);
+        listed.push_back(bam ? bam_of[path] : path);
         // sample name = listed path minus "<dir>/" and the 12 characters of ".PILEUP.ASEQ" (EE:831)
         std::string sample = n.size() > 12 ? n.substr(0, n.size() - 12) : std::string();
         hash.insert(std::make_pair(path, sample));
     }
-    for (auto it = hash.begin(); it != hash.end(); ++it) files.push_back(CountFile{it->first, it->second});
+    for (auto it = hash.begin(); it != hash.end(); ++it) files.push_back(CountFile{bam ? bam_of[it->first] : it->first, it->second});
     return true;
 }
 
@@ -1041,23 +1076,172 @@ int64_t add_spill_slots(const Panel& panel, HostCounts& hc, const std::vector<As
     return P2;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// BAM input: a count directory of *.bam files is piled up on the GPU (as_bam.h reads the files, as_pileup.cu counts) and
+// every sample ends straight in the wire tensor (as_pileup_end_wire), with what computeCounts mbq= mrq= mdc= for a position
+// file listing the panel's slots in order, followed by the ASEQ loader, would have given.
+// ---------------------------------------------------------------------------------------------------
+int env_int(const char* name, int fallback) {
+    const char* v = getenv(name);
+    return v && *v ? atoi(v) : fallback;
+}
+
+struct BamInput {
+    int mbq = env_int("AS_BAM_MBQ", 20), mrq = env_int("AS_BAM_MRQ", 20), mdc = env_int("AS_BAM_MDC", 20);  // computeCounts' defaults
+    std::map<std::string, int32_t> contig_id;  // panel chromosome -> pileup contig (= panel chromosome id)
+    std::vector<int64_t> contig_first;         // the pileup's positions: sorted, unique, 0-based per contig
+    std::vector<int32_t> upos;
+    std::vector<int32_t> slot_unique;          // panel slot -> its position in upos (0 for the slots below)
+    std::vector<int32_t> no_position;          // slots at a position below 1: computeCounts skips such lines, they stay absent
+    asbam::Reader reader;
+
+    void setup(const Panel& panel) {
+        const int64_t P = panel.size();
+        const int32_t n_contig = (int32_t)panel.chroms.size();
+        std::vector<std::vector<int32_t>> per((size_t)n_contig);
+        for (int64_t s = 0; s < P; ++s)
+            if (panel.slot_chrom[s] >= 0 && panel.slot_pos[s] >= 1) per[(size_t)panel.slot_chrom[s]].push_back(panel.slot_pos[s] - 1);
+        contig_first.assign((size_t)n_contig + 1, 0);
+        for (int32_t c = 0; c < n_contig; ++c) {
+            contig_id[panel.chroms[(size_t)c]] = c;
+            auto& v = per[(size_t)c];
+            std::sort(v.begin(), v.end());
+            v.erase(std::unique(v.begin(), v.end()), v.end());
+            contig_first[(size_t)c + 1] = contig_first[(size_t)c] + (int64_t)v.size();
+            upos.insert(upos.end(), v.begin(), v.end());
+        }
+        slot_unique.assign((size_t)P, 0);
+        for (int64_t s = 0; s < P; ++s) {
+            const int32_t c = panel.slot_chrom[s];
+            if (c < 0 || panel.slot_pos[s] < 1) { no_position.push_back((int32_t)s); continue; }
+            const auto b = upos.begin() + contig_first[(size_t)c], e = upos.begin() + contig_first[(size_t)c + 1];
+            slot_unique[(size_t)s] = (int32_t)(std::lower_bound(b, e, panel.slot_pos[s] - 1) - upos.begin());
+        }
+    }
+};
+
+// A packed group -> the 16-bit format, on the host and losslessly (the pileups are not run again): a record escaped in the
+// packed form may fit the 16-bit one (a second count above 15) and a record that fits the packed form may not (a count of
+// 65534 or 65535).  hc.wide must be sorted by (slot, sample).
+bool transcode_to_16(HostCounts& hc, size_t n, int64_t P) {
+    HostCounts out;
+    out.fmt = 2;
+    if (!out.reserve(std::max<size_t>(16, n * 2 * (size_t)P * 8))) return false;
+    std::vector<as_wide_record> wide;
+    std::mutex m;
+    const uint32_t* w = (const uint32_t*)hc.p;
+    uint16_t* o = (uint16_t*)out.p;
+    parallel_for(n * (size_t)P, [&](size_t i) {
+        const int64_t smp = (int64_t)i / P, s = (int64_t)i % P;
+        uint16_t* f = o + ((smp * 2) * P + s) * 4;
+        uint16_t* b = f + P * 4;
+        if (w[(smp * 2) * P + s] == AS_PACKED_ABSENT) {
+            for (int k = 0; k < 4; ++k) f[k] = b[k] = AS_WIRE_ABSENT;
+            return;
+        }
+        as_wide_record r;
+        hc.record(smp, s, P, r.fw, r.bw);
+        const bool fits = as_wire16_fits(r.fw) && as_wire16_fits(r.bw);
+        for (int k = 0; k < 4; ++k) {
+            f[k] = fits ? (uint16_t)r.fw[k] : (uint16_t)AS_WIRE_ESCAPE;
+            b[k] = fits ? (uint16_t)r.bw[k] : (uint16_t)AS_WIRE_ESCAPE;
+        }
+        if (!fits) {
+            r.sample = (int32_t)smp;
+            r.slot = (int32_t)s;
+            std::lock_guard<std::mutex> g(m);
+            wide.push_back(r);
+        }
+    });
+    std::sort(wide.begin(), wide.end(), [](const as_wide_record& x, const as_wide_record& y) {
+        return x.slot != y.slot ? x.slot < y.slot : x.sample < y.sample;
+    });
+    hc.release();
+    std::swap(hc.p, out.p);
+    std::swap(hc.bytes, out.bytes);
+    hc.fmt = 2;
+    hc.wide = std::move(wide);
+    return true;
+}
+
+// samples [first, first + n) of `files` (BAM files) with the contract of load_counts: the same HostCounts, one AseqStats per
+// file (rows = present slots, in panel order).  The wire-format policy is load_counts' too: packed, and the 16-bit format for
+// the group when more than 1 record in 16 escapes (AS_WIRE=16 / packed forces one).  Returns 0 ok, 1 pinned allocation
+// failed, 3 a BAM could not be read or piled up (computeCounts' message printed).  pctx runs the pileups: no other thread
+// may use it meanwhile.
+int load_bam_counts(const std::vector<CountFile>& files, size_t first, size_t n, const Panel& panel, BamInput& bi, as_ctx* pctx,
+                    HostCounts& hc, std::vector<AseqStats>& stats) {
+    const int64_t P = panel.size();
+    const char* force = getenv("AS_WIRE");
+    if (force && !strcmp(force, "16")) hc.fmt = 2;
+    const int fmt = hc.fmt;
+    const size_t per_sample = 2 * (size_t)P * 4 * (size_t)fmt;  // bytes of one sample's slice
+    if (!hc.reserve(std::max<size_t>(16, n * per_sample))) return 1;
+    hc.wide.clear();
+    stats.assign(n, AseqStats());
+    if (bi.upos.empty()) {
+        printf("Error from computeCounts: no positions in the panel\n");
+        return 3;
+    }
+    const int threads = (int)std::max(1u, std::thread::hardware_concurrency());
+    std::vector<as_wide_record> w((size_t)P);
+    int64_t rows_all = 0;
+    for (size_t i = 0; i < n; ++i) {
+        const int rc = bi.reader.pileup(files[first + i].path, bi.contig_id, threads, bi.mbq, bi.mrq, [&]() -> as_ctx* {
+            if (as_pileup_begin(pctx, bi.contig_first.data(), (int32_t)(bi.contig_first.size() - 1), bi.upos.data(), (int64_t)bi.upos.size()) != AS_OK) {
+                printf("Error from computeCounts: %s\n", as_last_error());
+                return nullptr;
+            }
+            return pctx;
+        }, nullptr);
+        if (rc != 0) return 3;
+        char* slice = (char*)hc.p + i * per_sample;
+        int64_t n_wide = 0, rows = 0;
+        if (as_pileup_end_wire(pctx, bi.slot_unique.data(), P, bi.mdc, fmt, (int32_t)i, slice, w.data(), P, &n_wide, &rows, nullptr) != AS_OK) {
+            printf("Error from computeCounts: %s\n", as_last_error());
+            return 3;
+        }
+        for (int32_t s : bi.no_position) {  // no line of the position file: absent whatever mdc is
+            const bool present = fmt == 1 ? ((uint32_t*)slice)[s] != AS_PACKED_ABSENT : ((uint16_t*)slice)[(size_t)s * 4] != AS_WIRE_ABSENT;
+            rows -= present ? 1 : 0;
+            if (fmt == 1) ((uint32_t*)slice)[s] = ((uint32_t*)slice)[P + s] = AS_PACKED_ABSENT;
+            else memset(slice + (size_t)s * 8, 0xFF, 8), memset(slice + (size_t)(P + s) * 8, 0xFF, 8);
+        }
+        for (int64_t k = 0; k < n_wide; ++k) {
+            const as_wide_record& r = w[(size_t)k];
+            if (bi.no_position.empty() || !std::binary_search(bi.no_position.begin(), bi.no_position.end(), r.slot)) hc.wide.push_back(r);
+        }
+        stats[i].rows = rows;
+        rows_all += rows;
+    }
+    std::sort(hc.wide.begin(), hc.wide.end(), [](const as_wide_record& x, const as_wide_record& y) {
+        return x.slot != y.slot ? x.slot < y.slot : x.sample < y.sample;
+    });
+    if (fmt == 1 && (int64_t)hc.wide.size() * 16 > rows_all && !(force && !strcmp(force, "packed")))  // the 16-bit format is denser
+        if (!transcode_to_16(hc, n, P)) return 1;
+    return 0;
+}
+
 // The GPUs of a run, chosen BEFORE the first CUDA call from the size of the ASEQ directory (bytes / 45 ~ records):
 //   AS_DEVICES ("0,2,3") names them; otherwise a job below 2^28 records (2 GB in the packed format, ~40 ms of GPU time) runs
 //   on one GPU -- several would only add start-up time -- and a larger one on every visible GPU (as_create_multi).
 // When the process's device list is not fixed from outside, CUDA_VISIBLE_DEVICES is narrowed to the chosen devices first, so
 // that the driver initialises those only (start-up grows with the number of visible GPUs).  The context is created on a
 // thread at program entry: CUDA start-up takes 0.2-4 s on the test boxes, the panel / noise table is read meanwhile.
+// A directory of BAM input (bam_input_dir) is sized from its BAM bytes: an amplicon BAM holds some thousands of compressed
+// bytes per panel position (150-base reads at a few thousand x), so bytes / 4096 ~ records errs towards one GPU.
 double aseq_dir_records(const std::string& dir) {
-    double bytes = 0;
+    double bytes = 0, bam_bytes = 0;
     if (DIR* d = opendir(dir.c_str())) {
         while (dirent* en = readdir(d)) {
             const std::string n = en->d_name;
             struct stat sb;
             if (n.size() >= 5 && n.compare(n.size() - 5, 5, ".ASEQ") == 0 && stat((dir + "/" + n).c_str(), &sb) == 0) bytes += (double)sb.st_size;
+            if (ends_with(n, ".bam") && n[0] != '.' && stat((dir + "/" + n).c_str(), &sb) == 0) bam_bytes += (double)sb.st_size;
         }
         closedir(d);
     }
-    return bytes / 45.0;
+    return bam_input_dir(dir) ? bam_bytes / 4096.0 : bytes / 45.0;
 }
 
 // In the resident service (as_serve.cpp: one request at a time) the context object of a finished program is parked, not
@@ -1281,11 +1465,18 @@ int report_gpu_error(const char* what) {
     return 1;
 }
 
+void usage_bam() {
+    std::cout << "\tA count directory that holds *.bam files and no *.ASEQ file is read as BAM input: every BAM is piled up on the GPU\n"
+                 "\tas computeCounts would (sample name = file name minus .bam), with AS_BAM_MBQ / AS_BAM_MRQ / AS_BAM_MDC in the\n"
+                 "\tenvironment for its mbq / mrq / mdc (default 20 / 20 / 20)."
+              << std::endl;
+}
+
 void usage_ee() {
     std::cout << "Please type the following: " << std::endl;
     std::cout << "\n./AmpliSolveErrorEstimation" << GREEN << " panel_design=" << RESET << "/your/panel/design/file/in/bed/format" << GREEN
               << " reference_genome=" << RESET << "/your/reference/genome/in/fasta/format/indexed" << GREEN << " germline_dir=" << RESET
-              << "/dir/with/normal/count/files" << GREEN << " C_value=" << RESET << "/C/value/of/the/error/model" << GREEN
+              << "/dir/with/normal/count/files/or/BAM/files" << GREEN << " C_value=" << RESET << "/C/value/of/the/error/model" << GREEN
               << " coverage_cutoff=" << RESET << "/coverage/per/strand" << GREEN << " default_error=" << RESET
               << "/platform/specific/error/used/without/normals" << GREEN << " output_dir=" << RESET << "/dir/to/store/all/outputs"
               << std::endl;
@@ -1294,13 +1485,14 @@ void usage_ee() {
                  "C_value=0.002 coverage_cutoff=100 default_error=0.01 output_dir=ErrorEstimation_Testing"
               << std::endl;
     std::cout << "\n\tIt is important to give the arguments in this order. Otherwise the program will crach !" << std::endl;
+    usage_bam();
     std::cout << STARS << std::endl;
 }
 
 void usage_vc() {
     std::cout << "Please type the following: " << std::endl;
     std::cout << "\n./AmpliSolveVariantCalling" << GREEN << " errorFile=" << RESET << "/the/file/produced/by/AmpliSolveErrorEstimation" << GREEN
-              << " tumour_dir=" << RESET << "/your/dir/with/tumour/read/count/files " << GREEN << "output_dir=" << RESET
+              << " tumour_dir=" << RESET << "/your/dir/with/tumour/read/count/files/or/BAM/files " << GREEN << "output_dir=" << RESET
               << "/dir/to/store/all/outputs" << GREEN << " coverage_cutoff=" << RESET << "/coverage/per/strand/required/to/do/predictions"
               << GREEN << " p_value=" << RESET << "/Fisher's/exact/test/p/value/for/strand/bias" << std::endl;
     std::cout << "\nExecution example:" << std::endl;
@@ -1308,6 +1500,7 @@ void usage_vc() {
                  "output_dir=VariantCalling_Testing coverage_cutoff=100 p_value=0.05"
               << std::endl;
     std::cout << "\n\tIt is important to give the arguments in this order. Otherwise the program will crach !" << std::endl;
+    usage_bam();
     std::cout << STARS << std::endl;
 }
 
@@ -1412,6 +1605,11 @@ int as_error_estimation_main(int argc, char** argv) {
         std::cout << "\t5. Coverage cutoff                                : " << GREEN << cut << RESET << std::endl;
     }
     std::cout << "\t6. Output dir                                     : " << GREEN << output_dir << RESET << std::endl;
+    const bool bam_input = with_germlines && bam_input_dir(germline_dir);
+    BamInput bam;
+    if (bam_input)
+        std::cout << "\t7. BAM pileup (AS_BAM_MBQ / AS_BAM_MRQ / AS_BAM_MDC) : " << GREEN << bam.mbq << " / " << bam.mrq << " / " << bam.mdc
+                  << RESET << std::endl;
 
     const std::string interm = output_dir + "/AmpliSolveErrorEstimation_interm_files";
     if (!make_dir(interm)) {
@@ -1498,7 +1696,8 @@ int as_error_estimation_main(int argc, char** argv) {
     // normals in the reference's file order
     std::vector<CountFile> files;
     std::vector<std::string> listed;
-    if (!list_count_files(germline_dir, files, listed)) {
+    bool bam_files = false;
+    if (!list_count_files(germline_dir, files, listed, &bam_files)) {
         std::cout << "Error: cannot list " << germline_dir << "/*.ASEQ" << std::endl;
         return 0;
     }
@@ -1515,8 +1714,11 @@ int as_error_estimation_main(int argc, char** argv) {
     std::cout << "Running function storeGermlineStatistics:" << std::endl;
     HostCounts counts;
     std::vector<AseqStats> stats;
-    const int lrc = load_counts(files, 0, files.size(), panel, counts, stats);
+    if (bam_files) bam.setup(panel);  // the pileups run on this program's context: nothing else uses it meanwhile
+    const int lrc = bam_files ? load_bam_counts(files, 0, files.size(), panel, bam, ctx, counts, stats)
+                              : load_counts(files, 0, files.size(), panel, counts, stats);
     if (lrc == 1) return report_gpu_error("pinned host allocation");
+    if (lrc == 3) return 0;  // a BAM that cannot be read: reported like an ASEQ file that cannot be opened
     if (lrc == 2) {
         for (int i = 0; i < S; ++i)
             if (!stats[i].ok) printf("Error: Cannot open %s\n", files[i].path.c_str());
@@ -1526,7 +1728,7 @@ int as_error_estimation_main(int argc, char** argv) {
     {
         double rows = 0;
         for (const AseqStats& st : stats) rows += (double)st.rows;
-        timer.lap("parse_normals", rows, "rows");
+        timer.lap(bam_files ? "pileup_normals" : "parse_normals", rows, "rows");
     }
 
     std::cout << "Running function estimateThresholds: ";
@@ -1800,6 +2002,10 @@ int as_variant_calling_main(int argc, char** argv) {
     } else {
         std::cout << "\t5. p-value                                        : " << GREEN << p_value_float << RESET << std::endl;
     }
+    BamInput bam;
+    if (bam_input_dir(tumour_dir))
+        std::cout << "\t6. BAM pileup (AS_BAM_MBQ / AS_BAM_MRQ / AS_BAM_MDC) : " << GREEN << bam.mbq << " / " << bam.mrq << " / " << bam.mdc
+                  << RESET << std::endl;
     std::cout << std::endl;
 
     const std::string interm = output_dir + "/AmpliSolveVariantCalling_interm_files";
@@ -1861,7 +2067,8 @@ int as_variant_calling_main(int argc, char** argv) {
     const int seed = rand() % 1000;  // VC:328-331
     std::vector<CountFile> files;
     std::vector<std::string> listed;
-    if (!list_count_files(tumour_dir, files, listed)) {
+    bool bam_files = false;
+    if (!list_count_files(tumour_dir, files, listed, &bam_files)) {
         std::cout << "Error: cannot list " << tumour_dir << "/*.ASEQ" << std::endl;
         return 0;
     }
@@ -1875,6 +2082,18 @@ int as_variant_calling_main(int argc, char** argv) {
         return 1;
     }
     as_ctx* ctx = gpu.ctx;
+    // BAM input: the pileups of group g + 1 run on the main thread while the caller of group g runs on the worker thread
+    // below, so they get a context of their own (as_ctx is not thread-safe) on the run's first device
+    struct PileupContext {
+        as_ctx* c = nullptr;
+        ~PileupContext() { if (c && as_process_is_resident()) as_destroy(c); }  // the service lives on; a program leaves through _exit
+    } pile;
+    if (bam_files) {
+        int dev = 0;
+        as_context_devices(ctx, &dev, 1);
+        if (as_create(dev, &pile.c) != AS_OK) return report_gpu_error("as_create (pileup)");
+        bam.setup(panel);
+    }
     timer.lap("cuda_context_wait");
     std::cout << "\nRunning function callVariants...." << std::endl;
 
@@ -1899,7 +2118,8 @@ int as_variant_calling_main(int argc, char** argv) {
             const double t0 = PhaseTimer::now();
             const size_t n = (size_t)std::min<int64_t>(G, T - first);
             buf[which].fmt = std::max(buf[which].fmt, buf[which ^ 1].fmt);  // once the 16-bit format was needed it stays
-            const int lrc = load_counts(files, (size_t)first, n, panel, buf[which], stats[which], true);
+            const int lrc = bam_files ? load_bam_counts(files, (size_t)first, n, panel, bam, pile.c, buf[which], stats[which])
+                                      : load_counts(files, (size_t)first, n, panel, buf[which], stats[which], true);
             if (lrc == 2)
                 for (size_t i = 0; i < n; ++i)
                     if (!stats[which][i].ok) printf("\tError from callVariants:  Cannot open %s\n", files[(size_t)first + i].path.c_str());
@@ -1908,7 +2128,7 @@ int as_variant_calling_main(int argc, char** argv) {
         };
         int lrc = load_group(0, 0);
         if (lrc == 1) return report_gpu_error("pinned host allocation");
-        if (lrc == 2) return 0;
+        if (lrc >= 2) return 0;  // 3: a BAM that cannot be read, reported like an ASEQ file that cannot be opened
         for (int64_t first = 0, g = 0; first < T; first += G, ++g) {
             const int which = (int)(g & 1);
             const int32_t Tg = (int32_t)std::min<int64_t>(G, T - first);
@@ -1949,7 +2169,7 @@ int as_variant_calling_main(int argc, char** argv) {
                 return 1;
             }
             if (next_rc == 1) return report_gpu_error("pinned host allocation");
-            if (next_rc == 2) return 0;
+            if (next_rc >= 2) return 0;
             part.resize((size_t)n_part);
             const size_t base = calls.size();
             calls.resize(base + part.size());
@@ -2077,8 +2297,8 @@ int as_variant_calling_main(int argc, char** argv) {
             std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)lo);
         }
     }
-    if (timer.on) fprintf(stderr, "AS_TIMING parse_tumours_busy %.6f (%.3g rows/s)\nAS_TIMING caller_gpu_busy %.6f\n", parse_s,
-                          total_rows / std::max(parse_s, 1e-9), gpu_s);
+    if (timer.on) fprintf(stderr, "AS_TIMING %s %.6f (%.3g rows/s)\nAS_TIMING caller_gpu_busy %.6f\n",
+                          bam_files ? "pileup_tumours_busy" : "parse_tumours_busy", parse_s, total_rows / std::max(parse_s, 1e-9), gpu_s);
     timer.lap("parse_and_call", 6.0 * (double)T * (double)P, "tests");
 
     // Fisher strand-bias p of every call (VC:902) on the device: one warp per call's 2x2 table

@@ -73,6 +73,12 @@ cudaError_t as_launch_pileup(const uint8_t* d_rec, const int64_t* d_rec_off, int
                              const int32_t* d_ref_contig, int32_t n_ref, const int64_t* d_contig_first,
                              const int32_t* d_slot_pos, int64_t P, int32_t mbq, int32_t mrq, uint32_t skip_flags,
                              uint32_t* d_counts, unsigned long long* d_stats, cudaStream_t st);
+// counts [2][U][4] of one sample -> its wire slice: fmt 1 packed [2][P] uint32, fmt 2 uint16 [2][P][4]; slot s takes
+// position d_slot_unique[s], a depth below mdc is absent; escaped records -> d_wide (at most cap kept), d_n[0] = escaped,
+// d_n[1] += present slots (zero d_n first)
+cudaError_t as_launch_pileup_encode(int fmt, const uint32_t* d_counts, int64_t U, const int32_t* d_slot_unique, int64_t P,
+                                    int32_t mdc, int32_t sample, void* d_wire, as_wide_record* d_wide, int64_t cap,
+                                    unsigned long long* d_n, cudaStream_t st);
 cudaError_t as_launch_poisson_test(const int32_t* k, const int32_t* rd, const float* err, int64_t n, double* p,
                                    double* q, cudaStream_t st);
 cudaError_t as_launch_gammaq(const double* s, const double* z, int64_t n, double* out, cudaStream_t st);

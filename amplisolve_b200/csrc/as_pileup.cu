@@ -9,13 +9,17 @@
 //   * a base is counted when its CIGAR op aligns it to the reference (M, =, X), its quality is >= mbq (a record without
 //     qualities, 0xFF, counts), and it is A, C, G or T;  deletions, reference skips, insertions, clips count nothing;
 //   * strand = flag 0x10;  counts[strand][slot][base] is exactly the layout of the count tensor of one sample
-//     (include/amplisolve_b200.h), so a pileup can feed the noise model / caller without a text file in between.
+//     (include/amplisolve_b200.h), so a pileup feeds the noise model / caller without a text file in between: the two
+//     programs read a directory of BAM files through pileup_encode_kernel (as_pileup_end_wire).
 //
 // Input: the UNCOMPRESSED record stream of a BAM file (what BGZF inflates to, header stripped) and the byte offset of
 // every record; the panel as sorted 0-based positions per contig.  One warp per read: the CIGAR is walked by the whole
 // warp (uniform); for an aligned block the range of panel slots under it is found by two binary searches and the lanes
 // walk those slots (not the read's bases: a base outside the panel costs nothing).
+//
+// pileup_encode_kernel (below) turns the counts of one sample into its slice of the programs' host wire tensor.
 #include "as_kernels.h"
+#include "as_wire.h"
 
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -114,9 +118,90 @@ pileup_kernel(const uint8_t* __restrict__ rec, const int64_t* __restrict__ rec_o
     }
 }
 
+// The pileup of one sample -> that sample's slice of a host wire tensor (include/amplisolve_b200.h), so the two programs
+// read BAM files without ASEQ text in between.  counts [2][U][4] over the U unique panel positions; slot s of the panel
+// takes the record of position slot_unique[s] (twin slots share one); a slot whose depth (64-bit sum of its eight counts,
+// as computeCounts sums it) is below mdc is ABSENT.  FMT 1: packed words [2][P] (as_pack_word); FMT 2: uint16 [2][P][4]
+// (escaped when a count is >= AS_WIRE_ESCAPE).  Escaped records go to wide[] by warp-ballot compaction (one atomic per
+// warp; n[0] counts all of them, entries beyond cap are dropped), present slots to n[1].  One thread per slot.
+template <int FMT>
+__global__ void __launch_bounds__(256)
+pileup_encode_kernel(const uint32_t* __restrict__ counts, int64_t U, const int32_t* __restrict__ slot_unique, int64_t P,
+                     int32_t mdc, int32_t sample, void* __restrict__ wire, as_wide_record* __restrict__ wide, int64_t cap,
+                     unsigned long long* __restrict__ n) {
+    const int lane = threadIdx.x & 31;
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bool present = false, escape = false;
+    uint32_t f[4] = {0u, 0u, 0u, 0u}, b[4] = {0u, 0u, 0u, 0u};
+    if (s < P) {
+        const int64_t u = slot_unique[s];
+        const uint4 fv = reinterpret_cast<const uint4*>(counts)[u];
+        const uint4 bv = reinterpret_cast<const uint4*>(counts)[U + u];
+        f[0] = fv.x; f[1] = fv.y; f[2] = fv.z; f[3] = fv.w;
+        b[0] = bv.x; b[1] = bv.y; b[2] = bv.z; b[3] = bv.w;
+        const unsigned long long depth = (unsigned long long)f[0] + f[1] + f[2] + f[3] + b[0] + b[1] + b[2] + b[3];
+        present = depth >= (unsigned long long)(mdc > 0 ? mdc : 0);
+        if (FMT == 1) {
+            uint32_t* w = static_cast<uint32_t*>(wire);
+            uint32_t wf = AS_PACKED_ABSENT, wb = AS_PACKED_ABSENT;
+            if (present) {
+                escape = !(as_pack_word(f, &wf) && as_pack_word(b, &wb));
+                if (escape) wf = wb = AS_PACKED_ESCAPE;
+            }
+            w[s] = wf;
+            w[P + s] = wb;
+        } else {
+            uint2* w = static_cast<uint2*>(wire);  // four uint16 counts = 8 bytes per (strand, slot)
+            uint2 wf = make_uint2(0xFFFFFFFFu, 0xFFFFFFFFu), wb = wf;  // AS_WIRE_ABSENT in all four
+            if (present) {
+                escape = !(as_wire16_fits(f) && as_wire16_fits(b));
+                if (escape) {
+                    wf = wb = make_uint2(0xFFFEFFFEu, 0xFFFEFFFEu);  // AS_WIRE_ESCAPE in all four
+                } else {
+                    wf = make_uint2(f[0] | f[1] << 16, f[2] | f[3] << 16);
+                    wb = make_uint2(b[0] | b[1] << 16, b[2] | b[3] << 16);
+                }
+            }
+            w[s] = wf;
+            w[P + s] = wb;
+        }
+    }
+    const unsigned esc = __ballot_sync(0xFFFFFFFFu, escape);
+    const unsigned pre = __ballot_sync(0xFFFFFFFFu, present);
+    unsigned long long base = 0;
+    if (lane == 0) {
+        if (esc) base = atomicAdd(&n[0], (unsigned long long)__popc(esc));
+        if (pre) atomicAdd(&n[1], (unsigned long long)__popc(pre));
+    }
+    base = __shfl_sync(0xFFFFFFFFu, base, 0);
+    if (escape) {
+        const unsigned long long k = base + (unsigned long long)__popc(esc & ((1u << lane) - 1u));
+        if ((int64_t)k < cap) {
+            as_wide_record r;
+            r.sample = sample;
+            r.slot = (int32_t)s;
+            for (int i = 0; i < 4; ++i) { r.fw[i] = f[i]; r.bw[i] = b[i]; }
+            wide[k] = r;
+        }
+    }
+}
+
 }  // namespace asdev
 
 using namespace asdev;
+
+cudaError_t as_launch_pileup_encode(int fmt, const uint32_t* d_counts, int64_t U, const int32_t* d_slot_unique, int64_t P,
+                                    int32_t mdc, int32_t sample, void* d_wire, as_wide_record* d_wide, int64_t cap,
+                                    unsigned long long* d_n, cudaStream_t st) {
+    if (P <= 0) return cudaSuccess;
+    const int threads = 256;
+    const unsigned blocks = (unsigned)((P + threads - 1) / threads);
+    if (fmt == 1)
+        pileup_encode_kernel<1><<<blocks, threads, 0, st>>>(d_counts, U, d_slot_unique, P, mdc, sample, d_wire, d_wide, cap, d_n);
+    else
+        pileup_encode_kernel<2><<<blocks, threads, 0, st>>>(d_counts, U, d_slot_unique, P, mdc, sample, d_wire, d_wide, cap, d_n);
+    return cudaGetLastError();
+}
 
 cudaError_t as_launch_pileup(const uint8_t* d_rec, const int64_t* d_rec_off, int64_t n_rec, int64_t n_bytes,
                              const int32_t* d_ref_contig, int32_t n_ref, const int64_t* d_contig_first,

@@ -28,8 +28,10 @@
  *     not the same as a row of zeros: absence changes N in the 0.338*N rule (EE:1742).  Valid counts
  *     are < 2^31 (the reference reads them with %d).
  *     Derivation from an ASEQ row (EE:1149-1176, VC:752-770): fw[b] = X - X_rs, bw[b] = X_rs; the RD
- *     column must equal the sum of the eight words (true of every row the reference's own pileup
- *     step writes; the loader rejects files where it is not).
+ *     column equals the sum of the eight words in every row the reference's own pileup step writes (the
+ *     programs still accept a row where it does not: the error estimation warns, the caller uses the
+ *     column as the reference does).  A BAM file
+ *     yields the same record without text in between (as_pileup_end_wire below).
  *   Twin slots: a position enumerated by two overlapping amplicons owns several slots.  The
  *     reference keys records by "chrom_pos" text, so all rows of all twins feed one noise estimate
  *     (EE:1241-1245).  twin_next[slot] = next slot of the same position (or -1); twin_head[slot] =
@@ -275,11 +277,29 @@ int as_synth_twin_links_dev(as_ctx* ctx, int64_t P, const as_synth_params* prm, 
  *                   == 0; a base when it is aligned (M, =, X), A/C/G/T and of quality >= mbq.  Any number of pieces.
  * as_pileup_end_host downloads counts (host, 2 * P * 4 uint32: forward strand first) and the number of reads / bases
  *                   used (stats_out[2], may be NULL).
- * The device buffer keeps the layout of one sample of the count tensor, [strand][slot][base]. */
+ * The device buffer keeps the layout of one sample of the count tensor, [strand][slot][base].
+ * How a BAM file yields the count tensor of the two programs (a germline_dir= / tumour_dir= that holds *.bam files and no
+ * *.ASEQ file): the P slots of the program's panel map to the U sorted unique positions of the pileup through
+ * slot_unique[P] (twin slots name the same position); the pileup of each BAM runs on the GPU and ends with
+ * as_pileup_end_wire instead of as_pileup_end_host, which writes that sample's slice of the host wire tensor directly:
+ * slot s gets the record of position slot_unique[s], or is ABSENT when the depth of that record (the sum of its eight
+ * counts, in 64 bits) is below mdc.  The result is the tensor the ASEQ loader builds from the files computeCounts writes
+ * with the same mbq / mrq / mdc for a position file that lists the panel's slots in order.
+ * as_pileup_end_wire: fmt 1 = packed, wire = uint32 [2][P] (forward words first, then reverse); fmt 2 = 16-bit, wire =
+ *                   uint16 [2][P][4]; ABSENT / ESCAPE markers as above.  Escaped records go to wide (sample = `sample`,
+ *                   sorted by slot); *n_wide = their number, AS_EOVERFLOW when it exceeds wide_cap (wire and *n_wide are
+ *                   complete; the pileup stays open, so the call can be repeated with a larger list).  *rows_out = present
+ *                   slots, stats_out[2] as in as_pileup_end_host (both may be NULL).  AS_EINVAL for a slot_unique entry
+ *                   outside [0, U).  Ends the pileup on success.
+ * as_pileup_set_host replaces the counts of the open pileup with host counts [2][U][4] (a pileup made elsewhere; tests).
+ * A context of several GPUs runs the pileup on its first. */
 int as_pileup_begin(as_ctx* ctx, const int64_t* contig_first, int32_t n_contig, const int32_t* slot_pos, int64_t P);
 int as_pileup_add_host(as_ctx* ctx, const uint8_t* records, int64_t n_bytes, const int64_t* rec_off, int64_t n_rec,
                        const int32_t* ref_contig, int32_t n_ref, int32_t mbq, int32_t mrq, uint32_t skip_flags);
 int as_pileup_end_host(as_ctx* ctx, uint32_t* counts, uint64_t* stats_out);
+int as_pileup_end_wire(as_ctx* ctx, const int32_t* slot_unique, int64_t P, int32_t mdc, int32_t fmt, int32_t sample, void* wire,
+                       as_wide_record* wide, int64_t wide_cap, int64_t* n_wide, int64_t* rows_out, uint64_t* stats_out);
+int as_pileup_set_host(as_ctx* ctx, const uint32_t* counts);
 
 /* ---- host side of the two programs (text formats; amplisolve_b200/csrc/as_host.cpp) ---------- */
 /* Iteration order of a libstdc++ std::unordered_map<std::string,std::string> after inserting keys
@@ -303,7 +323,10 @@ double as_fisher_test(int32_t fw, int32_t bw, int32_t alt_fw, int32_t alt_bw);
 int as_fisher_tests_host(as_ctx* ctx, const int32_t* tables, int64_t n, double* p);
 
 /* Whole programs, argv-compatible with the reference (EE:241-520, VC:199-360).  Exit status is
- * the return value; like the reference, usage errors print the usage text and return 0. */
+ * the return value; like the reference, usage errors print the usage text and return 0.  germline_dir= / tumour_dir= may
+ * also name a directory of *.bam files (and no *.ASEQ file): the programs then pile the BAMs up on the GPU themselves, with
+ * mbq / mrq / mdc from AS_BAM_MBQ / AS_BAM_MRQ / AS_BAM_MDC (default 20 / 20 / 20, skip flags 0x704), and write what
+ * computeCounts followed by the same program would write. */
 int as_error_estimation_main(int argc, char** argv);
 int as_variant_calling_main(int argc, char** argv);
 /* computeCounts / ASEQ PILEUP mode (Execution_examples.md:27): [vcf=positions] [bam=file.bam] [threads=n] [mbq=n] [mrq=n]
