@@ -29,7 +29,9 @@ EXPORTS = [
     "as_last_error", "as_version", "as_device_count", "as_create", "as_create_multi", "as_context_devices", "as_shard_bounds", "as_destroy", "as_host_alloc", "as_host_free",
     "as_set_call_kernel", "as_set_noise_kernel", "as_set_host_tile_slots", "as_set_option", "as_kernel_launches", "as_noise_estimate_dev", "as_noise_estimate_host",
     "as_noise_estimate_host16", "as_thresholds_caller_view_dev", "as_call_variants_dev", "as_call_variants_host",
-    "as_call_variants_host16", "as_sort_calls_dev", "as_call_variants_sweep_dev", "as_noise_estimate_sweep_dev", "as_pack_counts", "as_noise_estimate_host_packed", "as_call_variants_host_packed", "as_poisson_test_host",
+    "as_call_variants_host16", "as_sort_calls_dev", "as_call_variants_sweep_dev", "as_noise_estimate_sweep_dev", "as_pack_counts", "as_noise_estimate_host_packed", "as_call_variants_host_packed",
+    "as_noise_estimate_sweep_host", "as_noise_estimate_sweep_host16", "as_noise_estimate_sweep_host_packed", "as_call_variants_sweep_host",
+    "as_call_variants_sweep_host16", "as_call_variants_sweep_host_packed", "as_poisson_test_host",
     "as_kf_gammaq_host", "as_synth_counts_dev", "as_synth_twin_links_dev", "as_hash_iteration_order", "as_fisher_test", "as_fisher_tests_host", "as_error_estimation_main",
     "as_variant_calling_main", "as_pileup_begin", "as_pileup_add_host", "as_pileup_end_host", "as_pileup_end_wire", "as_pileup_set_host", "as_compute_counts_main", "as_serve_main", "as_client_run", "as_process_is_resident",
 ]
@@ -162,6 +164,12 @@ def lib():
     L.as_call_variants_host16.argtypes = [vp, vp, vp, i64, i32, i64, vp, vp, i32, vp, i64, C.POINTER(i64)]
     L.as_noise_estimate_host_packed.argtypes = L.as_noise_estimate_host16.argtypes
     L.as_call_variants_host_packed.argtypes = L.as_call_variants_host16.argtypes
+    L.as_noise_estimate_sweep_host.argtypes = [vp, vp, i32, i64, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp]
+    L.as_noise_estimate_sweep_host16.argtypes = [vp, vp, vp, i64, i32, i64, vp, vp, vp, i32, i32, vp, vp, vp, vp, vp, vp]
+    L.as_noise_estimate_sweep_host_packed.argtypes = L.as_noise_estimate_sweep_host16.argtypes
+    L.as_call_variants_sweep_host.argtypes = [vp, vp, i32, i64, vp, vp, i32, i32, vp, i64, vp]
+    L.as_call_variants_sweep_host16.argtypes = [vp, vp, vp, i64, i32, i64, vp, vp, i32, i32, vp, i64, vp]
+    L.as_call_variants_sweep_host_packed.argtypes = L.as_call_variants_sweep_host16.argtypes
     L.as_pack_counts.argtypes = [vp, i32, i64, vp, vp, i64, C.POINTER(i64)]
     L.as_poisson_test_host.argtypes = [vp, vp, vp, vp, i64, vp, vp]
     L.as_kf_gammaq_host.argtypes = [vp, vp, vp, i64, vp]
@@ -375,6 +383,59 @@ class Context:
             return self.call_variants(counts, ref, thr_view, coverage_cutoff, cap=int(n.value), wide_records=wide_records,
                                       pinned_outputs=pinned_outputs)
         return calls[:n.value]
+
+    def estimate_thresholds_sweep(self, counts, c_values, coverage_cutoff, twin_next=None, twin_head=None, wide_records=None):
+        """Noise-floor sweep on the host path (as_noise_estimate_sweep_host*): the dict of estimate_thresholds(with_view=True)
+        with thr / thr_view of shape [n_c][P][4][2], table i bit for bit that of c_values[i].  One upload of counts."""
+        fmt = _host_format(counts)
+        counts = _np(counts, np.uint16 if fmt == "u16" else np.uint32)
+        wr = _np(wide_records if wide_records is not None else np.zeros(0, WIDE_DTYPE), WIDE_DTYPE)
+        cv = _np(c_values, np.float32).reshape(-1)
+        S, two, P = counts.shape[:3]
+        assert two == 2 and (fmt == "packed" or counts.shape[3] == 4)
+        n_c = len(cv)
+        out = {"thr": np.empty((n_c, P, 4, 2), np.float32), "germ_val": np.empty((P, 4), np.float32),
+               "germ_state": np.empty((P, 4), np.uint8), "count": np.empty((P, 4), np.uint32), "nrec": np.empty(P, np.uint32),
+               "thr_view": np.empty((n_c, P, 4, 2), np.float32)}
+        tn = th = None
+        if twin_next is not None:
+            tn, th = _np(twin_next, np.int32), _np(twin_head, np.int32)
+        tail = (None if tn is None else _hp(tn), None if th is None else _hp(th), _hp(cv), n_c, int(coverage_cutoff),
+                _hp(out["thr"]), _hp(out["germ_val"]), _hp(out["germ_state"]), _hp(out["count"]), _hp(out["nrec"]),
+                _hp(out["thr_view"]))
+        if fmt == "u32":
+            _check(lib().as_noise_estimate_sweep_host(self._h, _hp(counts), S, P, *tail))
+        else:
+            fn = lib().as_noise_estimate_sweep_host16 if fmt == "u16" else lib().as_noise_estimate_sweep_host_packed
+            _check(fn(self._h, _hp(counts), _hp(wr), len(wr), S, P, *tail))
+        return out
+
+    def call_variants_sweep(self, counts, ref, thr_views, coverage_cutoff, cap=None, wide_records=None):
+        """Caller sweep on the host path (as_call_variants_sweep_host*): thr_views [n_c][P][4][2]; returns one call array
+        per table, each what call_variants returns for that table.  One upload of counts."""
+        fmt = _host_format(counts)
+        counts = _np(counts, np.uint16 if fmt == "u16" else np.uint32)
+        wr = _np(wide_records if wide_records is not None else np.zeros(0, WIDE_DTYPE), WIDE_DTYPE)
+        T, two, P = counts.shape[:3]
+        assert two == 2 and (fmt == "packed" or counts.shape[3] == 4)
+        ref = _np(ref, np.uint8)
+        thr_views = _np(thr_views, np.float32)
+        n_c = thr_views.shape[0]
+        assert ref.shape == (P,) and thr_views.shape == (n_c, P, 4, 2)
+        if cap is None:
+            cap = max(1024, T * P // 8)
+        calls = np.empty((n_c, cap), dtype=CALL_DTYPE)
+        n = np.zeros(n_c, np.int64)
+        tail = (T, P, _hp(ref), _hp(thr_views), n_c, int(coverage_cutoff), _hp(calls), cap, _hp(n))
+        if fmt == "u32":
+            rc = lib().as_call_variants_sweep_host(self._h, _hp(counts), *tail)
+        else:
+            fn = lib().as_call_variants_sweep_host16 if fmt == "u16" else lib().as_call_variants_sweep_host_packed
+            rc = fn(self._h, _hp(counts), _hp(wr), len(wr), *tail)
+        _check(rc, allow_overflow=True)
+        if rc == -5:
+            return self.call_variants_sweep(counts, ref, thr_views, coverage_cutoff, cap=int(n.max()), wide_records=wide_records)
+        return [calls[i, :n[i]].copy() for i in range(n_c)]
 
     def mutation_rules_poisson_quality_score(self, k, rd, err):
         k, rd, err = _np(k, np.int32), _np(rd, np.int32), _np(err, np.float32)

@@ -507,29 +507,33 @@ static int check_wide(const HostSrc& src, int32_t n_samples, int64_t P) {
     return AS_OK;
 }
 
-struct NoiseOutLayout {  // one device block per tile: thr | germ_val | count | nrec | germ_state | thr_view
+struct NoiseOutLayout {  // one device block per tile: thr [n_c][n] | germ_val | count | nrec | germ_state | thr_view [n_c][n]
     size_t thr, germ_val, count, nrec, germ_state, view, total;
-    explicit NoiseOutLayout(int64_t n) {
+    NoiseOutLayout(int64_t n, int32_t n_c) {
         thr = 0;
-        germ_val = thr + (size_t)n * 32;
+        germ_val = thr + (size_t)n_c * (size_t)n * 32;
         count = germ_val + (size_t)n * 16;
         nrec = count + (size_t)n * 16;
         germ_state = nrec + (size_t)n * 4;
         view = germ_state + (size_t)n * 4;
-        total = view + (size_t)n * 32;
+        total = view + (size_t)n_c * (size_t)n * 32;
     }
 };
 
 // Slots [B, E) of the panel on ONE device (c is a single-device context).  Twin groups must not straddle B or E.
+// n_c values of C (1..8): thr and thr_view are [n_c][P][4][2].  n_c == 1 runs the single-value kernels (the staged
+// streaming kernel is faster than the pattern kernel for one C); n_c > 1 runs noise_pattern_kernel once per tile and
+// the twin groups once per value, as as_noise_estimate_sweep_dev does.
 static int noise_estimate_host_range(as_ctx* c, const HostSrc& src, int32_t S, int64_t P, int64_t B, int64_t E,
-                                     const int32_t* twin_next, const int32_t* twin_head, float C, int32_t cut, float* thr,
-                                     float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
+                                     const int32_t* twin_next, const int32_t* twin_head, const float* c_values, int32_t n_c,
+                                     int32_t cut, float* thr, float* germ_val, uint8_t* germ_state, uint32_t* count,
+                                     uint32_t* nrec, float* thr_view) {
     const int elem = src.elem;
     PhaseClock clk;
     if (E <= B) return AS_OK;
     CU(cudaSetDevice(c->device));
     const int64_t TP = tile_slots(c, S, E - B, elem);
-    const NoiseOutLayout lay(TP);
+    const NoiseOutLayout lay(TP, n_c);
     for (int i = 0; i < 2; ++i) {
         CU(c->tile[i].need((size_t)TP * 32 * (size_t)std::max(1, S)));
         if (elem != 4) CU(c->tile16[i].need((size_t)TP * 8 * (size_t)elem * (size_t)std::max(1, S)));
@@ -606,24 +610,46 @@ static int noise_estimate_host_range(as_ctx* c, const HostSrc& src, int32_t S, i
         uint8_t* o_gs = (uint8_t*)(o + lay.germ_state);
         uint32_t* o_cnt = (uint32_t*)(o + lay.count);
         uint32_t* o_nrec = (uint32_t*)(o + lay.nrec);
-        CUT(as_launch_noise_main(c->noise_cfg, (const uint32_t*)c->tile[bsel].p, S, n, 0, n, d_tn, d_th, 0, C, (uint32_t)cut,
-                                 o_thr, o_gv, o_gs, o_cnt, o_nrec, c->exec_stream));
-        c->launches += 1;
-        if (twin_next) {
-            CUT(as_launch_noise_twins(c->noise_cfg, (const uint32_t*)c->tile[bsel].p, S, n, 0, n, d_tn, d_th,
-                                      (int32_t*)c->heads.p, (uint32_t*)c->nheads.p, C, (uint32_t)cut, o_thr, o_gv, o_gs, o_cnt,
-                                      o_nrec, c->exec_stream));
-            c->launches += 3;
+        const uint32_t* d_tile = (const uint32_t*)c->tile[bsel].p;
+        // table i of the tile at o_thr + i * TP * 8 (the layout's stride), downloaded to thr + i * P * 8
+        const int64_t tstride = TP * 8;
+        if (n_c == 1) {
+            CUT(as_launch_noise_main(c->noise_cfg, d_tile, S, n, 0, n, d_tn, d_th, 0, c_values[0], (uint32_t)cut, o_thr, o_gv, o_gs,
+                                     o_cnt, o_nrec, c->exec_stream));
+            c->launches += 1;
+            if (twin_next) {
+                CUT(as_launch_noise_twins(c->noise_cfg, d_tile, S, n, 0, n, d_tn, d_th, (int32_t*)c->heads.p, (uint32_t*)c->nheads.p,
+                                          c_values[0], (uint32_t)cut, o_thr, o_gv, o_gs, o_cnt, o_nrec, c->exec_stream));
+                c->launches += 3;
+            }
+        } else {
+            const int geom = c->noise_cfg >= 7 ? c->noise_cfg - 7 : 0;
+            CUT(as_launch_noise_pattern(geom, d_tile, S, n, 0, n, d_tn, d_th, 0, c_values, n_c, (uint32_t)cut, o_thr, tstride, o_gv,
+                                        o_gs, o_cnt, o_nrec, c->exec_stream));
+            c->launches += 1;
+            if (twin_next) {  // the groups the pattern kernel leaves out (pairs cut by a CTA tile, longer chains), value by value
+                CUT(as_launch_twin_heads(7, 0, n, d_tn, d_th, (int32_t*)c->heads.p, (uint32_t*)c->nheads.p, c->exec_stream));
+                c->launches += 1;
+                for (int32_t i = 0; i < n_c; ++i) {
+                    CUT(as_launch_noise_twin_groups(d_tile, S, n, 0, n, d_tn, (const int32_t*)c->heads.p, (const uint32_t*)c->nheads.p,
+                                                    c_values[i], (uint32_t)cut, o_thr + i * tstride, o_gv, o_gs, o_cnt, o_nrec,
+                                                    c->exec_stream));
+                    c->launches += 2;
+                }
+                if (ret1 != AS_OK) break;
+            }
         }
-        CUT(cudaMemcpyAsync(thr + p0 * 8, o + lay.thr, (size_t)n * 32, cudaMemcpyDeviceToHost, c->exec_stream));
+        CUT(cudaMemcpy2DAsync(thr + p0 * 8, (size_t)P * 32, o + lay.thr, (size_t)tstride * 4, (size_t)n * 32, (size_t)n_c,
+                              cudaMemcpyDeviceToHost, c->exec_stream));
         CUT(cudaMemcpyAsync(germ_val + p0 * 4, o + lay.germ_val, (size_t)n * 16, cudaMemcpyDeviceToHost, c->exec_stream));
         CUT(cudaMemcpyAsync(count + p0 * 4, o + lay.count, (size_t)n * 16, cudaMemcpyDeviceToHost, c->exec_stream));
         CUT(cudaMemcpyAsync(nrec + p0, o + lay.nrec, (size_t)n * 4, cudaMemcpyDeviceToHost, c->exec_stream));
         CUT(cudaMemcpyAsync(germ_state + p0 * 4, o + lay.germ_state, (size_t)n * 4, cudaMemcpyDeviceToHost, c->exec_stream));
         if (thr_view) {  // the "%f" hand-over of the thresholds, while they are still on the device
-            CUT(as_launch_thr_view(o_thr, (float*)(o + lay.view), n * 8, c->exec_stream));
+            CUT(as_launch_thr_view(o_thr, (float*)(o + lay.view), (n_c - 1) * tstride + n * 8, c->exec_stream));
             c->launches += 1;
-            CUT(cudaMemcpyAsync(thr_view + p0 * 8, o + lay.view, (size_t)n * 32, cudaMemcpyDeviceToHost, c->exec_stream));
+            CUT(cudaMemcpy2DAsync(thr_view + p0 * 8, (size_t)P * 32, o + lay.view, (size_t)tstride * 4, (size_t)n * 32, (size_t)n_c,
+                                  cudaMemcpyDeviceToHost, c->exec_stream));
         }
         CUT(cudaEventRecord(c->ev_done[bsel], c->exec_stream));
     }
@@ -662,7 +688,7 @@ static int noise_estimate_host_range(as_ctx* c, const HostSrc& src, int32_t S, i
     for (int64_t smp = 0; smp < S; ++smp)
         for (int64_t m = 0; m < M; ++m)
             host_record(src, P, smp, members[m], h_gather + ((smp * 2) * M + m) * 4, h_gather + ((smp * 2 + 1) * M + m) * 4);
-    const NoiseOutLayout ml(M);
+    const NoiseOutLayout ml(M, n_c);
     DevBuf d_cnt, d_out, d_links;
     cudaError_t e1 = d_cnt.need((size_t)M * 32 * (size_t)std::max(1, S));
     cudaError_t e2 = d_out.need(ml.total);
@@ -681,23 +707,28 @@ static int noise_estimate_host_range(as_ctx* c, const HostSrc& src, int32_t S, i
         CUB(cudaMemcpyAsync(d_next, c_next.data(), (size_t)M * 4, cudaMemcpyHostToDevice, st));
         CUB(cudaMemcpyAsync(d_head, c_head.data(), (size_t)M * 4, cudaMemcpyHostToDevice, st));
         char* o = (char*)d_out.p;
-        CUB(as_launch_noise_twins(0, (const uint32_t*)d_cnt.p, S, M, 0, M, d_next, d_head, d_heads, (uint32_t*)c->nheads.p, C,
-                                  (uint32_t)cut, (float*)(o + ml.thr), (float*)(o + ml.germ_val),
-                                  (uint8_t*)(o + ml.germ_state), (uint32_t*)(o + ml.count), (uint32_t*)(o + ml.nrec), st));
-        c->launches += 3;
-        CUB(as_launch_thr_view((float*)(o + ml.thr), (float*)(o + ml.view), M * 8, st));
+        for (int32_t i = 0; i < n_c; ++i) {  // once per value; the C-independent outputs are rewritten with the same values
+            CUB(as_launch_noise_twins(0, (const uint32_t*)d_cnt.p, S, M, 0, M, d_next, d_head, d_heads, (uint32_t*)c->nheads.p,
+                                      c_values[i], (uint32_t)cut, (float*)(o + ml.thr) + i * M * 8, (float*)(o + ml.germ_val),
+                                      (uint8_t*)(o + ml.germ_state), (uint32_t*)(o + ml.count), (uint32_t*)(o + ml.nrec), st));
+            c->launches += 3;
+        }
+        if (ret != AS_OK) break;
+        CUB(as_launch_thr_view((float*)(o + ml.thr), (float*)(o + ml.view), n_c * M * 8, st));
         c->launches += 1;
         CUB(cudaMemcpyAsync(h_out.data(), o, ml.total, cudaMemcpyDeviceToHost, st));
         CUB(cudaStreamSynchronize(st));
 #undef CUB
         for (int64_t m = 0; m < M; ++m) {
             const int64_t p = members[m];
-            memcpy(thr + p * 8, h_out.data() + ml.thr + m * 32, 32);
+            for (int64_t i = 0; i < n_c; ++i) {
+                memcpy(thr + (i * P + p) * 8, h_out.data() + ml.thr + (i * M + m) * 32, 32);
+                if (thr_view) memcpy(thr_view + (i * P + p) * 8, h_out.data() + ml.view + (i * M + m) * 32, 32);
+            }
             memcpy(germ_val + p * 4, h_out.data() + ml.germ_val + m * 16, 16);
             memcpy(count + p * 4, h_out.data() + ml.count + m * 16, 16);
             memcpy(nrec + p, h_out.data() + ml.nrec + m * 4, 4);
             memcpy(germ_state + p * 4, h_out.data() + ml.germ_state + m * 4, 4);
-            if (thr_view) memcpy(thr_view + p * 8, h_out.data() + ml.view + m * 32, 32);
         }
     } while (0);
     d_cnt.release(); d_out.release(); d_links.release();
@@ -707,13 +738,13 @@ static int noise_estimate_host_range(as_ctx* c, const HostSrc& src, int32_t S, i
 // ---- caller ----------------------------------------------------------------------------------------
 // the caller as scan -> resolve -> series kernels (as_call_deferred.cu), lists in scratch owned by the context
 static int call_deferred(as_ctx* c, const uint32_t* d_counts, int32_t T, int64_t P, int64_t b, int64_t e, const uint8_t* d_ref,
-                         const float* d_thr_views, int32_t n_c, int32_t cut, as_call* d_calls, int64_t cap,
+                         const float* d_thr_views, int32_t n_c, int64_t c_stride, int32_t cut, as_call* d_calls, int64_t cap,
                          unsigned long long* d_n_calls, cudaStream_t st) {
     int64_t cap_cand = 0, cap_surv = 0;
     const size_t bytes = as_deferred_scratch_bytes(T, e - b, &cap_cand, &cap_surv) + 256;
     if (c->defer_cap_override > 0) { cap_cand = c->defer_cap_override; cap_surv = std::max<int64_t>(1, cap_cand / 4); }
     CU(c->defer.need(bytes));
-    CU(as_launch_call_deferred(d_counts, T, P, b, e, d_ref, d_thr_views, n_c, P * 8, (uint32_t)cut, d_calls, cap, d_n_calls, c->defer.p,
+    CU(as_launch_call_deferred(d_counts, T, P, b, e, d_ref, d_thr_views, n_c, c_stride, (uint32_t)cut, d_calls, cap, d_n_calls, c->defer.p,
                                cap_cand, cap_surv, st, c->aux_stream, c->ev_chunk, c->defer_chunks));
     c->launches += 3 * as_deferred_chunks(e - b, c->defer_chunks);
     return AS_OK;
@@ -728,7 +759,7 @@ int as_call_variants_dev(as_ctx* c, const uint32_t* d_counts, int32_t T, int64_t
     if (T >= (1 << 27)) return fail(AS_EINVAL, "at most 2^27-1 samples per call");
     CU(cudaSetDevice(c->device));
     if (c->call_variant == AS_DEFERRED_CALL_KERNEL)
-        return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_view, 1, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
+        return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_view, 1, P * 8, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
     CU(as_launch_call(c->call_variant, d_counts, T, P, b, e, d_ref, d_thr_view, (uint32_t)cut, d_calls, cap, d_n_calls,
                       (cudaStream_t)stream));
     c->launches += 1;
@@ -747,20 +778,23 @@ int as_call_variants_sweep_dev(as_ctx* c, const uint32_t* d_counts, int32_t T, i
     CU(cudaSetDevice(c->device));
     // default: the deferred pipeline; a staged variant selected by hand runs the in-stage sweep kernel (cross-check)
     if (c->call_variant == AS_DEFERRED_CALL_KERNEL || (c->call_variant == AS_DEFAULT_CALL_KERNEL && n_c > 1))
-        return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_views, n_c, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
+        return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_views, n_c, P * 8, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
     CU(as_launch_call_sweep(c->call_variant, d_counts, T, P, b, e, d_ref, d_thr_views, n_c, P * 8, (uint32_t)cut, d_calls, cap,
                             d_n_calls, (cudaStream_t)stream));
     c->launches += 1;
     return AS_OK;
 }
 
-// Slots [B, E) of the panel on ONE device (c is a single-device context).  The calls stay on the device, unsorted, with
-// panel slot ids, in c->calls (capacity cap); *found = the number found (may exceed cap).
+// Slots [B, E) of the panel on ONE device (c is a single-device context).  n_c threshold tables (1..8), thr_views
+// [n_c][P][4][2].  The calls stay on the device, unsorted, with panel slot ids, in c->calls: list i at i * cap;
+// found[i] = the number found for table i (may exceed cap).  n_c == 1 runs the single-table kernel; n_c > 1 runs the
+// kernel as_call_variants_sweep_dev would choose (the deferred pipeline by default, the in-stage sweep kernel when a
+// staged variant is selected).
 static int call_variants_host_range(as_ctx* c, const HostSrc& src, int32_t T, int64_t P, int64_t B, int64_t E, const uint8_t* ref,
-                                    const float* thr_view, int32_t cut, int64_t cap, int64_t* found) {
+                                    const float* thr_views, int32_t n_c, int32_t cut, int64_t cap, int64_t* found) {
     const int elem = src.elem;
     PhaseClock clk;
-    *found = 0;
+    for (int32_t i = 0; i < n_c; ++i) found[i] = 0;
     if (E <= B || T == 0) return AS_OK;
     CU(cudaSetDevice(c->device));
     const int64_t TP = tile_slots(c, T, E - B, elem);
@@ -768,19 +802,24 @@ static int call_variants_host_range(as_ctx* c, const HostSrc& src, int32_t T, in
         CU(c->tile[i].need((size_t)TP * 32 * (size_t)T));
         if (elem != 4) CU(c->tile16[i].need((size_t)TP * 8 * (size_t)elem * (size_t)T));
     }
-    // thresholds (32 B/slot) and reference bases (1 B/slot) of the range go up once, ahead of the first tile: a
-    // per-tile copy from pageable memory would stall the upload queue at every tile
-    CU(c->aux[0].need((size_t)(E - B) * 33 + 64));
+    // thresholds (n_c * 32 B/slot) and reference bases (1 B/slot) of the range go up once, ahead of the first tile: a
+    // per-tile copy from pageable memory would stall the upload queue at every tile.  Table i at d_tv_all + i * (E - B) * 8.
+    const int64_t c_stride = (E - B) * 8;
+    CU(c->aux[0].need((size_t)(E - B) * (32 * (size_t)n_c + 1) + 64));
     float* d_tv_all = (float*)c->aux[0].p;
-    uint8_t* d_rf_all = (uint8_t*)c->aux[0].p + (size_t)(E - B) * 32;
-    CU(cudaMemcpyAsync(d_tv_all, thr_view + B * 8, (size_t)(E - B) * 32, cudaMemcpyHostToDevice, c->copy_stream));
+    uint8_t* d_rf_all = (uint8_t*)c->aux[0].p + (size_t)(E - B) * 32 * (size_t)n_c;
+    CU(cudaMemcpy2DAsync(d_tv_all, (size_t)(E - B) * 32, thr_views + B * 8, (size_t)P * 32, (size_t)(E - B) * 32, (size_t)n_c,
+                         cudaMemcpyHostToDevice, c->copy_stream));
     CU(cudaMemcpyAsync(d_rf_all, ref + B, (size_t)(E - B), cudaMemcpyHostToDevice, c->copy_stream));
-    CU(c->calls.need(sizeof(as_call) * (size_t)std::max<int64_t>(cap, 1)));
-    CU(c->misc.need(32));
-    CU(c->h_small.need(64));
-    unsigned long long* d_n = (unsigned long long*)c->misc.p;  // calls found so far; d_n[1] = the count before the current tile
+    CU(c->calls.need(sizeof(as_call) * (size_t)std::max<int64_t>(cap, 1) * (size_t)n_c));
+    CU(c->misc.need(16 * 8));
+    CU(c->h_small.need(8 * 8));
+    // d_n[i] = calls of table i found so far, d_n[8 + i] = the count before the current tile
+    unsigned long long* d_n = (unsigned long long*)c->misc.p;
     unsigned long long* h_total = (unsigned long long*)c->h_small.p;
-    CU(cudaMemsetAsync(d_n, 0, 16, c->exec_stream));
+    CU(cudaMemsetAsync(d_n, 0, 16 * 8, c->exec_stream));
+    const bool sweep = n_c > 1;
+    const bool deferred = sweep && (c->call_variant == AS_DEFERRED_CALL_KERNEL || c->call_variant == AS_DEFAULT_CALL_KERNEL);
     const int64_t ntiles = (E - B + TP - 1) / TP;
     clk.lap("call.checks_alloc");
     CU(stage_wide(c, src, c->copy_stream));
@@ -795,27 +834,38 @@ static int call_variants_host_range(as_ctx* c, const HostSrc& src, int32_t T, in
         CUB(cudaEventRecord(c->ev_up[bsel], c->copy_stream));
         CUB(cudaStreamWaitEvent(c->exec_stream, c->ev_up[bsel], 0));
         CUB(expand_tile(c, bsel, src, T, p0, n, c->exec_stream));
-        // the tile kernel emits tile-local slot ids; the entries it appended, [d_n[1], d_n[0]), get the tile offset
-        if (p0 > 0) CUB(cudaMemcpyAsync(d_n + 1, d_n, 8, cudaMemcpyDeviceToDevice, c->exec_stream));
-        CUB(as_launch_call(c->call_variant, (const uint32_t*)c->tile[bsel].p, T, n, 0, n, d_rf_all + (p0 - B), d_tv_all + (p0 - B) * 8,
-                           (uint32_t)cut, (as_call*)c->calls.p, cap, d_n, c->exec_stream));
-        c->launches += 1;
-        if (p0 > 0) {
-            CUB(as_launch_call_slot_offset((as_call*)c->calls.p, d_n + 1, d_n, cap, (int32_t)p0, c->exec_stream));
+        // the tile kernel emits tile-local slot ids; the entries it appended, [d_n[8 + i], d_n[i]), get the tile offset
+        if (p0 > 0) CUB(cudaMemcpyAsync(d_n + 8, d_n, 8 * (size_t)n_c, cudaMemcpyDeviceToDevice, c->exec_stream));
+        const uint32_t* d_tile = (const uint32_t*)c->tile[bsel].p;
+        if (deferred) {
+            if ((ret = call_deferred(c, d_tile, T, n, 0, n, d_rf_all + (p0 - B), d_tv_all + (p0 - B) * 8, n_c, c_stride, cut,
+                                     (as_call*)c->calls.p, cap, d_n, c->exec_stream)) != AS_OK)
+                break;
+        } else {
+            CUB(as_launch_call_sweep(c->call_variant, d_tile, T, n, 0, n, d_rf_all + (p0 - B), d_tv_all + (p0 - B) * 8, n_c, c_stride,
+                                     (uint32_t)cut, (as_call*)c->calls.p, cap, d_n, c->exec_stream));
             c->launches += 1;
+        }
+        if (p0 > 0) {
+            for (int32_t i = 0; i < n_c; ++i) {
+                CUB(as_launch_call_slot_offset((as_call*)c->calls.p + i * cap, d_n + 8 + i, d_n + i, cap, (int32_t)p0, c->exec_stream));
+                c->launches += 1;
+            }
+            if (ret != AS_OK) break;
         }
         CUB(cudaEventRecord(c->ev_done[bsel], c->exec_stream));
 #undef CUB
     }
     clk.lap("call.enqueue");
     if (ret == AS_OK) {
-        cudaError_t e0 = cudaMemcpyAsync(h_total, d_n, 8, cudaMemcpyDeviceToHost, c->exec_stream);
+        cudaError_t e0 = cudaMemcpyAsync(h_total, d_n, 8 * (size_t)n_c, cudaMemcpyDeviceToHost, c->exec_stream);
         cudaError_t e1 = cudaStreamSynchronize(c->exec_stream), e2 = cudaStreamSynchronize(c->copy_stream);
         clk.lap("call.drain");
         if (e0 != cudaSuccess || e1 != cudaSuccess || e2 != cudaSuccess)
             ret = fail(AS_ECUDA, "caller pipeline failed: %s", cudaGetErrorString(e0 != cudaSuccess ? e0 : e1 != cudaSuccess ? e1 : e2));
     }
-    if (ret == AS_OK) *found = (int64_t)*h_total;
+    if (ret == AS_OK)
+        for (int32_t i = 0; i < n_c; ++i) found[i] = (int64_t)h_total[i];
     return ret;
 }
 
@@ -887,8 +937,9 @@ static int run_on_devices(as_ctx* c, F body) {  // body(k, sub-context) on one h
 extern "C" {
 
 static int noise_estimate_host_impl(as_ctx* c, const HostSrc& src, int32_t S, int64_t P, const int32_t* twin_next,
-                                    const int32_t* twin_head, float C, int32_t cut, float* thr, float* germ_val,
-                                    uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
+                                    const int32_t* twin_head, const float* c_values, int32_t n_c, int32_t cut, float* thr,
+                                    float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
+    if (!c_values || n_c < 1 || n_c > 8) return fail(AS_EINVAL, "a sweep takes 1..8 values of C");
     int rc = check_common(c, src.counts, S, P, 0, P, cut);
     if (rc) return rc;
     if ((rc = check_wide(src, S, P)) != AS_OK) return rc;
@@ -896,65 +947,93 @@ static int noise_estimate_host_impl(as_ctx* c, const HostSrc& src, int32_t S, in
     if ((twin_next == nullptr) != (twin_head == nullptr)) return fail(AS_EINVAL, "twin_next and twin_head go together");
     if (P == 0) return AS_OK;
     if (c->subs.size() < 2)
-        return noise_estimate_host_range(c, src, S, P, 0, P, twin_next, twin_head, C, cut, thr, germ_val, germ_state, count, nrec, thr_view);
+        return noise_estimate_host_range(c, src, S, P, 0, P, twin_next, twin_head, c_values, n_c, cut, thr, germ_val, germ_state, count,
+                                         nrec, thr_view);
     const std::vector<int64_t> bounds = shard_bounds(P, (int)c->subs.size(), twin_next, twin_head);
     return run_on_devices(c, [&](int k, as_ctx* sub, ShardResult&) {
-        return noise_estimate_host_range(sub, src, S, P, bounds[(size_t)k], bounds[(size_t)k + 1], twin_next, twin_head, C, cut, thr,
-                                         germ_val, germ_state, count, nrec, thr_view);
+        return noise_estimate_host_range(sub, src, S, P, bounds[(size_t)k], bounds[(size_t)k + 1], twin_next, twin_head, c_values, n_c,
+                                         cut, thr, germ_val, germ_state, count, nrec, thr_view);
     });
 }
 
+// n_c tables: calls [n_c][cap], n_calls [n_c].  Each table's lists of all devices meet on the first one (peer copies of
+// exact sizes), are sorted there into the reference's row order (sample, slot, alt), one radix sort per table, and come
+// down with one copy per table.
 static int call_variants_host_impl(as_ctx* c, const HostSrc& src, int32_t T, int64_t P, const uint8_t* ref,
-                                   const float* thr_view, int32_t cut, as_call* calls, int64_t cap, int64_t* n_calls) {
+                                   const float* thr_views, int32_t n_c, int32_t cut, as_call* calls, int64_t cap, int64_t* n_calls) {
     PhaseClock clk;
+    if (n_c < 1 || n_c > 8) return fail(AS_EINVAL, "a sweep takes 1..8 threshold tables");
     int rc = check_common(c, src.counts, T, P, 0, P, cut);
     if (rc) return rc;
     if ((rc = check_wide(src, T, P)) != AS_OK) return rc;
-    if (!ref || !thr_view || !n_calls || (!calls && cap > 0) || cap < 0) return fail(AS_EINVAL, "bad pointer / cap");
-    *n_calls = 0;
+    if (!ref || !thr_views || !n_calls || (!calls && cap > 0) || cap < 0) return fail(AS_EINVAL, "bad pointer / cap");
+    if (c->call_variant < 2 && n_c > 1) return fail(AS_EINVAL, "the sweep needs a TMA-staged caller variant (>= 2)");
+    for (int32_t i = 0; i < n_c; ++i) n_calls[i] = 0;
     if (P == 0 || T == 0) return AS_OK;
     const int ndev = c->subs.size() < 2 ? 1 : (int)c->subs.size();
-    std::vector<int64_t> found((size_t)ndev, 0);
+    std::vector<int64_t> found((size_t)ndev * 8, 0);  // found[k * 8 + i]: device k, table i
     if (ndev == 1) {
-        rc = call_variants_host_range(c, src, T, P, 0, P, ref, thr_view, cut, cap, &found[0]);
+        rc = call_variants_host_range(c, src, T, P, 0, P, ref, thr_views, n_c, cut, cap, &found[0]);
     } else {
         const std::vector<int64_t> bounds = shard_bounds(P, ndev, nullptr, nullptr);
         rc = run_on_devices(c, [&](int k, as_ctx* sub, ShardResult&) {
-            return call_variants_host_range(sub, src, T, P, bounds[(size_t)k], bounds[(size_t)k + 1], ref, thr_view, cut, cap,
-                                            &found[(size_t)k]);
+            return call_variants_host_range(sub, src, T, P, bounds[(size_t)k], bounds[(size_t)k + 1], ref, thr_views, n_c, cut, cap,
+                                            &found[(size_t)k * 8]);
         });
     }
     if (rc != AS_OK) return rc;
-    // the lists of all devices meet on the first one (peer copies of exact sizes), are sorted there into the reference's
-    // row order (sample, slot, alt) and come down in one copy
     CU(cudaSetDevice(c->device));
-    int64_t total = 0, have = 0;
-    for (int k = 0; k < ndev; ++k) { total += found[(size_t)k]; have += std::min(found[(size_t)k], cap); }
-    *n_calls = total;
-    const int64_t keep = std::min(have, cap);
-    if (have > 0) {
-        const size_t scratch = as_sort_calls_scratch_bytes(have), list = ((size_t)have * sizeof(as_call) + 255) & ~(size_t)255;
-        CU(c->sortbuf.need(2 * list + scratch));
-        as_call* gathered = (as_call*)c->calls.p;
-        if (ndev > 1) {
-            gathered = (as_call*)((char*)c->sortbuf.p + list + scratch);
-            int64_t off = 0;
-            for (int k = 0; k < ndev; ++k) {
-                const int64_t n = std::min(found[(size_t)k], cap);
-                if (n > 0) CU(cudaMemcpyPeerAsync(gathered + off, c->device, c->subs[(size_t)k]->calls.p, c->subs[(size_t)k]->device,
-                                                  sizeof(as_call) * (size_t)n, c->exec_stream));
-                off += n;
-            }
+    std::vector<int64_t> have((size_t)n_c, 0);
+    int64_t max_have = 0, sum_list = 0;
+    bool over = false;
+    for (int32_t i = 0; i < n_c; ++i) {
+        int64_t total = 0;
+        for (int k = 0; k < ndev; ++k) {
+            const int64_t f = found[(size_t)k * 8 + i];
+            total += f;
+            have[(size_t)i] += std::min(f, cap);
+            over = over || f > cap;
         }
-        CU(as_launch_sort_calls(gathered, have, (as_call*)c->sortbuf.p, (char*)c->sortbuf.p + list, scratch, c->exec_stream));
-        c->launches += 3;
-        CU(cudaMemcpyAsync(calls, c->sortbuf.p, sizeof(as_call) * (size_t)keep, cudaMemcpyDeviceToHost, c->exec_stream));
+        n_calls[i] = total;
+        over = over || total > cap;
+        max_have = std::max(max_have, have[(size_t)i]);
+        sum_list += (int64_t)(((size_t)have[(size_t)i] * sizeof(as_call) + 255) & ~(size_t)255);
+    }
+    if (max_have > 0) {
+        // sortbuf: sorted lists of every table | sort scratch | gathered list of one table (several devices)
+        const size_t scratch = as_sort_calls_scratch_bytes(max_have);
+        const size_t gather = ndev > 1 ? (size_t)max_have * sizeof(as_call) : 0;
+        CU(c->sortbuf.need((size_t)sum_list + scratch + gather));
+        char* sorted = (char*)c->sortbuf.p;
+        char* sort_scratch = sorted + sum_list;
+        for (int32_t i = 0; i < n_c; ++i) {
+            const int64_t h = have[(size_t)i];
+            if (h == 0) continue;
+            as_call* gathered = (as_call*)c->calls.p + i * cap;
+            if (ndev > 1) {
+                gathered = (as_call*)(sort_scratch + scratch);
+                int64_t off = 0;
+                for (int k = 0; k < ndev; ++k) {
+                    const int64_t n = std::min(found[(size_t)k * 8 + i], cap);
+                    if (n > 0) CU(cudaMemcpyPeerAsync(gathered + off, c->device, (as_call*)c->subs[(size_t)k]->calls.p + i * cap,
+                                                      c->subs[(size_t)k]->device, sizeof(as_call) * (size_t)n, c->exec_stream));
+                    off += n;
+                }
+            }
+            CU(as_launch_sort_calls(gathered, h, (as_call*)sorted, sort_scratch, scratch, c->exec_stream));
+            c->launches += 3;
+            CU(cudaMemcpyAsync(calls + i * cap, sorted, sizeof(as_call) * (size_t)std::min(h, cap), cudaMemcpyDeviceToHost,
+                               c->exec_stream));
+            sorted += ((size_t)h * sizeof(as_call) + 255) & ~(size_t)255;
+        }
         CU(cudaStreamSynchronize(c->exec_stream));
         clk.lap("call.sort_download");
     }
-    bool over = total > cap;
-    for (int k = 0; k < ndev; ++k) over = over || found[(size_t)k] > cap;
-    if (over) return fail(AS_EOVERFLOW, "%lld calls found, capacity %lld", (long long)total, (long long)cap);
+    if (over) {
+        int32_t worst = 0;
+        for (int32_t i = 1; i < n_c; ++i) if (n_calls[i] > n_calls[worst]) worst = i;
+        return fail(AS_EOVERFLOW, "%lld calls found, capacity %lld", (long long)n_calls[worst], (long long)cap);
+    }
     return AS_OK;
 }
 
@@ -962,31 +1041,31 @@ int as_noise_estimate_host(as_ctx* c, const uint32_t* counts, int32_t S, int64_t
                            const int32_t* twin_head, float C, int32_t cut, float* thr, float* germ_val,
                            uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
     const HostSrc src{counts, 4, nullptr, 0};
-    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, C, cut, thr, germ_val, germ_state, count, nrec, thr_view);
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, &C, 1, cut, thr, germ_val, germ_state, count, nrec, thr_view);
 }
 int as_noise_estimate_host16(as_ctx* c, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t S,
                              int64_t P, const int32_t* twin_next, const int32_t* twin_head, float C, int32_t cut, float* thr,
                              float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
     const HostSrc src{counts, 2, wide, n_wide};
-    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, C, cut, thr, germ_val, germ_state, count, nrec, thr_view);
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, &C, 1, cut, thr, germ_val, germ_state, count, nrec, thr_view);
 }
 int as_call_variants_host(as_ctx* c, const uint32_t* counts, int32_t T, int64_t P, const uint8_t* ref,
                           const float* thr_view, int32_t cut, as_call* calls, int64_t cap, int64_t* n_calls) {
     const HostSrc src{counts, 4, nullptr, 0};
-    return call_variants_host_impl(c, src, T, P, ref, thr_view, cut, calls, cap, n_calls);
+    return call_variants_host_impl(c, src, T, P, ref, thr_view, 1, cut, calls, cap, n_calls);
 }
 int as_noise_estimate_host_packed(as_ctx* c, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t S,
                                   int64_t P, const int32_t* twin_next, const int32_t* twin_head, float C, int32_t cut,
                                   float* thr, float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec,
                                   float* thr_view) {
     const HostSrc src{packed, 1, wide, n_wide};
-    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, C, cut, thr, germ_val, germ_state, count, nrec, thr_view);
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, &C, 1, cut, thr, germ_val, germ_state, count, nrec, thr_view);
 }
 int as_call_variants_host_packed(as_ctx* c, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T,
                                  int64_t P, const uint8_t* ref, const float* thr_view, int32_t cut, as_call* calls,
                                  int64_t cap, int64_t* n_calls) {
     const HostSrc src{packed, 1, wide, n_wide};
-    return call_variants_host_impl(c, src, T, P, ref, thr_view, cut, calls, cap, n_calls);
+    return call_variants_host_impl(c, src, T, P, ref, thr_view, 1, cut, calls, cap, n_calls);
 }
 
 // uint32 counts -> packed wire format + escaped records.  Threads over samples; the per-sample lists are concatenated
@@ -1039,7 +1118,49 @@ int as_call_variants_host16(as_ctx* c, const uint16_t* counts, const as_wide_rec
                             int64_t P, const uint8_t* ref, const float* thr_view, int32_t cut, as_call* calls, int64_t cap,
                             int64_t* n_calls) {
     const HostSrc src{counts, 2, wide, n_wide};
-    return call_variants_host_impl(c, src, T, P, ref, thr_view, cut, calls, cap, n_calls);
+    return call_variants_host_impl(c, src, T, P, ref, thr_view, 1, cut, calls, cap, n_calls);
+}
+
+// Noise-floor sweep on the _host path: n_c values of C / n_c threshold tables through the same pipelines
+int as_noise_estimate_sweep_host(as_ctx* c, const uint32_t* counts, int32_t S, int64_t P, const int32_t* twin_next,
+                                 const int32_t* twin_head, const float* c_values, int32_t n_c, int32_t cut, float* thr,
+                                 float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view) {
+    const HostSrc src{counts, 4, nullptr, 0};
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, c_values, n_c, cut, thr, germ_val, germ_state, count, nrec,
+                                    thr_view);
+}
+int as_noise_estimate_sweep_host16(as_ctx* c, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t S,
+                                   int64_t P, const int32_t* twin_next, const int32_t* twin_head, const float* c_values,
+                                   int32_t n_c, int32_t cut, float* thr, float* germ_val, uint8_t* germ_state, uint32_t* count,
+                                   uint32_t* nrec, float* thr_view) {
+    const HostSrc src{counts, 2, wide, n_wide};
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, c_values, n_c, cut, thr, germ_val, germ_state, count, nrec,
+                                    thr_view);
+}
+int as_noise_estimate_sweep_host_packed(as_ctx* c, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t S,
+                                        int64_t P, const int32_t* twin_next, const int32_t* twin_head, const float* c_values,
+                                        int32_t n_c, int32_t cut, float* thr, float* germ_val, uint8_t* germ_state,
+                                        uint32_t* count, uint32_t* nrec, float* thr_view) {
+    const HostSrc src{packed, 1, wide, n_wide};
+    return noise_estimate_host_impl(c, src, S, P, twin_next, twin_head, c_values, n_c, cut, thr, germ_val, germ_state, count, nrec,
+                                    thr_view);
+}
+int as_call_variants_sweep_host(as_ctx* c, const uint32_t* counts, int32_t T, int64_t P, const uint8_t* ref,
+                                const float* thr_views, int32_t n_c, int32_t cut, as_call* calls, int64_t cap, int64_t* n_calls) {
+    const HostSrc src{counts, 4, nullptr, 0};
+    return call_variants_host_impl(c, src, T, P, ref, thr_views, n_c, cut, calls, cap, n_calls);
+}
+int as_call_variants_sweep_host16(as_ctx* c, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t T,
+                                  int64_t P, const uint8_t* ref, const float* thr_views, int32_t n_c, int32_t cut, as_call* calls,
+                                  int64_t cap, int64_t* n_calls) {
+    const HostSrc src{counts, 2, wide, n_wide};
+    return call_variants_host_impl(c, src, T, P, ref, thr_views, n_c, cut, calls, cap, n_calls);
+}
+int as_call_variants_sweep_host_packed(as_ctx* c, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T,
+                                       int64_t P, const uint8_t* ref, const float* thr_views, int32_t n_c, int32_t cut,
+                                       as_call* calls, int64_t cap, int64_t* n_calls) {
+    const HostSrc src{packed, 1, wide, n_wide};
+    return call_variants_host_impl(c, src, T, P, ref, thr_views, n_c, cut, calls, cap, n_calls);
 }
 
 // Device call list -> the reference's row order (sample, slot, alt), on the device (radix sort of 64-bit keys + row gather).

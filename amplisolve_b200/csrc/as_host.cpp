@@ -1565,6 +1565,37 @@ int as_error_estimation_main(int argc, char** argv) {
     const std::string default_error = arg_value(argv[6], "default_error=");
     const std::string output_dir = arg_value(argv[7], "output_dir=");
     float C_value_float = (float)atof(C_value.c_str());  // EE:329
+    // C_value=a,b,c: a noise-floor sweep, one table per value from one parse of the normals.  Every element is converted
+    // like a single value (atof, <= 0 -> 0.002); a value without a comma takes the single-value path unchanged.
+    const bool sweep = C_value.find(',') != std::string::npos;
+    std::vector<std::string> c_texts;
+    std::vector<float> c_values;
+    if (sweep) {
+        for (size_t b = 0;;) {
+            const size_t e = C_value.find(',', b);
+            c_texts.push_back(C_value.substr(b, e == std::string::npos ? std::string::npos : e - b));
+            if (e == std::string::npos) break;
+            b = e + 1;
+        }
+        std::vector<std::string> names;
+        for (const std::string& t : c_texts) {
+            if (t.empty()) {
+                std::cout << "Error: C_value=" << C_value << " has an empty value" << std::endl;
+                return 0;
+            }
+            float v = (float)atof(t.c_str());
+            if (v <= 0) v = 0.002f;
+            char name[64];
+            snprintf(name, sizeof name, "%.4f", v);
+            if (std::find(names.begin(), names.end(), name) != names.end()) {
+                std::cout << "Error: C_value=" << C_value << ": " << t << " gives positionSpecificNoise_" << name
+                          << ".txt a second time" << std::endl;
+                return 0;
+            }
+            names.push_back(name);
+            c_values.push_back(v);
+        }
+    }
     int cut = atoi(coverage_cutoff.c_str());
     const bool with_germlines = germline_dir != "not_available";  // EE:349
     float default_error_float = 0.01f;
@@ -1590,7 +1621,17 @@ int as_error_estimation_main(int argc, char** argv) {
     } else {
         std::cout << "\t3. Germline count dir                             : " << GREEN << germline_dir << RESET << std::endl;
     }
-    if (C_value_float <= 0) {
+    if (sweep) {
+        std::cout << "\t4. C values                                       : " << GREEN;
+        for (size_t i = 0; i < c_values.size(); ++i) {
+            if (i) std::cout << ",";
+            std::cout << c_values[i];
+        }
+        std::cout << RESET;
+        for (size_t i = 0; i < c_values.size(); ++i)
+            if ((float)atof(c_texts[i].c_str()) <= 0) std::cout << ". User gave: " << c_texts[i] << ", converted to 0.002";
+        std::cout << std::endl;
+    } else if (C_value_float <= 0) {
         C_value_float = 0.002f;  // EE:372-376
         std::cout << "\t4. C value                                         : " << RED << "User gave: " << C_value << RESET
                   << ". The value is converted to 0.002" << std::endl;
@@ -1735,27 +1776,35 @@ int as_error_estimation_main(int argc, char** argv) {
     std::vector<int32_t> links_next, links_head;
     const int64_t PS = add_spill_slots(panel, counts, stats, links_next, links_head);  // P + spill slots for rows beyond the panel's slots
     if (PS < 0) return report_gpu_error("pinned host allocation");
-    std::vector<float> thr((size_t)PS * 8), germ_val((size_t)PS * 4);
+    if (!sweep) c_values.assign(1, C_value_float);
+    const size_t n_tables = c_values.size();
+    std::vector<float> thr(n_tables * (size_t)PS * 8), germ_val((size_t)PS * 4);
     std::vector<uint8_t> germ_state((size_t)PS * 4);
     std::vector<uint32_t> count((size_t)PS * 4), nrec((size_t)PS);
     const bool linked = panel.has_twins || PS > P;
     const int32_t* tn = linked ? links_next.data() : nullptr;
     const int32_t* th = linked ? links_head.data() : nullptr;
-    const int rc = counts.fmt == 2
-                       ? as_noise_estimate_host16(ctx, (const uint16_t*)counts.p, counts.wide.data(), (int64_t)counts.wide.size(),
-                                                  S, PS, tn, th, C_value_float, cut, thr.data(), germ_val.data(),
-                                                  germ_state.data(), count.data(), nrec.data(), nullptr)
-                       : as_noise_estimate_host_packed(ctx, (const uint32_t*)counts.p, counts.wide.data(),
-                                                       (int64_t)counts.wide.size(), S, PS, tn, th, C_value_float, cut, thr.data(),
-                                                       germ_val.data(), germ_state.data(), count.data(), nrec.data(), nullptr);
-    if (rc != AS_OK) return report_gpu_error("as_noise_estimate_host");
-    timer.lap("noise_model_gpu", (double)P, "positions");
+    for (size_t c0 = 0; c0 < n_tables; c0 += 8) {  // at most 8 values of C per pass over the normals
+        const int32_t nc = (int32_t)std::min<size_t>(8, n_tables - c0);
+        float* thr_c = thr.data() + c0 * (size_t)PS * 8;
+        const int rc = counts.fmt == 2
+                           ? as_noise_estimate_sweep_host16(ctx, (const uint16_t*)counts.p, counts.wide.data(), (int64_t)counts.wide.size(),
+                                                            S, PS, tn, th, &c_values[c0], nc, cut, thr_c, germ_val.data(),
+                                                            germ_state.data(), count.data(), nrec.data(), nullptr)
+                           : as_noise_estimate_sweep_host_packed(ctx, (const uint32_t*)counts.p, counts.wide.data(),
+                                                                 (int64_t)counts.wide.size(), S, PS, tn, th, &c_values[c0], nc, cut,
+                                                                 thr_c, germ_val.data(), germ_state.data(), count.data(), nrec.data(),
+                                                                 nullptr);
+        if (rc != AS_OK) return report_gpu_error("as_noise_estimate_host");
+    }
+    timer.lap("noise_model_gpu", (double)P * (double)n_tables, "positions");
     std::cout << "thresholds for " << panel.n_positions << " positions estimated on the GPU" << std::endl;
 
-    // generateFinalOutput (EE:2546-2944)
+    // generateFinalOutput (EE:2546-2944), one table per value of C
     char out_name[4096];
-    snprintf(out_name, sizeof out_name, "%s/positionSpecificNoise_%.4f.txt", output_dir.c_str(), C_value_float);
-    {
+    for (size_t ti = 0; ti < n_tables; ++ti) {
+        snprintf(out_name, sizeof out_name, "%s/positionSpecificNoise_%.4f.txt", output_dir.c_str(), c_values[ti]);
+        const float* thr_t = thr.data() + ti * (size_t)PS * 8;
         // rows are formatted in chunks on all host threads (2 M rows took 2.7 s on one: "%f" eight times a row) and written
         // in order; the bytes are what the reference's streams produce: "%f" (EE:1787), operator<<(double) = "%g" (EE:2815)
         std::ofstream output(out_name);
@@ -1783,7 +1832,7 @@ int as_error_estimation_main(int argc, char** argv) {
                         o += panel.ref[i];
                         o += panel.dup[i] ? "\tYES" : "\tNO";
                         for (int b = 0; b < 4; ++b) {
-                            const float tf = thr[(size_t)i * 8 + b * 2], tb = thr[(size_t)i * 8 + b * 2 + 1];
+                            const float tf = thr_t[(size_t)i * 8 + b * 2], tb = thr_t[(size_t)i * 8 + b * 2 + 1];
                             if (panel.ref[i].size() == 1 && panel.ref[i][0] == L[b]) {
                                 o += "\t-2_-2";  // EE:2668-2673
                             } else if (std::isnan(tf) || std::isnan(tb)) {
@@ -1817,11 +1866,20 @@ int as_error_estimation_main(int argc, char** argv) {
             for (size_t k = 0; k < wn; ++k) output.write(text[k].data(), (std::streamsize)text[k].size());
         }
     }
-    timer.lap("write_noise_table", (double)P, "rows");
+    timer.lap("write_noise_table", (double)P * (double)n_tables, "rows");
     char msg_name[4096];
-    snprintf(msg_name, sizeof msg_name, "%s/positionSpecific_%.4f.txt", output_dir.c_str(), C_value_float);  // sic, EE:458
-    std::cout << "\nAmpliSolveErrorEstimation execution was successful. Results can be found at: " << YELLOW << msg_name << RESET
-              << std::endl;
+    if (sweep) {
+        std::cout << "\nAmpliSolveErrorEstimation execution was successful. Results can be found at:";
+        for (const float v : c_values) {
+            snprintf(msg_name, sizeof msg_name, "%s/positionSpecificNoise_%.4f.txt", output_dir.c_str(), v);
+            std::cout << " " << YELLOW << msg_name << RESET;
+        }
+        std::cout << std::endl;
+    } else {
+        snprintf(msg_name, sizeof msg_name, "%s/positionSpecific_%.4f.txt", output_dir.c_str(), C_value_float);  // sic, EE:458
+        std::cout << "\nAmpliSolveErrorEstimation execution was successful. Results can be found at: " << YELLOW << msg_name << RESET
+                  << std::endl;
+    }
     std::cout << "\n" << STARS << std::endl;
     return 0;
 }
@@ -2008,9 +2066,39 @@ int as_variant_calling_main(int argc, char** argv) {
                   << RESET << std::endl;
     std::cout << std::endl;
 
-    const std::string interm = output_dir + "/AmpliSolveVariantCalling_interm_files";
-    if (!make_dir(interm)) {
-        std::cout << "Error: cannot create " << interm << std::endl;
+    // errorFile=<directory>: a noise-floor sweep over every positionSpecificNoise_*.txt in it, in name order.  Table X.txt
+    // writes to <output_dir>/X/ what errorFile=<directory>/X.txt output_dir=<output_dir>/X writes alone; the tumours are
+    // parsed (or piled up) once and go through the caller once per pass of up to 8 tables.
+    std::vector<std::string> table_paths, out_dirs;
+    struct stat est;
+    const bool sweep = stat(error_file.c_str(), &est) == 0 && S_ISDIR(est.st_mode);
+    if (sweep) {
+        std::vector<std::string> names;
+        if (DIR* d = opendir(error_file.c_str())) {
+            const std::string pre = "positionSpecificNoise_";
+            while (dirent* de = readdir(d)) {
+                const std::string n = de->d_name;
+                if (n.size() > pre.size() + 4 && n.compare(0, pre.size(), pre) == 0 && ends_with(n, ".txt")) names.push_back(n);
+            }
+            closedir(d);
+        }
+        std::sort(names.begin(), names.end());
+        if (names.empty()) {
+            printf("Error from storeInputFile function: Cannot open %s\n", error_file.c_str());
+            return 0;
+        }
+        for (const std::string& n : names) {
+            table_paths.push_back(error_file + "/" + n);
+            out_dirs.push_back(output_dir + "/" + n.substr(0, n.size() - 4));
+        }
+    } else {
+        table_paths.push_back(error_file);
+        out_dirs.push_back(output_dir);
+    }
+    const size_t NT = table_paths.size();
+    const std::string interm_name = "/AmpliSolveVariantCalling_interm_files";
+    if (!sweep && !make_dir(output_dir + interm_name)) {  // a sweep creates its directories once the tables agree
+        std::cout << "Error: cannot create " << output_dir + interm_name << std::endl;
         return 0;
     }
 
@@ -2019,19 +2107,48 @@ int as_variant_calling_main(int argc, char** argv) {
     PhaseTimer timer;
     // ---- noise table (storeInputFile, VC:430-576): one slot per row; also re-emits the dummy VCF (VC:564)
     Panel panel;
-    std::vector<float> thr_view;              // [P][4][2] through std::stof (VC:889-890)
-    std::vector<std::string> germ_text;       // [P][4]
-    {
+    std::vector<float> thr_view;                         // [NT][P][4][2] through std::stof (VC:889-890)
+    std::vector<std::vector<std::string>> germ_texts(NT);  // [NT][P][4]
+    std::vector<std::vector<std::string>> dummy_pieces(NT);  // dummyVCF_1.vcf (VC:564) of every table
+    for (size_t k = 0; k < NT; ++k) {
         std::string text;
-        if (!read_file(error_file, text)) {
-            printf("Error from storeInputFile function: Cannot open %s\n", error_file.c_str());
+        if (!read_file(table_paths[k], text)) {
+            printf("Error from storeInputFile function: Cannot open %s\n", table_paths[k].c_str());
             return 0;
         }
-        std::vector<std::string> dummy_pieces;  // dummyVCF_1.vcf (VC:564)
-        parse_noise_table(text, 0, panel, thr_view, germ_text, dummy_pieces);
-        std::ofstream dummy((interm + "/dummyVCF_1.vcf").c_str());
-        for (const std::string& d : dummy_pieces) dummy.write(d.data(), (std::streamsize)d.size());
+        if (k == 0) {
+            parse_noise_table(text, 0, panel, thr_view, germ_texts[0], dummy_pieces[0]);
+            continue;
+        }
+        // the tables of a sweep must describe the same panel; their thresholds and Germ_Max cells may differ
+        Panel pk;
+        std::vector<float> tv;
+        parse_noise_table(text, 0, pk, tv, germ_texts[k], dummy_pieces[k]);
+        const size_t rows = panel.slot_pos.size(), rows_k = pk.slot_pos.size();
+        size_t bad = std::min(rows, rows_k);
+        for (size_t r = 0; r < std::min(rows, rows_k); ++r)
+            if (panel.chroms[(size_t)panel.slot_chrom[r]] != pk.chroms[(size_t)pk.slot_chrom[r]] || panel.pos_text[r] != pk.pos_text[r] ||
+                panel.ref[r] != pk.ref[r] || panel.dup[r] != pk.dup[r]) {
+                bad = r;
+                break;
+            }
+        if (bad < std::max(rows, rows_k)) {
+            printf("Error from storeInputFile function: %s line %zu does not describe the panel of %s\n", table_paths[k].c_str(),
+                   bad + 2, table_paths[0].c_str());
+            return 0;
+        }
+        thr_view.insert(thr_view.end(), tv.begin(), tv.end());
     }
+    for (size_t k = 0; k < NT; ++k) {
+        const std::string interm = out_dirs[k] + interm_name;
+        if (sweep && !make_dir(interm)) {
+            std::cout << "Error: cannot create " << interm << std::endl;
+            return 0;
+        }
+        std::ofstream dummy((interm + "/dummyVCF_1.vcf").c_str());
+        for (const std::string& d : dummy_pieces[k]) dummy.write(d.data(), (std::streamsize)d.size());
+    }
+    dummy_pieces.clear();
     panel.link();
     const int64_t P = panel.size();
     // rows of a duplicated position: the hashes keep the FIRST row's reference, thresholds, Germ_Max (insert does
@@ -2047,8 +2164,12 @@ int as_variant_calling_main(int argc, char** argv) {
         if (h != (int32_t)i) {
             panel.dup[i] = panel.dup[h];
             panel.ref[i] = panel.ref[h];
-            for (int k = 0; k < 8; ++k) thr_view[(size_t)i * 8 + k] = thr_view[(size_t)h * 8 + k];
-            for (int k = 0; k < 4; ++k) germ_text[(size_t)i * 4 + k] = germ_text[(size_t)h * 4 + k];
+            for (size_t t = 0; t < NT; ++t) {
+                float* tv = thr_view.data() + t * (size_t)P * 8;
+                std::vector<std::string>& gt = germ_texts[t];
+                for (int k = 0; k < 8; ++k) tv[(size_t)i * 8 + k] = tv[(size_t)h * 8 + k];
+                for (int k = 0; k < 4; ++k) gt[(size_t)i * 4 + k] = gt[(size_t)h * 4 + k];
+            }
         }
     }
     std::cout << "Running function storeInputFile: the error levels have stored with success " << P << RESET << std::endl;
@@ -2072,8 +2193,9 @@ int as_variant_calling_main(int argc, char** argv) {
         std::cout << "Error: cannot list " << tumour_dir << "/*.ASEQ" << std::endl;
         return 0;
     }
-    const std::string list_name = interm + "/" + std::to_string(seed) + "_tumour_count_list_original.txt";
-    write_list_file(list_name, listed);
+    const std::string list_tail = interm_name + "/" + std::to_string(seed) + "_tumour_count_list_original.txt";
+    for (size_t k = 0; k < NT; ++k) write_list_file(out_dirs[k] + list_tail, listed);
+    const std::string list_name = out_dirs[0] + list_tail;
     std::cout << "\nRunning function storeList: " << GREEN << list_name << RESET << " stored with success. It contains " << GREEN
               << files.size() << RESET << " samples" << std::endl;
     const int T = (int)files.size();
@@ -2101,10 +2223,13 @@ int as_variant_calling_main(int argc, char** argv) {
     // download) the host threads parse the next one into the other pinned buffer, so pinned memory is two groups, not
     // the whole run, and the text parse hides behind the GPU step (or the other way round)
     struct CallCounts { uint32_t fw[4], bw[4]; };  // the record of a call, kept for the Fisher test and the writers
-    std::vector<as_call> calls;
-    std::vector<CallCounts> call_counts;
-    std::vector<int32_t> call_row;     // file row of a call that came from a row beyond its position's slots (-1: see slot_of_row)
-    std::vector<long long> call_rd;    // RD column of the call's row where it is not A+C+G+T (-1: the sum); VC:814-817 divide by the column
+    struct TableCalls {  // the calls of one noise table
+        std::vector<as_call> calls;
+        std::vector<CallCounts> call_counts;
+        std::vector<int32_t> call_row;   // file row of a call that came from a row beyond its position's slots (-1: see slot_of_row)
+        std::vector<long long> call_rd;  // RD column of the call's row where it is not A+C+G+T (-1: the sum); VC:814-817 divide by the column
+    };
+    std::vector<TableCalls> per_table(NT);
     std::vector<AseqStats> file_stats((size_t)T);  // order information of every file (slot_of_row only when out of order)
     double total_rows = 0, parse_s = 0, gpu_s = 0;
     if (T > 0 && P > 0) {
@@ -2138,24 +2263,32 @@ int as_variant_calling_main(int argc, char** argv) {
                 total_rows += (double)stats[which][(size_t)i].rows;
                 file_stats[(size_t)(first + i)] = std::move(stats[which][(size_t)i]);
             }
-            // GPU step of this group on a worker thread ...
-            std::vector<as_call> part;
-            int64_t n_part = 0;
+            // GPU step of this group on a worker thread (passes of up to 8 tables) ...
+            std::vector<std::vector<as_call>> parts(NT);
             int rc = AS_OK;
             std::string gpu_error;
             const HostCounts& hc = buf[which];
             std::thread worker([&]() {
                 const double t0 = PhaseTimer::now();
-                int64_t cap = std::max<int64_t>(1 << 16, (int64_t)Tg * P / 256);
-                for (;;) {
-                    part.resize((size_t)cap);
-                    rc = hc.fmt == 2
-                             ? as_call_variants_host16(ctx, (const uint16_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(), Tg, P,
-                                                       ref_code.data(), thr_view.data(), cut, part.data(), cap, &n_part)
-                             : as_call_variants_host_packed(ctx, (const uint32_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(), Tg,
-                                                            P, ref_code.data(), thr_view.data(), cut, part.data(), cap, &n_part);
-                    if (rc != AS_EOVERFLOW) break;
-                    cap = n_part;  // the true count: run the group again with room for all of them
+                std::vector<as_call> list;
+                int64_t n_part[8];
+                for (size_t c0 = 0; c0 < NT && rc == AS_OK; c0 += 8) {
+                    const int32_t nc = (int32_t)std::min<size_t>(8, NT - c0);
+                    const float* tv = thr_view.data() + c0 * (size_t)P * 8;
+                    int64_t cap = std::max<int64_t>(1 << 16, (int64_t)Tg * P / 256);
+                    for (;;) {
+                        list.resize((size_t)cap * (size_t)nc);
+                        rc = hc.fmt == 2
+                                 ? as_call_variants_sweep_host16(ctx, (const uint16_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(), Tg,
+                                                                 P, ref_code.data(), tv, nc, cut, list.data(), cap, n_part)
+                                 : as_call_variants_sweep_host_packed(ctx, (const uint32_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(),
+                                                                      Tg, P, ref_code.data(), tv, nc, cut, list.data(), cap, n_part);
+                        if (rc != AS_EOVERFLOW) break;
+                        cap = *std::max_element(n_part, n_part + nc);  // the largest true count: run the group again with room for all
+                    }
+                    if (rc == AS_OK)
+                        for (int32_t i = 0; i < nc; ++i)
+                            parts[c0 + (size_t)i].assign(list.begin() + (long)(i * cap), list.begin() + (long)(i * cap + n_part[i]));
                 }
                 if (rc != AS_OK) gpu_error = as_last_error();
                 gpu_s += PhaseTimer::now() - t0;
@@ -2170,18 +2303,6 @@ int as_variant_calling_main(int argc, char** argv) {
             }
             if (next_rc == 1) return report_gpu_error("pinned host allocation");
             if (next_rc >= 2) return 0;
-            part.resize((size_t)n_part);
-            const size_t base = calls.size();
-            calls.resize(base + part.size());
-            call_counts.resize(base + part.size());
-            call_row.resize(base + part.size(), -1);
-            call_rd.resize(base + part.size(), -1);
-            parallel_for(part.size(), [&](size_t i) {
-                as_call c = part[i];
-                hc.record(c.sample, c.slot, P, call_counts[base + i].fw, call_counts[base + i].bw);
-                c.sample += (int32_t)first;
-                calls[base + i] = c;
-            });
             // ---- rows the tensor has no slot for (a file listing a position more often than the panel enumerates it): the
             // reference tests every row (VC:869-3288), so they go through the caller as well, in one small pass of their own
             // (one "sample", one "slot" per row, thresholds and reference base of the row's position)
@@ -2191,12 +2312,13 @@ int as_variant_calling_main(int argc, char** argv) {
                 for (const AseqStats::ExtraRow& x : file_stats[(size_t)(first + i)].extras) xr.emplace_back((int32_t)(first + i), &x);
                 fixes = fixes || !file_stats[(size_t)(first + i)].rd_fix.empty();
             }
+            std::vector<std::pair<int32_t, const AseqStats::ExtraRow*>> use;
+            std::vector<std::vector<as_call>> xcalls(NT);
             if (!xr.empty()) {
                 // The reference's strand tests take (alt_fw, RD - reverse reads) and (alt_bw, reverse reads), RD being the COLUMN
                 // (VC:895-896); the coverage gate takes the sums (VC:898).  So the gate is applied here and the row goes to the
                 // caller with its forward depth set to RD - reverse reads (the reference base's count absorbs the difference;
                 // alt counts are untouched) and a cutoff of 1.
-                std::vector<std::pair<int32_t, const AseqStats::ExtraRow*>> use;
                 std::vector<uint32_t> fwadj;
                 for (const auto& pr : xr) {
                     const AseqStats::ExtraRow& x = *pr.second;
@@ -2217,214 +2339,258 @@ int as_variant_calling_main(int argc, char** argv) {
                 std::vector<uint32_t> xc((size_t)M * 8 + 4);
                 uint32_t* xcp = (uint32_t*)(((uintptr_t)xc.data() + 15) & ~(uintptr_t)15);
                 std::vector<uint8_t> xref((size_t)M);
-                std::vector<float> xthr((size_t)M * 8);
+                std::vector<float> xthr(NT * (size_t)M * 8);  // [NT][M][4][2]
                 for (int64_t m = 0; m < M; ++m) {
                     const AseqStats::ExtraRow& x = *use[(size_t)m].second;
                     memcpy(xcp + m * 4, x.fw, 16);
                     memcpy(xcp + (M + m) * 4, x.bw, 16);
                     xref[(size_t)m] = ref_code[(size_t)x.slot];
                     xcp[m * 4 + xref[(size_t)m]] = fwadj[(size_t)m];
-                    memcpy(&xthr[(size_t)m * 8], &thr_view[(size_t)x.slot * 8], 32);
+                    for (size_t k = 0; k < NT; ++k)
+                        memcpy(&xthr[(k * (size_t)M + (size_t)m) * 8], &thr_view[(k * (size_t)P + (size_t)x.slot) * 8], 32);
                 }
-                std::vector<as_call> xcalls((size_t)M * 3 + 1);
-                int64_t nx = 0;
-                if (M > 0 && as_call_variants_host(ctx, xcp, 1, M, xref.data(), xthr.data(), 1, xcalls.data(), (int64_t)xcalls.size(), &nx) != AS_OK)
-                    return report_gpu_error("as_call_variants_host");
-                for (int64_t i = 0; i < nx; ++i) {
-                    const AseqStats::ExtraRow& x = *use[(size_t)xcalls[(size_t)i].slot].second;
-                    as_call c = xcalls[(size_t)i];
-                    c.sample = use[(size_t)xcalls[(size_t)i].slot].first;
-                    c.slot = x.slot;
-                    CallCounts k;
-                    memcpy(k.fw, x.fw, 16);
-                    memcpy(k.bw, x.bw, 16);
-                    long long sum = 0;
-                    for (int b = 0; b < 4; ++b) sum += (long long)x.fw[b] + x.bw[b];
-                    calls.push_back(c);
-                    call_counts.push_back(k);
-                    call_row.push_back(x.row);
-                    call_rd.push_back(x.rd != sum ? x.rd : -1);
+                const int64_t xcap = M * 3 + 1;  // at most three calls per row: never an overflow
+                std::vector<as_call> xlist;
+                int64_t nx[8];
+                for (size_t c0 = 0; M > 0 && c0 < NT; c0 += 8) {
+                    const int32_t nc = (int32_t)std::min<size_t>(8, NT - c0);
+                    xlist.resize((size_t)xcap * (size_t)nc);
+                    if (as_call_variants_sweep_host(ctx, xcp, 1, M, xref.data(), xthr.data() + c0 * (size_t)M * 8, nc, 1, xlist.data(), xcap,
+                                                    nx) != AS_OK)
+                        return report_gpu_error("as_call_variants_host");
+                    for (int32_t i = 0; i < nc; ++i)
+                        xcalls[c0 + (size_t)i].assign(xlist.begin() + (long)(i * xcap), xlist.begin() + (long)(i * xcap + nx[i]));
                 }
             }
-            if (fixes) {  // RD column of rows where it is not the sum of the counts
-                for (size_t i = base; i < base + part.size(); ++i) {
-                    for (const AseqStats::RdFix& f : file_stats[(size_t)calls[i].sample].rd_fix)
-                        if (f.slot == calls[i].slot) call_rd[i] = f.rd;
+            for (size_t tk = 0; tk < NT; ++tk) {
+                std::vector<as_call>& calls = per_table[tk].calls;
+                std::vector<CallCounts>& call_counts = per_table[tk].call_counts;
+                std::vector<int32_t>& call_row = per_table[tk].call_row;
+                std::vector<long long>& call_rd = per_table[tk].call_rd;
+                const std::vector<as_call>& part = parts[tk];
+                const size_t base = calls.size();
+                calls.resize(base + part.size());
+                call_counts.resize(base + part.size());
+                call_row.resize(base + part.size(), -1);
+                call_rd.resize(base + part.size(), -1);
+                parallel_for(part.size(), [&](size_t i) {
+                    as_call c = part[i];
+                    hc.record(c.sample, c.slot, P, call_counts[base + i].fw, call_counts[base + i].bw);
+                    c.sample += (int32_t)first;
+                    calls[base + i] = c;
+                });
+                if (!xr.empty()) {
+                    const std::vector<as_call>& xc = xcalls[tk];
+                    for (size_t i = 0; i < xc.size(); ++i) {
+                        const AseqStats::ExtraRow& x = *use[(size_t)xc[i].slot].second;
+                        as_call c = xc[i];
+                        c.sample = use[(size_t)xc[i].slot].first;
+                        c.slot = x.slot;
+                        CallCounts k;
+                        memcpy(k.fw, x.fw, 16);
+                        memcpy(k.bw, x.bw, 16);
+                        long long sum = 0;
+                        for (int b = 0; b < 4; ++b) sum += (long long)x.fw[b] + x.bw[b];
+                        calls.push_back(c);
+                        call_counts.push_back(k);
+                        call_row.push_back(x.row);
+                        call_rd.push_back(x.rd != sum ? x.rd : -1);
+                    }
+                }
+                if (fixes) {  // RD column of rows where it is not the sum of the counts
+                    for (size_t i = base; i < base + part.size(); ++i) {
+                        for (const AseqStats::RdFix& f : file_stats[(size_t)calls[i].sample].rd_fix)
+                            if (f.slot == calls[i].slot) call_rd[i] = f.rd;
+                    }
+                }
+                if (!xr.empty()) {  // back into sample order (the calls of the extra rows were appended behind the group's)
+                    std::vector<size_t> order(calls.size() - base);
+                    for (size_t i = 0; i < order.size(); ++i) order[i] = base + i;
+                    std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return calls[a].sample < calls[b].sample; });
+                    std::vector<as_call> c2(order.size());
+                    std::vector<CallCounts> k2(order.size());
+                    std::vector<int32_t> r2(order.size());
+                    std::vector<long long> d2(order.size());
+                    for (size_t i = 0; i < order.size(); ++i) { c2[i] = calls[order[i]]; k2[i] = call_counts[order[i]]; r2[i] = call_row[order[i]]; d2[i] = call_rd[order[i]]; }
+                    std::copy(c2.begin(), c2.end(), calls.begin() + (long)base);
+                    std::copy(k2.begin(), k2.end(), call_counts.begin() + (long)base);
+                    std::copy(r2.begin(), r2.end(), call_row.begin() + (long)base);
+                    std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)base);
                 }
             }
-            if (!xr.empty()) {  // back into sample order (the calls of the extra rows were appended behind the group's)
-                std::vector<size_t> order(calls.size() - base);
-                for (size_t i = 0; i < order.size(); ++i) order[i] = base + i;
-                std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return calls[a].sample < calls[b].sample; });
+        }
+        // The device returns (sample, slot, alt) order = the reference's file-row order (VC:869-3288: rows, then alts
+        // A,C,G,T) for every file whose rows follow the panel enumeration.  A file that does not is re-ordered by its rows.
+        for (TableCalls& tc : per_table) {
+            std::vector<as_call>& calls = tc.calls;
+            std::vector<CallCounts>& call_counts = tc.call_counts;
+            std::vector<int32_t>& call_row = tc.call_row;
+            std::vector<long long>& call_rd = tc.call_rd;
+            std::vector<size_t> run_begin((size_t)T + 1, calls.size());
+            for (size_t i = calls.size(); i-- > 0;) run_begin[(size_t)calls[i].sample] = i;
+            for (int t = T - 1; t >= 0; --t) run_begin[(size_t)t] = std::min(run_begin[(size_t)t], run_begin[(size_t)t + 1]);
+            for (int t = 0; t < T; ++t) {
+                if (file_stats[(size_t)t].in_order) continue;
+                std::vector<int32_t> row_of((size_t)P, -1);
+                const std::vector<int32_t>& sor = file_stats[(size_t)t].slot_of_row;
+                for (size_t r = 0; r < sor.size(); ++r)
+                    if (sor[r] >= 0) row_of[(size_t)sor[r]] = (int32_t)r;
+                const size_t lo = run_begin[(size_t)t], hi = run_begin[(size_t)t + 1];
+                std::vector<size_t> order(hi - lo);
+                for (size_t i = 0; i < order.size(); ++i) order[i] = lo + i;
+                std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) {
+                    const int32_t rx = call_row[x] >= 0 ? call_row[x] : row_of[(size_t)calls[x].slot];
+                    const int32_t ry = call_row[y] >= 0 ? call_row[y] : row_of[(size_t)calls[y].slot];
+                    return rx != ry ? rx < ry : calls[x].alt < calls[y].alt;
+                });
                 std::vector<as_call> c2(order.size());
                 std::vector<CallCounts> k2(order.size());
                 std::vector<int32_t> r2(order.size());
                 std::vector<long long> d2(order.size());
                 for (size_t i = 0; i < order.size(); ++i) { c2[i] = calls[order[i]]; k2[i] = call_counts[order[i]]; r2[i] = call_row[order[i]]; d2[i] = call_rd[order[i]]; }
-                std::copy(c2.begin(), c2.end(), calls.begin() + (long)base);
-                std::copy(k2.begin(), k2.end(), call_counts.begin() + (long)base);
-                std::copy(r2.begin(), r2.end(), call_row.begin() + (long)base);
-                std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)base);
+                std::copy(c2.begin(), c2.end(), calls.begin() + (long)lo);
+                std::copy(k2.begin(), k2.end(), call_counts.begin() + (long)lo);
+                std::copy(r2.begin(), r2.end(), call_row.begin() + (long)lo);
+                std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)lo);
             }
-        }
-        // The device returns (sample, slot, alt) order = the reference's file-row order (VC:869-3288: rows, then alts
-        // A,C,G,T) for every file whose rows follow the panel enumeration.  A file that does not is re-ordered by its rows.
-        std::vector<size_t> run_begin((size_t)T + 1, calls.size());
-        for (size_t i = calls.size(); i-- > 0;) run_begin[(size_t)calls[i].sample] = i;
-        for (int t = T - 1; t >= 0; --t) run_begin[(size_t)t] = std::min(run_begin[(size_t)t], run_begin[(size_t)t + 1]);
-        for (int t = 0; t < T; ++t) {
-            if (file_stats[(size_t)t].in_order) continue;
-            std::vector<int32_t> row_of((size_t)P, -1);
-            const std::vector<int32_t>& sor = file_stats[(size_t)t].slot_of_row;
-            for (size_t r = 0; r < sor.size(); ++r)
-                if (sor[r] >= 0) row_of[(size_t)sor[r]] = (int32_t)r;
-            const size_t lo = run_begin[(size_t)t], hi = run_begin[(size_t)t + 1];
-            std::vector<size_t> order(hi - lo);
-            for (size_t i = 0; i < order.size(); ++i) order[i] = lo + i;
-            std::stable_sort(order.begin(), order.end(), [&](size_t x, size_t y) {
-                const int32_t rx = call_row[x] >= 0 ? call_row[x] : row_of[(size_t)calls[x].slot];
-                const int32_t ry = call_row[y] >= 0 ? call_row[y] : row_of[(size_t)calls[y].slot];
-                return rx != ry ? rx < ry : calls[x].alt < calls[y].alt;
-            });
-            std::vector<as_call> c2(order.size());
-            std::vector<CallCounts> k2(order.size());
-            std::vector<int32_t> r2(order.size());
-            std::vector<long long> d2(order.size());
-            for (size_t i = 0; i < order.size(); ++i) { c2[i] = calls[order[i]]; k2[i] = call_counts[order[i]]; r2[i] = call_row[order[i]]; d2[i] = call_rd[order[i]]; }
-            std::copy(c2.begin(), c2.end(), calls.begin() + (long)lo);
-            std::copy(k2.begin(), k2.end(), call_counts.begin() + (long)lo);
-            std::copy(r2.begin(), r2.end(), call_row.begin() + (long)lo);
-            std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)lo);
         }
     }
     if (timer.on) fprintf(stderr, "AS_TIMING %s %.6f (%.3g rows/s)\nAS_TIMING caller_gpu_busy %.6f\n",
                           bam_files ? "pileup_tumours_busy" : "parse_tumours_busy", parse_s, total_rows / std::max(parse_s, 1e-9), gpu_s);
     timer.lap("parse_and_call", 6.0 * (double)T * (double)P, "tests");
 
-    // Fisher strand-bias p of every call (VC:902) on the device: one warp per call's 2x2 table
-    std::vector<double> fisher_p(calls.size());
-    {
-        std::vector<int32_t> tables(calls.size() * 4);
-        parallel_for(calls.size(), [&](size_t i) {
-            const CallCounts& k = call_counts[i];
-            const int32_t FWs = (int32_t)(k.fw[0] + k.fw[1] + k.fw[2] + k.fw[3]), BWs = (int32_t)(k.bw[0] + k.bw[1] + k.bw[2] + k.bw[3]);
-            tables[i * 4 + 0] = call_rd[i] >= 0 ? (int32_t)(call_rd[i] - BWs) : FWs;  // fisherTest(RD - RD_reverse, RD_reverse, alt_fw, alt_bw), VC:902
-            tables[i * 4 + 1] = BWs;
-            tables[i * 4 + 2] = (int32_t)k.fw[calls[i].alt];
-            tables[i * 4 + 3] = (int32_t)k.bw[calls[i].alt];
-        });
-        const int frc = as_fisher_tests_host(ctx, tables.data(), (int64_t)calls.size(), fisher_p.data());
-        if (frc != AS_OK) return report_gpu_error("as_fisher_tests_host");
-    }
-    timer.lap("fisher_tests", (double)calls.size(), "calls");
-
-    // ---- writers (VC:662-688, VC:1040-1066)
-    const std::string summary_name = output_dir + "/Summary_Variant_Info.txt";
-    std::ofstream output(summary_name.c_str());
-    output << "Filename\tChrom\tPosition\tSubtitution\tRD\tRD_fw\tRD_bw\tAF\tReads_fw\tReads_bw\tAF_fw\tAF_bw\tAmpliconEdge_"
-              "StrandBias\tFisherPvalue\tQscore_fw\tQscore_bw\tReadTier\tGermlineInfo\tMaxGermlineAF\t10merDownstream\t10merUpstream\tHo"
-              "mopolymerFlag"
-           << "\n";
-    const char* L = "ACGT";
-    // One tumour = one VCF and one run of summary rows: the tumours are formatted on all host threads (ostream formatting of
-    // ~20 numbers per call was the largest phase of a configs[1] run), every thread writes its own VCFs, and the summary
-    // runs are written in tumour order afterwards.
-    std::vector<size_t> call_begin((size_t)T + 1, calls.size());
-    for (size_t i = calls.size(); i-- > 0;) call_begin[(size_t)calls[i].sample] = i;
-    for (int t = T - 1; t >= 0; --t) call_begin[(size_t)t] = std::min(call_begin[(size_t)t], call_begin[(size_t)t + 1]);
-    std::vector<std::string> summary_rows((size_t)T);
-    auto write_tumour = [&](int t) {
-        std::ostringstream output;
-        // setprecision(4) is sticky on the reference's summary stream (VC:1066): only the first row of the run prints its
-        // leading columns with the default precision
-        if (call_begin[(size_t)t] > 0) output << std::setprecision(4);
-        const std::string vcf_name = output_dir + "/" + files[t].sample + ".vcf";
-        std::ofstream vcf(vcf_name.c_str());
-        time_t now = time(nullptr);
-        char dt_buf[64];
-        const char* dt = ctime_r(&now, dt_buf);
-        vcf << "##fileformat=VCF-like\n##fileDate=" << dt
-            << "##source=AmpliSolveVariantCalling\n##reference=Not_Specified_here\n##phasing=Not_Specified_here\n##FILTER=<ID="
-               "XXXXXXXXX,Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,"
-               "Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,Description='XXXXXXXXX'>\n##INFO=<ID=RD,Number=1,Type=Integer,"
-               "Description='Total Read Depth'>\n##SAMPLE=<ID=Not_Specified_here,SampleName="
-            << files[t].sample
-            << ">\n##INFO=<ID=AF,Number=.,Type=Float,Description='Allele Frequency'>\n##INFO=<ID=SR,Number=1,Type=String,"
-               "Description='Supporting Reads'>\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO"
-            << "\n";
-        for (size_t ci = call_begin[(size_t)t]; ci < call_begin[(size_t)t + 1]; ++ci) {
-            const as_call& c = calls[ci];
-            const int64_t s = c.slot;
-            const uint32_t* fw = call_counts[ci].fw;
-            const uint32_t* bw = call_counts[ci].bw;
-            const int FW = (int)(fw[0] + fw[1] + fw[2] + fw[3]), BW = (int)(bw[0] + bw[1] + bw[2] + bw[3]);
-            const int RD = call_rd[ci] >= 0 ? (int)call_rd[ci] : FW + BW;  // the RD column (VC:752), normally the sum
-            const int a = c.alt;
-            const int k_fw = (int)fw[a], k_bw = (int)bw[a];
-            const float AF = float(k_fw + k_bw) / float(RD);                    // VC:814-817
-            const float AF_fw = FW == 0 ? 0.f : float(k_fw) / float(FW);        // VC:776-795
-            const float AF_bw = BW == 0 ? 0.f : float(k_bw) / float(BW);        // VC:797-812
-            const long double Q_fw = q_from_p(c.p_fw), Q_bw = q_from_p(c.p_bw);  // VC:895-896
-            const double p = fisher_p[ci];                                      // VC:902
-            const char* flag_fisher = (p <= p_value_float) ? "YES" : "NO";      // VC:903-910
-            const char* flag_dup = panel.dup[s] ? "YES" : "NO";
-            const bool high = !(k_fw < 5 || k_bw < 5);                          // VC:912-919
-            const char* tier = high ? "HighQual" : "LowQual";
-            const std::string& max_germ_text = germ_text[(size_t)s * 4 + a];    // VC:943-954
-            const double max_germ = atof(max_germ_text.c_str());                // VC:972
-            const std::string chrom = panel.chroms[panel.slot_chrom[s]];
-            const std::string down = kmer(panel, panel.slot_chrom[s], panel.slot_pos[s], true);   // VC:964
-            const std::string up = kmer(panel, panel.slot_chrom[s], panel.slot_pos[s], false);    // VC:965
-            const int homo = homopolymer_test(down, up, L[a]);
-            const double Q = double(Q_fw + Q_bw) / 2.000;                       // VC:967
-            const std::string cat = std::string(flag_dup) + "_" + flag_fisher;
-            // FILTER: keys of an unordered_map in ITS iteration order (VC:993-1059)
-            std::unordered_map<std::string, std::string> flags;
-            int not_pass = 0;
-            if (cat == "YES_NO") { flags.insert(std::make_pair(std::string("AmpliconEdge"), std::string("AmpliconEdge"))); not_pass = 1; }
-            if (cat == "YES_YES") { flags.insert(std::make_pair(std::string("AmpliconEdge;StrandBias"), std::string("AmpliconEdge;StrandBias"))); not_pass = 1; }
-            if (cat == "NO_YES") { flags.insert(std::make_pair(std::string("StrandBias"), std::string("StrandBias"))); not_pass = 1; }
-            if (AF < max_germ && cat == "NO_NO" && !high) { flags.insert(std::make_pair(std::string("PositionWithHighNoise"), std::string("PositionWithHighNoise"))); not_pass = 1; }
-            if (homo == 1) { flags.insert(std::make_pair(std::string("HomoPolymerRegion"), std::string("HomoPolymerRegion"))); not_pass = 1; }
-            if (Q_fw < 20 || Q_bw < 20) { flags.insert(std::make_pair(std::string("LowQ"), std::string("LowQ"))); not_pass = 1; }
-            if (!high) { flags.insert(std::make_pair(std::string("LowSupportingReads"), std::string("LowSupportingReads"))); not_pass = 1; }
-            const std::string& pos_text = panel.pos_text[s];
-            const char* id = ".";
-            std::string filter = "PASS";
-            if (not_pass) {
-                filter.clear();
-                int first = 0;
-                for (auto it = flags.begin(); it != flags.end(); ++it) {
-                    filter = first == 0 ? it->first : filter + ";" + it->first;
-                    ++first;
-                }
-                if (c.ref == 1 && a == 2) id = "-";  // the reference writes ID "-" for non-PASS C->G rows (VC:1856)
-            }
-            vcf << chrom << "\t" << pos_text << "\t" << id << "\t" << L[c.ref] << "\t" << L[a] << "\t" << Q << "\t" << filter << "\t"
-                << AF << ";" << RD << ";" << k_fw + k_bw << "\n";
-            // summary row; setprecision(4) is sticky on this stream exactly as in VC:1066
-            output << files[t].sample << "\t" << chrom << "\t" << pos_text << "\t" << L[c.ref] << "->" << L[a] << "\t" << RD << "\t"
-                   << FW << "\t" << BW << "\t" << AF << "\t" << k_fw << "\t" << k_bw << "\t" << AF_fw << "\t" << AF_bw << "\t"
-                   << flag_dup << "_" << flag_fisher << "\t" << p << "\t" << std::setprecision(4) << Q_fw << "\t"
-                   << std::setprecision(4) << Q_bw << "\t" << tier << "\t" << "-" << "\t" << max_germ_text << "\t" << down << "\t"
-                   << up << "\t" << homo << "\n";
+    std::string summary_name;
+    for (size_t tk = 0; tk < NT; ++tk) {  // every table's outputs in its own directory
+        const std::vector<as_call>& calls = per_table[tk].calls;
+        const std::vector<CallCounts>& call_counts = per_table[tk].call_counts;
+        const std::vector<long long>& call_rd = per_table[tk].call_rd;
+        const std::vector<std::string>& germ_text = germ_texts[tk];
+        const std::string& output_dir = out_dirs[tk];
+        // Fisher strand-bias p of every call (VC:902) on the device: one warp per call's 2x2 table
+        std::vector<double> fisher_p(calls.size());
+        {
+            std::vector<int32_t> tables(calls.size() * 4);
+            parallel_for(calls.size(), [&](size_t i) {
+                const CallCounts& k = call_counts[i];
+                const int32_t FWs = (int32_t)(k.fw[0] + k.fw[1] + k.fw[2] + k.fw[3]), BWs = (int32_t)(k.bw[0] + k.bw[1] + k.bw[2] + k.bw[3]);
+                tables[i * 4 + 0] = call_rd[i] >= 0 ? (int32_t)(call_rd[i] - BWs) : FWs;  // fisherTest(RD - RD_reverse, RD_reverse, alt_fw, alt_bw), VC:902
+                tables[i * 4 + 1] = BWs;
+                tables[i * 4 + 2] = (int32_t)k.fw[calls[i].alt];
+                tables[i * 4 + 3] = (int32_t)k.bw[calls[i].alt];
+            });
+            const int frc = as_fisher_tests_host(ctx, tables.data(), (int64_t)calls.size(), fisher_p.data());
+            if (frc != AS_OK) return report_gpu_error("as_fisher_tests_host");
         }
-        summary_rows[(size_t)t] = output.str();
-    };
-    {
-        std::atomic<int> next(0);
-        auto work = [&]() {
-            for (int t = next.fetch_add(1); t < T; t = next.fetch_add(1)) write_tumour(t);
+        timer.lap("fisher_tests", (double)calls.size(), "calls");  // once per table in a sweep
+
+        // ---- writers (VC:662-688, VC:1040-1066)
+        summary_name = output_dir + "/Summary_Variant_Info.txt";
+        std::ofstream output(summary_name.c_str());
+        output << "Filename\tChrom\tPosition\tSubtitution\tRD\tRD_fw\tRD_bw\tAF\tReads_fw\tReads_bw\tAF_fw\tAF_bw\tAmpliconEdge_"
+                  "StrandBias\tFisherPvalue\tQscore_fw\tQscore_bw\tReadTier\tGermlineInfo\tMaxGermlineAF\t10merDownstream\t10merUpstream\tHo"
+                  "mopolymerFlag"
+               << "\n";
+        const char* L = "ACGT";
+        // One tumour = one VCF and one run of summary rows: the tumours are formatted on all host threads (ostream formatting of
+        // ~20 numbers per call was the largest phase of a configs[1] run), every thread writes its own VCFs, and the summary
+        // runs are written in tumour order afterwards.
+        std::vector<size_t> call_begin((size_t)T + 1, calls.size());
+        for (size_t i = calls.size(); i-- > 0;) call_begin[(size_t)calls[i].sample] = i;
+        for (int t = T - 1; t >= 0; --t) call_begin[(size_t)t] = std::min(call_begin[(size_t)t], call_begin[(size_t)t + 1]);
+        std::vector<std::string> summary_rows((size_t)T);
+        auto write_tumour = [&](int t) {
+            std::ostringstream output;
+            // setprecision(4) is sticky on the reference's summary stream (VC:1066): only the first row of the run prints its
+            // leading columns with the default precision
+            if (call_begin[(size_t)t] > 0) output << std::setprecision(4);
+            const std::string vcf_name = output_dir + "/" + files[t].sample + ".vcf";
+            std::ofstream vcf(vcf_name.c_str());
+            time_t now = time(nullptr);
+            char dt_buf[64];
+            const char* dt = ctime_r(&now, dt_buf);
+            vcf << "##fileformat=VCF-like\n##fileDate=" << dt
+                << "##source=AmpliSolveVariantCalling\n##reference=Not_Specified_here\n##phasing=Not_Specified_here\n##FILTER=<ID="
+                   "XXXXXXXXX,Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,"
+                   "Description='XXXXXXXXX'>\n##FILTER=<ID=XXXXXXXXX,Description='XXXXXXXXX'>\n##INFO=<ID=RD,Number=1,Type=Integer,"
+                   "Description='Total Read Depth'>\n##SAMPLE=<ID=Not_Specified_here,SampleName="
+                << files[t].sample
+                << ">\n##INFO=<ID=AF,Number=.,Type=Float,Description='Allele Frequency'>\n##INFO=<ID=SR,Number=1,Type=String,"
+                   "Description='Supporting Reads'>\n#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO"
+                << "\n";
+            for (size_t ci = call_begin[(size_t)t]; ci < call_begin[(size_t)t + 1]; ++ci) {
+                const as_call& c = calls[ci];
+                const int64_t s = c.slot;
+                const uint32_t* fw = call_counts[ci].fw;
+                const uint32_t* bw = call_counts[ci].bw;
+                const int FW = (int)(fw[0] + fw[1] + fw[2] + fw[3]), BW = (int)(bw[0] + bw[1] + bw[2] + bw[3]);
+                const int RD = call_rd[ci] >= 0 ? (int)call_rd[ci] : FW + BW;  // the RD column (VC:752), normally the sum
+                const int a = c.alt;
+                const int k_fw = (int)fw[a], k_bw = (int)bw[a];
+                const float AF = float(k_fw + k_bw) / float(RD);                    // VC:814-817
+                const float AF_fw = FW == 0 ? 0.f : float(k_fw) / float(FW);        // VC:776-795
+                const float AF_bw = BW == 0 ? 0.f : float(k_bw) / float(BW);        // VC:797-812
+                const long double Q_fw = q_from_p(c.p_fw), Q_bw = q_from_p(c.p_bw);  // VC:895-896
+                const double p = fisher_p[ci];                                      // VC:902
+                const char* flag_fisher = (p <= p_value_float) ? "YES" : "NO";      // VC:903-910
+                const char* flag_dup = panel.dup[s] ? "YES" : "NO";
+                const bool high = !(k_fw < 5 || k_bw < 5);                          // VC:912-919
+                const char* tier = high ? "HighQual" : "LowQual";
+                const std::string& max_germ_text = germ_text[(size_t)s * 4 + a];    // VC:943-954
+                const double max_germ = atof(max_germ_text.c_str());                // VC:972
+                const std::string chrom = panel.chroms[panel.slot_chrom[s]];
+                const std::string down = kmer(panel, panel.slot_chrom[s], panel.slot_pos[s], true);   // VC:964
+                const std::string up = kmer(panel, panel.slot_chrom[s], panel.slot_pos[s], false);    // VC:965
+                const int homo = homopolymer_test(down, up, L[a]);
+                const double Q = double(Q_fw + Q_bw) / 2.000;                       // VC:967
+                const std::string cat = std::string(flag_dup) + "_" + flag_fisher;
+                // FILTER: keys of an unordered_map in ITS iteration order (VC:993-1059)
+                std::unordered_map<std::string, std::string> flags;
+                int not_pass = 0;
+                if (cat == "YES_NO") { flags.insert(std::make_pair(std::string("AmpliconEdge"), std::string("AmpliconEdge"))); not_pass = 1; }
+                if (cat == "YES_YES") { flags.insert(std::make_pair(std::string("AmpliconEdge;StrandBias"), std::string("AmpliconEdge;StrandBias"))); not_pass = 1; }
+                if (cat == "NO_YES") { flags.insert(std::make_pair(std::string("StrandBias"), std::string("StrandBias"))); not_pass = 1; }
+                if (AF < max_germ && cat == "NO_NO" && !high) { flags.insert(std::make_pair(std::string("PositionWithHighNoise"), std::string("PositionWithHighNoise"))); not_pass = 1; }
+                if (homo == 1) { flags.insert(std::make_pair(std::string("HomoPolymerRegion"), std::string("HomoPolymerRegion"))); not_pass = 1; }
+                if (Q_fw < 20 || Q_bw < 20) { flags.insert(std::make_pair(std::string("LowQ"), std::string("LowQ"))); not_pass = 1; }
+                if (!high) { flags.insert(std::make_pair(std::string("LowSupportingReads"), std::string("LowSupportingReads"))); not_pass = 1; }
+                const std::string& pos_text = panel.pos_text[s];
+                const char* id = ".";
+                std::string filter = "PASS";
+                if (not_pass) {
+                    filter.clear();
+                    int first = 0;
+                    for (auto it = flags.begin(); it != flags.end(); ++it) {
+                        filter = first == 0 ? it->first : filter + ";" + it->first;
+                        ++first;
+                    }
+                    if (c.ref == 1 && a == 2) id = "-";  // the reference writes ID "-" for non-PASS C->G rows (VC:1856)
+                }
+                vcf << chrom << "\t" << pos_text << "\t" << id << "\t" << L[c.ref] << "\t" << L[a] << "\t" << Q << "\t" << filter << "\t"
+                    << AF << ";" << RD << ";" << k_fw + k_bw << "\n";
+                // summary row; setprecision(4) is sticky on this stream exactly as in VC:1066
+                output << files[t].sample << "\t" << chrom << "\t" << pos_text << "\t" << L[c.ref] << "->" << L[a] << "\t" << RD << "\t"
+                       << FW << "\t" << BW << "\t" << AF << "\t" << k_fw << "\t" << k_bw << "\t" << AF_fw << "\t" << AF_bw << "\t"
+                       << flag_dup << "_" << flag_fisher << "\t" << p << "\t" << std::setprecision(4) << Q_fw << "\t"
+                       << std::setprecision(4) << Q_bw << "\t" << tier << "\t" << "-" << "\t" << max_germ_text << "\t" << down << "\t"
+                       << up << "\t" << homo << "\n";
+            }
+            summary_rows[(size_t)t] = output.str();
         };
-        run_on_threads(std::max(1u, std::min(std::thread::hardware_concurrency(), (unsigned)std::max(1, T))), work);
+        {
+            std::atomic<int> next(0);
+            auto work = [&]() {
+                for (int t = next.fetch_add(1); t < T; t = next.fetch_add(1)) write_tumour(t);
+            };
+            run_on_threads(std::max(1u, std::min(std::thread::hardware_concurrency(), (unsigned)std::max(1, T))), work);
+        }
+        for (int t = 0; t < T; ++t) {
+            if ((t + 1) % 50 == 0)
+                std::cout << "\tParsed successfully " << GREEN << (t + 1) << "/" << T << RESET << "  samples" << std::endl;
+            output.write(summary_rows[(size_t)t].data(), (std::streamsize)summary_rows[(size_t)t].size());
+        }
+        output.close();
+        timer.lap("write_outputs", (double)calls.size(), "calls");
     }
-    for (int t = 0; t < T; ++t) {
-        if ((t + 1) % 50 == 0)
-            std::cout << "\tParsed successfully " << GREEN << (t + 1) << "/" << T << RESET << "  samples" << std::endl;
-        output.write(summary_rows[(size_t)t].data(), (std::streamsize)summary_rows[(size_t)t].size());
-    }
-    output.close();
-    timer.lap("write_outputs", (double)calls.size(), "calls");
     std::cout << "\nAmpliSolveVariantCalling execution was successful. The results can be found at : " << YELLOW << summary_name
               << RESET << std::endl;
     std::cout << "\n" << STARS << std::endl;

@@ -190,6 +190,25 @@ int as_noise_estimate_host_packed(as_ctx* ctx, const uint32_t* packed, const as_
                                   float* thr, float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec,
                                   float* thr_view);
 
+/* Noise-floor sweep on the _host path, in each of the three host formats (counts [+ wide, n_wide] as in the
+ * single-value form): c_values is a host array [n_c], 1 <= n_c <= 8 (anything else: AS_EINVAL); thr and thr_view (when
+ * not NULL) are [n_c][P][4][2].  Table i and its caller view are bit for bit what the single-value form returns for
+ * c_values[i]; germ_val, germ_state, count and nrec (independent of C) are written once.  The counts go up once: each
+ * upload tile runs noise_pattern_kernel for all values, the twin groups the tile holds once per value, and the twin
+ * groups that straddle tiles are gathered once and reduced once per value.  n_c == 1 runs exactly the single-value
+ * path (same kernels, same launches).  A multi-device context shards as the single-value forms do. */
+int as_noise_estimate_sweep_host(as_ctx* ctx, const uint32_t* counts, int32_t S, int64_t P, const int32_t* twin_next,
+                                 const int32_t* twin_head, const float* c_values, int32_t n_c, int32_t cut, float* thr,
+                                 float* germ_val, uint8_t* germ_state, uint32_t* count, uint32_t* nrec, float* thr_view);
+int as_noise_estimate_sweep_host16(as_ctx* ctx, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t S,
+                                   int64_t P, const int32_t* twin_next, const int32_t* twin_head, const float* c_values,
+                                   int32_t n_c, int32_t cut, float* thr, float* germ_val, uint8_t* germ_state, uint32_t* count,
+                                   uint32_t* nrec, float* thr_view);
+int as_noise_estimate_sweep_host_packed(as_ctx* ctx, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t S,
+                                        int64_t P, const int32_t* twin_next, const int32_t* twin_head, const float* c_values,
+                                        int32_t n_c, int32_t cut, float* thr, float* germ_val, uint8_t* germ_state,
+                                        uint32_t* count, uint32_t* nrec, float* thr_view);
+
 /* The noise table crosses to the caller as "%f" text (EE:1787 -> std::stof at VC:889-890) with
  * "-1_-1" replaced by "0.01_0.01" (EE:2680-2684).  This applies exactly that mapping to thr
  * [n] floats in place of the text round trip: NaN -> 0.01f, v -> strtof(sprintf("%f", v)). */
@@ -226,6 +245,22 @@ int as_call_variants_host16(as_ctx* ctx, const uint16_t* counts, const as_wide_r
 int as_call_variants_host_packed(as_ctx* ctx, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T,
                                  int64_t P, const uint8_t* ref, const float* thr_view, int32_t cut, as_call* calls,
                                  int64_t cap, int64_t* n_calls);
+
+/* Caller sweep on the _host path, in each of the three host formats: thr_views [n_c][P][4][2], 1 <= n_c <= 8 (anything
+ * else: AS_EINVAL), calls [n_c][cap], n_calls [n_c].  List i is what the single-table form returns for table i, in the same
+ * order (sample, slot, alt); n_calls[i] is its true count.  AS_EOVERFLOW when any table has more than cap calls (the
+ * first cap entries of every list are valid).  The tumour tensor goes up once; the n_c tables go up once ahead of the
+ * first tile.  The kernel is chosen as as_call_variants_sweep_dev chooses it (the deferred pipeline by default, the
+ * in-stage sweep kernel when a staged variant is selected); n_c == 1 runs exactly the single-table path.  Every table's
+ * lists are sorted with one radix sort per table.  A multi-device context shards as the single-table forms do. */
+int as_call_variants_sweep_host(as_ctx* ctx, const uint32_t* counts, int32_t T, int64_t P, const uint8_t* ref,
+                                const float* thr_views, int32_t n_c, int32_t cut, as_call* calls, int64_t cap, int64_t* n_calls);
+int as_call_variants_sweep_host16(as_ctx* ctx, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t T,
+                                  int64_t P, const uint8_t* ref, const float* thr_views, int32_t n_c, int32_t cut, as_call* calls,
+                                  int64_t cap, int64_t* n_calls);
+int as_call_variants_sweep_host_packed(as_ctx* ctx, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T,
+                                       int64_t P, const uint8_t* ref, const float* thr_views, int32_t n_c, int32_t cut,
+                                       as_call* calls, int64_t cap, int64_t* n_calls);
 
 /* A device call list into the reference's row order (sample, slot, alt; VC:672, VC:723, VC:869-3288) without leaving the
  * device: slot_offset is added to every slot of d_calls first, IN PLACE (a shard's local slot ids -> panel slot ids), then one
