@@ -6,6 +6,7 @@ The function names mirror the reference code each one replaces:
                                   (AmpliSolveErrorEstimation.cpp:1484-2544, :1247-1467)
     Context.thresholds_caller_view  the "%f" -> std::stof hand-over (EE:1787 -> VC:889-890)
     Context.call_variants         the row loop of callVariants (AmpliSolveVariantCalling.cpp:723-3296)
+    Context.site_tests            VC:895-898 for listed sites in every tumour, called or not
     Context.mutation_rules_poisson_quality_score   VC:3834-3884, element-wise
     Context.kf_gammaq             VC:3726, element-wise
 
@@ -24,6 +25,11 @@ ABSENT = 0xFFFFFFFF
 CALL_DTYPE = np.dtype([("sample", "<i4"), ("slot", "<i4"), ("alt", "<i4"), ("ref", "<i4"), ("p_fw", "<f8"),
                        ("p_bw", "<f8"), ("q_fw", "<f8"), ("q_bw", "<f8")])
 assert CALL_DTYPE.itemsize == 48
+# as_site_test and its statuses (include/amplisolve_b200.h)
+SITE_TEST_DTYPE = np.dtype([("depth_fw", "<u4"), ("depth_bw", "<u4"), ("alt_fw", "<u4"), ("alt_bw", "<u4"), ("p_fw", "<f8"),
+                            ("p_bw", "<f8"), ("status", "<i4"), ("pad", "<i4")])
+assert SITE_TEST_DTYPE.itemsize == 40
+SITE_CALLED, SITE_NOT_CALLED, SITE_LOW_COVERAGE, SITE_NO_DATA, SITE_NOT_TESTABLE = 1, 2, 3, 4, 5
 
 EXPORTS = [
     "as_last_error", "as_version", "as_device_count", "as_create", "as_create_multi", "as_context_devices", "as_shard_bounds", "as_destroy", "as_host_alloc", "as_host_free",
@@ -31,7 +37,8 @@ EXPORTS = [
     "as_noise_estimate_host16", "as_thresholds_caller_view_dev", "as_call_variants_dev", "as_call_variants_host",
     "as_call_variants_host16", "as_sort_calls_dev", "as_call_variants_sweep_dev", "as_noise_estimate_sweep_dev", "as_pack_counts", "as_noise_estimate_host_packed", "as_call_variants_host_packed",
     "as_noise_estimate_sweep_host", "as_noise_estimate_sweep_host16", "as_noise_estimate_sweep_host_packed", "as_call_variants_sweep_host",
-    "as_call_variants_sweep_host16", "as_call_variants_sweep_host_packed", "as_poisson_test_host",
+    "as_call_variants_sweep_host16", "as_call_variants_sweep_host_packed", "as_site_tests_host", "as_site_tests_host16",
+    "as_site_tests_host_packed", "as_poisson_test_host",
     "as_kf_gammaq_host", "as_synth_counts_dev", "as_synth_twin_links_dev", "as_hash_iteration_order", "as_fisher_test", "as_fisher_tests_host", "as_error_estimation_main",
     "as_variant_calling_main", "as_pileup_begin", "as_pileup_add_host", "as_pileup_end_host", "as_pileup_end_wire", "as_pileup_set_host", "as_compute_counts_main", "as_serve_main", "as_client_run", "as_process_is_resident",
 ]
@@ -170,6 +177,9 @@ def lib():
     L.as_call_variants_sweep_host.argtypes = [vp, vp, i32, i64, vp, vp, i32, i32, vp, i64, vp]
     L.as_call_variants_sweep_host16.argtypes = [vp, vp, vp, i64, i32, i64, vp, vp, i32, i32, vp, i64, vp]
     L.as_call_variants_sweep_host_packed.argtypes = L.as_call_variants_sweep_host16.argtypes
+    L.as_site_tests_host.argtypes = [vp, vp, i32, i64, vp, vp, i32, vp, vp, i64, i32, vp]
+    L.as_site_tests_host16.argtypes = [vp, vp, vp, i64, i32, i64, vp, vp, i32, vp, vp, i64, i32, vp]
+    L.as_site_tests_host_packed.argtypes = L.as_site_tests_host16.argtypes
     L.as_pack_counts.argtypes = [vp, i32, i64, vp, vp, i64, C.POINTER(i64)]
     L.as_poisson_test_host.argtypes = [vp, vp, vp, vp, i64, vp, vp]
     L.as_kf_gammaq_host.argtypes = [vp, vp, vp, i64, vp]
@@ -436,6 +446,32 @@ class Context:
         if rc == -5:
             return self.call_variants_sweep(counts, ref, thr_views, coverage_cutoff, cap=int(n.max()), wide_records=wide_records)
         return [calls[i, :n[i]].copy() for i in range(n_c)]
+
+    def site_tests(self, counts, ref, thr_view, coverage_cutoff, site_slot, site_alt, wide_records=None):
+        """Site report (as_site_tests_host*): the strand tests of the listed sites (site_slot[i], site_alt[i]) in every tumour,
+        called or not.  counts / wide_records as in call_variants, thr_view [P][4][2] or [n_c][P][4][2].  Returns a
+        SITE_TEST_DTYPE array [n_c][T][H]: strand depths, alt reads, p_fw / p_bw (NaN where not evaluated) and status
+        (SITE_CALLED is the caller's decision)."""
+        fmt = _host_format(counts)
+        counts = _np(counts, np.uint16 if fmt == "u16" else np.uint32)
+        wr = _np(wide_records if wide_records is not None else np.zeros(0, WIDE_DTYPE), WIDE_DTYPE)
+        T, two, P = counts.shape[:3]
+        assert two == 2 and (fmt == "packed" or counts.shape[3] == 4)
+        ref = _np(ref, np.uint8)
+        tv = _np(thr_view, np.float32)
+        tv = tv.reshape((-1, P, 4, 2)) if tv.size or P == 0 else tv.reshape((0, P, 4, 2))
+        n_c = tv.shape[0]
+        slot, alt = _np(site_slot, np.int32).reshape(-1), _np(site_alt, np.int32).reshape(-1)
+        assert ref.shape == (P,) and slot.shape == alt.shape
+        H = len(slot)
+        out = np.zeros((n_c, T, H), SITE_TEST_DTYPE)
+        tail = (T, P, _hp(ref), _hp(tv), n_c, _hp(slot), _hp(alt), H, int(coverage_cutoff), _hp(out))
+        if fmt == "u32":
+            _check(lib().as_site_tests_host(self._h, _hp(counts), *tail))
+        else:
+            fn = lib().as_site_tests_host16 if fmt == "u16" else lib().as_site_tests_host_packed
+            _check(fn(self._h, _hp(counts), _hp(wr), len(wr), *tail))
+        return out
 
     def mutation_rules_poisson_quality_score(self, k, rd, err):
         k, rd, err = _np(k, np.int32), _np(rd, np.int32), _np(err, np.float32)

@@ -19,7 +19,7 @@ CSRC = PKG / "csrc"
 LIB = PKG / "lib" / "libamplisolve_b200.so"
 BIN = PKG / "bin"
 OBJ = PKG / "lib" / "obj"
-CU_SOURCES = ["as_kernels.cu", "as_noise_pattern.cu", "as_call_deferred.cu", "as_capi.cu", "as_sort.cu", "as_fisher.cu", "as_pileup.cu"]
+CU_SOURCES = ["as_kernels.cu", "as_noise_pattern.cu", "as_call_deferred.cu", "as_capi.cu", "as_sort.cu", "as_fisher.cu", "as_pileup.cu", "as_sites.cu"]
 CXX_SOURCES = ["as_host.cpp", "as_bam.cpp", "as_serve.cpp"]  # as_bam.cpp inflates BGZF blocks with zlib (-lz)
 HEADERS = ["as_device.cuh", "as_noise.cuh", "as_pipeline.cuh", "as_call.cuh", "as_kernels.h", "as_wire.h", "as_bam.h",
            "../../include/amplisolve_b200.h"]

@@ -103,6 +103,8 @@ struct as_ctx {
     DevBuf tile[2], tile16[2], wide[2], out[2], aux[2], misc, calls, sortbuf;  // _host pipelines
     DevBuf defer;                                                              // candidate / survivor lists of the deferred caller
     DevBuf lgtab;                                                              // lgamma(i + 1), i < lg_n (as_fisher_tests_host)
+    DevBuf sites;                                                              // as_site_tests_host*
+    PinnedGrow h_sites;
     int64_t lg_n = 0;
     PinnedGrow h_links, h_small;                                              // _host pipelines, host side
     DevBuf pile_first, pile_pos, pile_counts, pile_rec, pile_off, pile_ref, pile_stats;  // as_pileup_*
@@ -215,7 +217,7 @@ void as_destroy(as_ctx* c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     c->heads.release(); c->nheads.release(); c->misc.release(); c->calls.release(); c->sortbuf.release();
-    c->h_links.release(); c->h_small.release(); c->lgtab.release(); c->defer.release();
+    c->h_links.release(); c->h_small.release(); c->lgtab.release(); c->defer.release(); c->sites.release(); c->h_sites.release();
     c->pile_first.release(); c->pile_pos.release(); c->pile_counts.release(); c->pile_rec.release(); c->pile_off.release();
     c->pile_ref.release(); c->pile_stats.release(); c->pile_slots.release(); c->pile_wire.release(); c->pile_wide.release();
     for (int i = 0; i < 2; ++i) {
@@ -1161,6 +1163,136 @@ int as_call_variants_sweep_host_packed(as_ctx* c, const uint32_t* packed, const 
                                        as_call* calls, int64_t cap, int64_t* n_calls) {
     const HostSrc src{packed, 1, wide, n_wide};
     return call_variants_host_impl(c, src, T, P, ref, thr_views, n_c, cut, calls, cap, n_calls);
+}
+
+// ---- site report ---------------------------------------------------------------------------------------------------
+// The sites' columns of the host tensor are gathered in its own format into pinned memory ([T][2][H] words), go up as a count
+// tensor of H slots and through the path of an upload tile (widen / unpack, escaped records patched in after renumbering them
+// by site); site_test_kernel then evaluates every (table, site, tumour, strand) into out [n_c][T][H].
+static int site_tests_impl(as_ctx* c, const HostSrc& src, int32_t T, int64_t P, const uint8_t* ref, const float* thr_views,
+                           int32_t n_c, const int32_t* site_slot, const int32_t* site_alt, int64_t H, int32_t cut, as_site_test* out) {
+    if (n_c < 1 || n_c > 8) return fail(AS_EINVAL, "site tests take 1..8 threshold tables");
+    int rc = check_common(c, src.counts, T, P, 0, P, cut);
+    if (rc) return rc;
+    if (H < 0 || H > 0x7fffffffll) return fail(AS_EINVAL, "bad number of sites %lld", (long long)H);
+    if (H > 0 && (!ref || !thr_views || !site_slot || !site_alt || !out)) return fail(AS_EINVAL, "bad pointer");
+    for (int64_t h = 0; h < H; ++h) {
+        if (site_slot[h] < 0 || site_slot[h] >= P)
+            return fail(AS_EINVAL, "site %lld: slot %d outside [0, %lld)", (long long)h, site_slot[h], (long long)P);
+        if (site_alt[h] < 0 || site_alt[h] > 3) return fail(AS_EINVAL, "site %lld: alt %d is not 0..3", (long long)h, site_alt[h]);
+    }
+    if (H == 0 || T == 0) return AS_OK;
+    if ((rc = check_wide(src, T, P)) != AS_OK) return rc;
+    PhaseClock clk;
+    CU(cudaSetDevice(c->device));
+    const size_t word = (size_t)src.elem * 4;  // bytes per (sample, strand, slot) in the host format
+    const int64_t rows = (int64_t)T * 2;
+    const size_t n_words = (size_t)rows * (size_t)H;
+    std::vector<as_wide_record> wide;  // escaped records of the sites' slots, slot = site index
+    if (src.elem != 4)
+        for (int64_t h = 0; h < H; ++h) {
+            const as_wide_record* r = std::lower_bound(src.wide, src.wide + src.n_wide, (int64_t)site_slot[h],
+                                                       [](const as_wide_record& x, int64_t v) { return (int64_t)x.slot < v; });
+            for (; r < src.wide + src.n_wide && r->slot == site_slot[h]; ++r) {
+                wide.push_back(*r);
+                wide.back().slot = (int32_t)h;
+            }
+        }
+    // pinned host block: gathered columns | site_ra [H] | thr [n_c][H][2]
+    const size_t o_ra = (n_words * word + 15) & ~(size_t)15;
+    const size_t o_thr = (o_ra + (size_t)H * 2 + 15) & ~(size_t)15;
+    const size_t h_bytes = o_thr + (size_t)n_c * (size_t)H * 8;
+    CU(c->h_sites.need(h_bytes));
+    char* hb = (char*)c->h_sites.p;
+    {
+        const int nth = (int)std::max<int64_t>(1, std::min<int64_t>(std::min(std::thread::hardware_concurrency(), 16u), rows / 64));
+        auto work = [&](int k) {
+            for (int64_t r = rows * k / nth; r < rows * (k + 1) / nth; ++r) {
+                const char* row = (const char*)src.counts + (size_t)r * (size_t)P * word;
+                char* dst = hb + (size_t)r * (size_t)H * word;
+                for (int64_t h = 0; h < H; ++h) memcpy(dst + (size_t)h * word, row + (size_t)site_slot[h] * word, word);
+            }
+        };
+        std::vector<std::thread> th;
+        for (int k = 1; k < nth; ++k) th.emplace_back(work, k);
+        work(0);
+        for (auto& x : th) x.join();
+    }
+    uint16_t* ra = (uint16_t*)(hb + o_ra);
+    float* thr = (float*)(hb + o_thr);
+    for (int64_t h = 0; h < H; ++h) {
+        const int64_t s = site_slot[h], a = site_alt[h];
+        ra[h] = (uint16_t)(ref[s] | (a << 8));
+        for (int32_t i = 0; i < n_c; ++i) {
+            thr[((int64_t)i * H + h) * 2 + 0] = thr_views[(((int64_t)i * P + s) * 4 + a) * 2 + 0];
+            thr[((int64_t)i * H + h) * 2 + 1] = thr_views[(((int64_t)i * P + s) * 4 + a) * 2 + 1];
+        }
+    }
+    clk.lap("sites.gather");
+    // device block: tile [T][2][H][4] | staging (wire formats) | wide | site_ra | thr | out
+    const size_t d_stg = n_words * 16;
+    const size_t d_wide = d_stg + (src.elem == 4 ? 0 : ((n_words * word + 15) & ~(size_t)15));
+    const size_t d_ra = d_wide + wide.size() * sizeof(as_wide_record);
+    const size_t d_out = (d_ra + (h_bytes - o_ra) + 15) & ~(size_t)15;
+    const size_t out_bytes = (size_t)n_c * (size_t)T * (size_t)H * sizeof(as_site_test);
+    CU(c->sites.need(d_out + out_bytes));
+    char* db = (char*)c->sites.p;
+    cudaStream_t st = c->exec_stream;
+    cudaEvent_t ev[5] = {};
+    if (clk.on)
+        for (cudaEvent_t& x : ev) CU(cudaEventCreate(&x));
+    if (clk.on) CU(cudaEventRecord(ev[0], st));
+    CU(cudaMemcpyAsync(db + (src.elem == 4 ? 0 : d_stg), hb, n_words * word, cudaMemcpyHostToDevice, st));
+    if (!wide.empty())
+        CU(cudaMemcpyAsync(db + d_wide, wide.data(), wide.size() * sizeof(as_wide_record), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(db + d_ra, hb + o_ra, h_bytes - o_ra, cudaMemcpyHostToDevice, st));
+    if (clk.on) CU(cudaEventRecord(ev[1], st));
+    if (src.elem != 4) {
+        CU(src.elem == 2 ? as_launch_widen16((const uint16_t*)(db + d_stg), (uint32_t*)db, (int64_t)n_words, st)
+                         : as_launch_unpack((const uint32_t*)(db + d_stg), (uint32_t*)db, (int64_t)n_words, st));
+        c->launches += 1;
+        if (!wide.empty()) {
+            CU(as_launch_patch_wide((const as_wide_record*)(db + d_wide), (int64_t)wide.size(), (uint32_t*)db, H, 0, T, st));
+            c->launches += 1;
+        }
+    }
+    if (clk.on) CU(cudaEventRecord(ev[2], st));
+    CU(as_launch_site_test((const uint32_t*)db, T, (int)H, (const uint16_t*)(db + d_ra), (const float*)(db + d_ra + (o_thr - o_ra)), n_c,
+                           (uint32_t)cut, (as_site_test*)(db + d_out), st));
+    c->launches += 1;
+    if (clk.on) CU(cudaEventRecord(ev[3], st));
+    CU(cudaMemcpyAsync(out, db + d_out, out_bytes, cudaMemcpyDeviceToHost, st));
+    if (clk.on) CU(cudaEventRecord(ev[4], st));
+    CU(cudaStreamSynchronize(st));
+    if (clk.on) {
+        const char* name[4] = {"upload", "expand", "kernel", "download"};
+        for (int i = 0; i < 4; ++i) {
+            float ms = 0.f;
+            CU(cudaEventElapsedTime(&ms, ev[i], ev[i + 1]));
+            fprintf(stderr, "AS_TIMING capi.sites.%s_event %.6f\n", name[i], ms * 1e-3);
+        }
+        for (cudaEvent_t x : ev) cudaEventDestroy(x);
+    }
+    clk.lap("sites.device");
+    return AS_OK;
+}
+
+int as_site_tests_host(as_ctx* c, const uint32_t* counts, int32_t T, int64_t P, const uint8_t* ref, const float* thr_views,
+                       int32_t n_c, const int32_t* site_slot, const int32_t* site_alt, int64_t n_sites, int32_t cut, as_site_test* out) {
+    const HostSrc src{counts, 4, nullptr, 0};
+    return site_tests_impl(c, src, T, P, ref, thr_views, n_c, site_slot, site_alt, n_sites, cut, out);
+}
+int as_site_tests_host16(as_ctx* c, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t T, int64_t P,
+                         const uint8_t* ref, const float* thr_views, int32_t n_c, const int32_t* site_slot, const int32_t* site_alt,
+                         int64_t n_sites, int32_t cut, as_site_test* out) {
+    const HostSrc src{counts, 2, wide, n_wide};
+    return site_tests_impl(c, src, T, P, ref, thr_views, n_c, site_slot, site_alt, n_sites, cut, out);
+}
+int as_site_tests_host_packed(as_ctx* c, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T, int64_t P,
+                              const uint8_t* ref, const float* thr_views, int32_t n_c, const int32_t* site_slot,
+                              const int32_t* site_alt, int64_t n_sites, int32_t cut, as_site_test* out) {
+    const HostSrc src{packed, 1, wide, n_wide};
+    return site_tests_impl(c, src, T, P, ref, thr_views, n_c, site_slot, site_alt, n_sites, cut, out);
 }
 
 // Device call list -> the reference's row order (sample, slot, alt), on the device (radix sort of 64-bit keys + row gather).

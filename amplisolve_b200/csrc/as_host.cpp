@@ -14,6 +14,7 @@
 #include <algorithm>
 #include <atomic>
 #include <clocale>
+#include <cerrno>
 #include <cmath>
 #include <condition_variable>
 #include <cstdint>
@@ -1501,6 +1502,12 @@ void usage_vc() {
               << std::endl;
     std::cout << "\n\tIt is important to give the arguments in this order. Otherwise the program will crach !" << std::endl;
     usage_bam();
+    std::cout << "\tAn optional sixth argument " << GREEN << "sites=" << RESET << "/listed/SNVs.vcf writes <output_dir>/Site_Report.txt: the\n"
+                 "\tstrand tests of every listed SNV in every tumour, called or not.  The file is VCF-like: '#' lines are skipped,\n"
+                 "\tcolumns are CHROM POS ID REF ALT..., tab-separated; ALT may list several bases (A,T); records whose REF or ALT is\n"
+                 "\tnot one base are skipped.  A site is tested at the first panel slot of its position.  Status: CALLED,\n"
+                 "\tNOT_CALLED, LOW_COVERAGE, NO_DATA, NOT_TESTABLE, NOT_IN_PANEL or REF_MISMATCH."
+              << std::endl;
     std::cout << STARS << std::endl;
 }
 
@@ -2018,13 +2025,126 @@ void parse_noise_table(const std::string& text, int force_pieces, Panel& panel, 
     for (Piece& pc : pieces) dummy_pieces.push_back(std::move(pc.dummy));
 }
 
+// ---------------------------------------------------------------------------------------------------
+// sites=<file> of the variant-calling program: listed SNVs whose strand tests are reported for every tumour, called or not
+// (Site_Report.txt).  VCF-like text: '#' lines are skipped, columns are CHROM POS ID REF ALT..., tab-separated, so a
+// program's own <sample>.vcf or a hotspot list is read as is; an ALT list "A,T" gives one site per base.
+// ---------------------------------------------------------------------------------------------------
+enum { SITE_NOT_IN_PANEL = 6, SITE_REF_MISMATCH = 7 };  // statuses set on the host, after the AS_SITE_* of the device
+const char* site_status_text(int32_t st) {
+    switch (st) {
+        case AS_SITE_CALLED: return "CALLED";
+        case AS_SITE_NOT_CALLED: return "NOT_CALLED";
+        case AS_SITE_LOW_COVERAGE: return "LOW_COVERAGE";
+        case AS_SITE_NO_DATA: return "NO_DATA";
+        case AS_SITE_NOT_TESTABLE: return "NOT_TESTABLE";
+        case SITE_NOT_IN_PANEL: return "NOT_IN_PANEL";
+        default: return "REF_MISMATCH";
+    }
+}
+
+struct SiteList {
+    std::vector<std::string> chrom, pos_text;  // as the file writes them
+    std::vector<long> pos;
+    std::vector<char> ref, alt;
+    // resolve_sites: the first panel slot of the site's position, the status set on the host (0: tested on the device) and
+    // the site's index among the tested ones
+    std::vector<int32_t> slot, host_status, dev;
+    std::vector<int32_t> dev_slot, dev_alt;  // the tested sites
+};
+
+// 0 ok, 1 the file cannot be opened, 2 a malformed line (reported)
+int load_sites(const std::string& path, SiteList& sl) {
+    std::string text;
+    if (!read_file(path, text)) return 1;
+    auto split = [](const std::string& s, char sep, size_t max_parts) {
+        std::vector<std::string> v;
+        for (size_t a = 0;;) {
+            const size_t b = v.size() + 1 == max_parts ? std::string::npos : s.find(sep, a);
+            v.push_back(s.substr(a, b == std::string::npos ? std::string::npos : b - a));
+            if (b == std::string::npos) return v;
+            a = b + 1;
+        }
+    };
+    auto base = [](const std::string& b) { return b.size() == 1 && strchr("ACGT", b[0]) != nullptr; };
+    size_t line = 0;
+    for (size_t p = 0; p < text.size();) {
+        size_t e = text.find('\n', p);
+        if (e == std::string::npos) e = text.size();
+        std::string ln = text.substr(p, e - p);
+        p = e + 1;
+        ++line;
+        if (!ln.empty() && ln.back() == '\r') ln.pop_back();
+        if (ln.empty() || ln[0] == '#') continue;
+        const std::vector<std::string> col = split(ln, '\t', 6);
+        if (col.size() < 5) {
+            printf("Error: %s line %zu has fewer than five tab-separated columns (CHROM POS ID REF ALT)\n", path.c_str(), line);
+            return 2;
+        }
+        char* end = nullptr;
+        errno = 0;
+        const long pos = strtol(col[1].c_str(), &end, 10);
+        if (col[1].empty() || *end != '\0' || errno != 0) {
+            printf("Error: %s line %zu: POS \"%s\" is not an integer\n", path.c_str(), line, col[1].c_str());
+            return 2;
+        }
+        const std::vector<std::string> alt = split(col[4], ',', 0);
+        bool snv = base(col[3]);
+        for (const std::string& x : alt) snv = snv && base(x);
+        if (!snv) {
+            std::cout << "Warning: " << path << " line " << line << ": REF or ALT is not a single base (A, C, G, T); record skipped"
+                      << std::endl;
+            continue;
+        }
+        for (const std::string& x : alt) {
+            sl.chrom.push_back(col[0]);
+            sl.pos_text.push_back(col[1]);
+            sl.pos.push_back(pos);
+            sl.ref.push_back(col[3][0]);
+            sl.alt.push_back(x[0]);
+        }
+    }
+    return 0;
+}
+
+// Sites -> panel slots: CHROM is matched as text against the noise table's names; a site is tested at the FIRST slot of its
+// position (rows beyond a position's slots are not reported) and its REF must be the panel's reference text.
+void resolve_sites(const Panel& panel, SiteList& sl) {
+    const size_t n = sl.chrom.size();
+    sl.slot.assign(n, -1);
+    sl.host_status.assign(n, 0);
+    sl.dev.assign(n, -1);
+    for (size_t i = 0; i < n; ++i) {
+        const int32_t c = panel.find_chrom(sl.chrom[i].data(), sl.chrom[i].size());
+        const int32_t s = (c < 0 || sl.pos[i] != (long)(int32_t)sl.pos[i]) ? -1 : panel.lookup(c, (int32_t)sl.pos[i]);
+        if (s < 0) { sl.host_status[i] = SITE_NOT_IN_PANEL; continue; }
+        sl.slot[i] = s;
+        if (panel.ref[(size_t)s] != std::string(1, sl.ref[i])) { sl.host_status[i] = SITE_REF_MISMATCH; continue; }
+        sl.dev[i] = (int32_t)sl.dev_slot.size();
+        sl.dev_slot.push_back(s);
+        sl.dev_alt.push_back((int32_t)(strchr("ACGT", sl.alt[i]) - "ACGT"));
+    }
+}
+
+// A row whose RD column is not A+C+G+T: the reference's forward-strand test takes (alt_fw, RD - reverse reads) (VC:895),
+// so the row goes to the device with the reference base's forward count absorbing the difference (alt counts untouched).
+// False when the column is too small for that (rb = the slot's reference base, 0..3).
+bool rd_column_forward(const AseqStats::ExtraRow& x, uint8_t rb, uint32_t& ref_fw) {
+    long long FW = 0, BW = 0;
+    for (int b = 0; b < 4; ++b) { FW += x.fw[b]; BW += x.bw[b]; }
+    const long long v = (long long)x.fw[rb] + (x.rd - (FW + BW));
+    if (v < 0 || x.rd - BW < 1) return false;
+    ref_fw = (uint32_t)v;
+    return true;
+}
+
 }  // namespace
 
 // ===================================================================================================
 // AmpliSolveVariantCalling (VC:199-360, VC:430-576, VC:633-3304)
 // ===================================================================================================
 int as_variant_calling_main(int argc, char** argv) {
-    if (argc != 6) {
+    if ((argc != 6 && argc != 7) || (argc == 7 && strncmp(argv[6], "sites=", 6) != 0)) {
         std::cout << STARS << std::endl;
         std::cout << RED << "                                        Your input arguments are not correct !" << RESET << std::endl;
         std::cout << "                         amplisolve_b200 (B200-native AmpliSolveVariantCalling, argv-compatible)\n" << std::endl;
@@ -2036,6 +2156,7 @@ int as_variant_calling_main(int argc, char** argv) {
     const std::string output_dir = arg_value(argv[3], "output_dir=");
     const std::string coverage_cutoff = arg_value(argv[4], "coverage_cutoff=");
     const std::string p_value = arg_value(argv[5], "p_value=");
+    const std::string sites_file = argc == 7 ? arg_value(argv[6], "sites=") : std::string();
     float p_value_float = (float)atof(p_value.c_str());  // VC:263
     int cut = atoi(coverage_cutoff.c_str());
 
@@ -2064,7 +2185,17 @@ int as_variant_calling_main(int argc, char** argv) {
     if (bam_input_dir(tumour_dir))
         std::cout << "\t6. BAM pileup (AS_BAM_MBQ / AS_BAM_MRQ / AS_BAM_MDC) : " << GREEN << bam.mbq << " / " << bam.mrq << " / " << bam.mdc
                   << RESET << std::endl;
+    if (argc == 7)
+        std::cout << "\t" << (bam_input_dir(tumour_dir) ? 7 : 6) << ". Sites (Site_Report.txt)                        : " << GREEN << sites_file
+                  << RESET << std::endl;
     std::cout << std::endl;
+    // sites=<file>: read before anything is written, so that a malformed file leaves no output behind
+    SiteList sites;
+    if (argc == 7) {
+        const int src = load_sites(sites_file, sites);
+        if (src == 1) printf("Error from the sites file: Cannot open %s\n", sites_file.c_str());
+        if (src != 0) return 0;
+    }
 
     // errorFile=<directory>: a noise-floor sweep over every positionSpecificNoise_*.txt in it, in name order.  Table X.txt
     // writes to <output_dir>/X/ what errorFile=<directory>/X.txt output_dir=<output_dir>/X writes alone; the tumours are
@@ -2173,6 +2304,16 @@ int as_variant_calling_main(int argc, char** argv) {
         }
     }
     std::cout << "Running function storeInputFile: the error levels have stored with success " << P << RESET << std::endl;
+    resolve_sites(panel, sites);
+    const int64_t HS = (int64_t)sites.dev_slot.size();  // sites tested on the device
+    // Site_Report.txt of every table, rows appended group by group (tumours in the summary's order, sites in file order)
+    std::vector<std::ofstream> site_reports;
+    if (argc == 7)
+        for (size_t k = 0; k < NT; ++k) {
+            site_reports.emplace_back((out_dirs[k] + "/Site_Report.txt").c_str());
+            site_reports.back() << "Filename\tChrom\tPosition\tRef\tAlt\tRD_fw\tRD_bw\tReads_fw\tReads_bw\tAF\tNoise_fw\tNoise_bw\tQscore_fw\t"
+                                   "Qscore_bw\tStatus\n";
+        }
     std::vector<uint8_t> ref_code((size_t)P, 255);
     for (int64_t i = 0; i < P; ++i) {
         const std::string& r = panel.ref[i];
@@ -2251,6 +2392,8 @@ int as_variant_calling_main(int argc, char** argv) {
             parse_s += PhaseTimer::now() - t0;
             return lrc;
         };
+        std::unordered_map<int32_t, std::vector<int32_t>> sites_at;  // slot -> the tested sites there
+        for (int64_t h = 0; h < HS; ++h) sites_at[sites.dev_slot[(size_t)h]].push_back((int32_t)h);
         int lrc = load_group(0, 0);
         if (lrc == 1) return report_gpu_error("pinned host allocation");
         if (lrc >= 2) return 0;  // 3: a BAM that cannot be read, reported like an ASEQ file that cannot be opened
@@ -2265,8 +2408,10 @@ int as_variant_calling_main(int argc, char** argv) {
             }
             // GPU step of this group on a worker thread (passes of up to 8 tables) ...
             std::vector<std::vector<as_call>> parts(NT);
+            std::vector<as_site_test> site_part;  // [NT][Tg][HS]
             int rc = AS_OK;
             std::string gpu_error;
+            const char* gpu_what = "as_call_variants_host";
             const HostCounts& hc = buf[which];
             std::thread worker([&]() {
                 const double t0 = PhaseTimer::now();
@@ -2290,6 +2435,21 @@ int as_variant_calling_main(int argc, char** argv) {
                         for (int32_t i = 0; i < nc; ++i)
                             parts[c0 + (size_t)i].assign(list.begin() + (long)(i * cap), list.begin() + (long)(i * cap + n_part[i]));
                 }
+                // the listed sites of this group, while its buffer is valid: all tables in one kernel pass per 8
+                if (rc == AS_OK && HS > 0) {
+                    site_part.resize(NT * (size_t)Tg * (size_t)HS);
+                    for (size_t c0 = 0; c0 < NT && rc == AS_OK; c0 += 8) {
+                        const int32_t nc = (int32_t)std::min<size_t>(8, NT - c0);
+                        const float* tv = thr_view.data() + c0 * (size_t)P * 8;
+                        as_site_test* o = site_part.data() + c0 * (size_t)Tg * (size_t)HS;
+                        rc = hc.fmt == 2 ? as_site_tests_host16(ctx, (const uint16_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(), Tg, P,
+                                                                ref_code.data(), tv, nc, sites.dev_slot.data(), sites.dev_alt.data(), HS, cut, o)
+                                         : as_site_tests_host_packed(ctx, (const uint32_t*)hc.p, hc.wide.data(), (int64_t)hc.wide.size(), Tg,
+                                                                     P, ref_code.data(), tv, nc, sites.dev_slot.data(), sites.dev_alt.data(),
+                                                                     HS, cut, o);
+                    }
+                    if (rc != AS_OK) gpu_what = "as_site_tests_host";
+                }
                 if (rc != AS_OK) gpu_error = as_last_error();
                 gpu_s += PhaseTimer::now() - t0;
             });
@@ -2298,7 +2458,7 @@ int as_variant_calling_main(int argc, char** argv) {
             if (first + G < T) next_rc = load_group(first + G, which ^ 1);
             worker.join();
             if (rc != AS_OK) {
-                std::cout << RED << "Error: as_call_variants_host: " << gpu_error << RESET << std::endl;
+                std::cout << RED << "Error: " << gpu_what << ": " << gpu_error << RESET << std::endl;
                 return 1;
             }
             if (next_rc == 1) return report_gpu_error("pinned host allocation");
@@ -2326,14 +2486,14 @@ int as_variant_calling_main(int argc, char** argv) {
                     for (int b = 0; b < 4; ++b) { FW += x.fw[b]; BW += x.bw[b]; }
                     const uint8_t rb = ref_code[(size_t)x.slot];
                     if (FW < cut || BW < cut || rb > 3) continue;  // VC:898 / VC:3290: never a call
-                    const long long ref_fw = (long long)x.fw[rb] + (x.rd - (FW + BW));
-                    if (ref_fw < 0 || x.rd - BW < 1) {
+                    uint32_t ref_fw = 0;
+                    if (!rd_column_forward(x, rb, ref_fw)) {
                         std::cout << "Warning: " << files[(size_t)pr.first].path << " row " << x.row + 2
                                   << ": RD column smaller than the alt reads; row skipped" << std::endl;
                         continue;
                     }
                     use.push_back(pr);
-                    fwadj.push_back((uint32_t)ref_fw);
+                    fwadj.push_back(ref_fw);
                 }
                 const int64_t M = (int64_t)use.size();
                 std::vector<uint32_t> xc((size_t)M * 8 + 4);
@@ -2416,6 +2576,95 @@ int as_variant_calling_main(int argc, char** argv) {
                     std::copy(k2.begin(), k2.end(), call_counts.begin() + (long)base);
                     std::copy(r2.begin(), r2.end(), call_row.begin() + (long)base);
                     std::copy(d2.begin(), d2.end(), call_rd.begin() + (long)base);
+                }
+            }
+            if (!site_reports.empty()) {
+                // a site whose row was set aside because its RD column is not A+C+G+T (extras with k = -1: the tensor holds
+                // no record there) is tested as the extra-row pass tests that row: forward depth RD - reverse reads
+                // (rd_column_forward), cutoff 1 on the device, the coverage gate on the sums (VC:898) here
+                struct SetAside { int32_t i; const AseqStats::ExtraRow* x; bool ok; };
+                std::vector<SetAside> aside;
+                std::vector<int32_t> a_slot, a_alt, a_entry;  // per tested entry: mini-tensor slot, alt, index into aside
+                for (int i = 0; i < Tg && !sites_at.empty(); ++i)
+                    for (const AseqStats::ExtraRow& x : file_stats[(size_t)(first + i)].extras) {
+                        auto it = sites_at.find(x.slot);
+                        if (x.k >= 0 || it == sites_at.end()) continue;
+                        const int32_t m = (int32_t)aside.size();
+                        uint32_t ref_fw = 0;
+                        const uint8_t rb = ref_code[(size_t)x.slot];
+                        aside.push_back(SetAside{i, &x, rb > 3 || rd_column_forward(x, rb, ref_fw)});
+                        for (int32_t h : it->second) { a_slot.push_back(m); a_alt.push_back(h); }
+                    }
+                const int64_t M = (int64_t)aside.size(), NA = (int64_t)a_slot.size();
+                if (M > 0) {
+                    std::vector<uint32_t> xc((size_t)M * 8 + 4);
+                    uint32_t* xcp = (uint32_t*)(((uintptr_t)xc.data() + 15) & ~(uintptr_t)15);
+                    std::vector<uint8_t> xref((size_t)M);
+                    std::vector<float> xthr(NT * (size_t)M * 8);  // [NT][M][4][2]
+                    for (int64_t m = 0; m < M; ++m) {
+                        const AseqStats::ExtraRow& x = *aside[(size_t)m].x;
+                        memcpy(xcp + m * 4, x.fw, 16);
+                        memcpy(xcp + (M + m) * 4, x.bw, 16);
+                        xref[(size_t)m] = ref_code[(size_t)x.slot];
+                        uint32_t ref_fw = 0;
+                        if (xref[(size_t)m] <= 3 && rd_column_forward(x, xref[(size_t)m], ref_fw)) xcp[m * 4 + xref[(size_t)m]] = ref_fw;
+                        for (size_t k = 0; k < NT; ++k)
+                            memcpy(&xthr[(k * (size_t)M + (size_t)m) * 8], &thr_view[(k * (size_t)P + (size_t)x.slot) * 8], 32);
+                    }
+                    std::vector<int32_t> alt_of((size_t)NA);
+                    for (int64_t j = 0; j < NA; ++j) alt_of[(size_t)j] = sites.dev_alt[(size_t)a_alt[(size_t)j]];
+                    std::vector<as_site_test> xo(NT * (size_t)NA);
+                    for (size_t c0 = 0; c0 < NT; c0 += 8) {
+                        const int32_t nc = (int32_t)std::min<size_t>(8, NT - c0);
+                        if (as_site_tests_host(ctx, xcp, 1, M, xref.data(), xthr.data() + c0 * (size_t)M * 8, nc, a_slot.data(), alt_of.data(),
+                                               NA, 1, xo.data() + c0 * (size_t)NA) != AS_OK)
+                            return report_gpu_error("as_site_tests_host");
+                    }
+                    for (size_t k = 0; k < NT; ++k)
+                        for (int64_t j = 0; j < NA; ++j) {
+                            const SetAside& a = aside[(size_t)a_slot[(size_t)j]];
+                            as_site_test r = xo[k * (size_t)NA + (size_t)j];
+                            long long FW = 0, BW = 0;
+                            for (int b = 0; b < 4; ++b) { FW += a.x->fw[b]; BW += a.x->bw[b]; }
+                            if (!a.ok) {  // the RD column is smaller than the alt reads: the caller skips the row (warning above)
+                                r.status = AS_SITE_NOT_TESTABLE;
+                                r.p_fw = r.p_bw = std::nan("");
+                            } else if (r.status != AS_SITE_NOT_TESTABLE && (FW < cut || BW < cut)) {
+                                r.status = AS_SITE_LOW_COVERAGE;
+                            }
+                            site_part[(k * (size_t)Tg + (size_t)a.i) * (size_t)HS + (size_t)a_alt[(size_t)j]] = r;
+                        }
+                }
+                // rows of this group: tumours in order, sites in file order
+                for (size_t k = 0; k < NT; ++k) {
+                    std::ostringstream os;
+                    os << std::setprecision(4);
+                    const float* tv = thr_view.data() + k * (size_t)P * 8;
+                    char nf[64], nb[64];
+                    for (int i = 0; i < Tg; ++i)
+                        for (size_t j = 0; j < sites.chrom.size(); ++j) {
+                            os << files[(size_t)(first + i)].sample << "\t" << sites.chrom[j] << "\t" << sites.pos_text[j] << "\t" << sites.ref[j]
+                               << "\t" << sites.alt[j] << "\t";
+                            int32_t st = sites.host_status[j];
+                            const as_site_test* r = st ? nullptr : &site_part[(k * (size_t)Tg + (size_t)i) * (size_t)HS + (size_t)sites.dev[j]];
+                            if (r) st = r->status;
+                            if (!r || st == AS_SITE_NO_DATA) {
+                                os << "-\t-\t-\t-\t-\t-\t-\t-\t-\t";
+                            } else {
+                                const uint32_t depth = r->depth_fw + r->depth_bw, reads = r->alt_fw + r->alt_bw;
+                                const float* e = tv + (size_t)sites.slot[j] * 8 + (size_t)sites.dev_alt[(size_t)sites.dev[j]] * 2;
+                                snprintf(nf, sizeof nf, "%f", (double)e[0]);
+                                snprintf(nb, sizeof nb, "%f", (double)e[1]);
+                                os << r->depth_fw << "\t" << r->depth_bw << "\t" << r->alt_fw << "\t" << r->alt_bw << "\t"
+                                   << (depth == 0 ? 0.f : float(reads) / float(depth)) << "\t" << nf << "\t" << nb << "\t";
+                                for (double pv : {r->p_fw, r->p_bw}) {  // Q as the summary prints it (VC:895-896, VC:1066)
+                                    if (std::isnan(pv)) os << "-\t";
+                                    else os << std::setprecision(4) << q_from_p(pv) << "\t";
+                                }
+                            }
+                            os << site_status_text(st) << "\n";
+                        }
+                    site_reports[k] << os.str();
                 }
             }
         }

@@ -79,6 +79,9 @@ cudaError_t as_launch_pileup(const uint8_t* d_rec, const int64_t* d_rec_off, int
 cudaError_t as_launch_pileup_encode(int fmt, const uint32_t* d_counts, int64_t U, const int32_t* d_slot_unique, int64_t P,
                                     int32_t mdc, int32_t sample, void* d_wire, as_wide_record* d_wide, int64_t cap,
                                     unsigned long long* d_n, cudaStream_t st);
+// as_sites.cu: site_test_kernel over counts [T][2][H][4]; site_ra[h] = ref | alt << 8, thr [n_c][H][2], out [n_c][T][H]
+cudaError_t as_launch_site_test(const uint32_t* d_counts, int T, int H, const uint16_t* d_site_ra, const float* d_thr, int n_c,
+                                uint32_t cut, as_site_test* d_out, cudaStream_t st);
 cudaError_t as_launch_poisson_test(const int32_t* k, const int32_t* rd, const float* err, int64_t n, double* p,
                                    double* q, cudaStream_t st);
 cudaError_t as_launch_gammaq(const double* s, const double* z, int64_t n, double* out, cudaStream_t st);

@@ -268,6 +268,46 @@ int as_call_variants_sweep_host_packed(as_ctx* ctx, const uint32_t* packed, cons
  * every rank's compacted list is sent to one rank (exact sizes), concatenated and sorted there (amplisolve_b200/shard.py). */
 int as_sort_calls_dev(as_ctx* ctx, as_call* d_calls, int64_t n, int32_t slot_offset, as_call* d_sorted, void* stream);
 
+/* ---- site report: the strand tests of listed SNVs in every tumour, called or not -------------------------------------
+ * The reference evaluates mutationRulesPoissonQualityScore (VC:3834-3884, over the kfunc incomplete gamma VC:3720-3830 with
+ * both branches and their 99-step caps) for both strands of every row and alt (VC:895-896) and applies the decision of VC:898
+ * afterwards; the caller entry points above keep only the calls.  These entry points keep every test of the listed sites:
+ * site i is (site_slot[i], site_alt[i]), and for every table c and tumour t, out[(c * T + t) * n_sites + i] holds the record's
+ * strand depths (the sums of the four counts, VC:760-770), the alt reads, p_fw / p_bw = the double p of VC:3858-3866 on the
+ * caller view of table c (1 when k = 0; no screen: the p of every present, testable record, whatever its coverage) and one
+ * of the statuses below.  AS_SITE_CALLED is exactly the decision of the caller entry points (same device arithmetic):
+ * present, FW >= cut and BW >= cut, ref in 0..3, alt != ref and both strands reach Q >= 5.
+ * p is NaN where it is not evaluated (NO_DATA, NOT_TESTABLE, and a threshold of -1, whose Q is the reference's -888); the
+ * counts of a NO_DATA entry are 0. */
+#define AS_SITE_CALLED 1       /* the caller calls (tumour, slot, alt) with this table */
+#define AS_SITE_NOT_CALLED 2   /* present and covered; a strand's Q is below 5 */
+#define AS_SITE_LOW_COVERAGE 3 /* present, FW < cut or BW < cut (VC:898); p is still evaluated */
+#define AS_SITE_NO_DATA 4      /* the record is absent (no ASEQ row) */
+#define AS_SITE_NOT_TESTABLE 5 /* the slot's reference base is not A/C/G/T (VC:3290-3293), or alt = ref */
+typedef struct {
+    uint32_t depth_fw, depth_bw; /* FW, BW of VC:760-770 */
+    uint32_t alt_fw, alt_bw;     /* alt reads per strand */
+    double p_fw, p_bw;           /* VC:3858-3866 per strand (VC:895-896) */
+    int32_t status;              /* AS_SITE_* */
+    int32_t pad;
+} as_site_test; /* 40 bytes */
+/* counts [T][2][P][4] (+ wide, n_wide) in any of the three host formats, ref [P] and thr_views [n_c][P][4][2] exactly as
+ * as_call_variants_sweep_host* take them; site_slot / site_alt [n_sites]; out [n_c][T][n_sites].  1 <= n_c <= 8, every
+ * slot in [0, P) and every alt in 0..3, else AS_EINVAL; n_sites = 0 or T = 0 return AS_OK with nothing written.  The host
+ * gathers the sites' columns of counts in their format (escaped records follow, renumbered by site) and uploads them as a
+ * count tensor of n_sites slots, which the wire-format path widens on the device; site_test_kernel (as_sites.cu) then
+ * evaluates every (table, site, tumour, strand).  A multi-device context runs this on its first device: the work is the
+ * sites' columns, not the panel. */
+int as_site_tests_host(as_ctx* ctx, const uint32_t* counts, int32_t T, int64_t P, const uint8_t* ref, const float* thr_views,
+                       int32_t n_c, const int32_t* site_slot, const int32_t* site_alt, int64_t n_sites, int32_t cut,
+                       as_site_test* out);
+int as_site_tests_host16(as_ctx* ctx, const uint16_t* counts, const as_wide_record* wide, int64_t n_wide, int32_t T, int64_t P,
+                         const uint8_t* ref, const float* thr_views, int32_t n_c, const int32_t* site_slot, const int32_t* site_alt,
+                         int64_t n_sites, int32_t cut, as_site_test* out);
+int as_site_tests_host_packed(as_ctx* ctx, const uint32_t* packed, const as_wide_record* wide, int64_t n_wide, int32_t T, int64_t P,
+                              const uint8_t* ref, const float* thr_views, int32_t n_c, const int32_t* site_slot,
+                              const int32_t* site_alt, int64_t n_sites, int32_t cut, as_site_test* out);
+
 /* Element-wise Poisson test on the device: p[i] = the double p-value of VC:3858-3866 and
  * q[i] = the Q score of VC:3868-3882 for (k[i], rd[i], err[i]).  Host pointers.  Used by the
  * parity tests to compare the device incomplete gamma with the reference's on arbitrary grids. */
