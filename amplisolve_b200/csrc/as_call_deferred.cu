@@ -331,13 +331,15 @@ call_series_kernel(DeferredLists L, CallSink sink) {
 
 using namespace asdev;
 
-size_t as_deferred_scratch_bytes(int T, int64_t n_slots, int64_t* cap_cand, int64_t* cap_surv) {
+size_t as_deferred_scratch_bytes(int T, int64_t n_slots, int64_t cap_override, int64_t* cap_cand, int64_t* cap_surv) {
     // candidates: a few per thousand (record, alt) pairs on real panels; room for one record in 24, within 1 Mi .. 64 Mi
     // entries (1.5 GB).  Survivors: a quarter of that.  Whatever does not fit is resolved inline by the kernels.
+    // cap_override > 0 sets the candidate capacity (a quarter of it, at least 1, for the survivors): the scratch is sized
+    // for the capacities in use, whichever way they were chosen.
     int64_t cc = (int64_t)T * n_slots / 24;
-    cc = std::max<int64_t>(1 << 20, std::min<int64_t>(cc, 64ll << 20));
+    cc = cap_override > 0 ? cap_override : std::max<int64_t>(1 << 20, std::min<int64_t>(cc, 64ll << 20));
     *cap_cand = cc;
-    *cap_surv = std::max<int64_t>(1 << 18, cc / 4);  // per table
+    *cap_surv = cap_override > 0 ? std::max<int64_t>(1, cc / 4) : std::max<int64_t>(1 << 18, cc / 4);  // per table
     return 4096 + (size_t)cc * sizeof(StagedCand) + 8 * (size_t)*cap_surv * sizeof(Survivor) + 512 * AS_DEFER_MAX_CHUNKS;
 }
 

@@ -743,8 +743,7 @@ static int call_deferred(as_ctx* c, const uint32_t* d_counts, int32_t T, int64_t
                          const float* d_thr_views, int32_t n_c, int64_t c_stride, int32_t cut, as_call* d_calls, int64_t cap,
                          unsigned long long* d_n_calls, cudaStream_t st) {
     int64_t cap_cand = 0, cap_surv = 0;
-    const size_t bytes = as_deferred_scratch_bytes(T, e - b, &cap_cand, &cap_surv) + 256;
-    if (c->defer_cap_override > 0) { cap_cand = c->defer_cap_override; cap_surv = std::max<int64_t>(1, cap_cand / 4); }
+    const size_t bytes = as_deferred_scratch_bytes(T, e - b, c->defer_cap_override, &cap_cand, &cap_surv) + 256;
     CU(c->defer.need(bytes));
     CU(as_launch_call_deferred(d_counts, T, P, b, e, d_ref, d_thr_views, n_c, c_stride, (uint32_t)cut, d_calls, cap, d_n_calls, c->defer.p,
                                cap_cand, cap_surv, st, c->aux_stream, c->ev_chunk, c->defer_chunks));

@@ -34,13 +34,14 @@ cudaError_t as_launch_noise_twin_groups(const uint32_t* d_counts, int S, int64_t
                                         float C, uint32_t cut, float* d_thr, float* d_germ_val, uint8_t* d_germ_state,
                                         uint32_t* d_count, uint32_t* d_nrec, cudaStream_t st);
 // as_noise_pattern.cu: every output of the noise model for n_c (1..8) values of C in ONE pass over the normals; table c at
-// d_thr + c * thr_stride floats.  geom selects the ring: 0 = (4 samples, 3 stages), 1 = (3, 3), 2 = (4, 2).
+// d_thr + c * thr_stride floats.  The ring is (4 samples, 3 stages); geom 0 unrolls the 4 records of a stage, geom 1
+// (n_c = 1 and n_c 4..5 only; others run geom 0) walks them one by one.
 cudaError_t as_launch_noise_pattern(int geom, const uint32_t* d_counts, int S, int64_t P, int64_t p0, int64_t p1,
                                     const int32_t* d_twin_next, const int32_t* d_twin_head, int64_t twin_base,
                                     const float* c_values, int n_c, uint32_t cut, float* d_thr, int64_t thr_stride,
                                     float* d_germ_val, uint8_t* d_germ_state, uint32_t* d_count, uint32_t* d_nrec, cudaStream_t st);
 // as_call_deferred.cu: the caller as scan -> resolve -> series kernels over candidate / survivor lists in d_scratch
-size_t as_deferred_scratch_bytes(int T, int64_t n_slots, int64_t* cap_cand, int64_t* cap_surv);
+size_t as_deferred_scratch_bytes(int T, int64_t n_slots, int64_t cap_override, int64_t* cap_cand, int64_t* cap_surv);
 #define AS_DEFER_MAX_CHUNKS 8
 int as_deferred_chunks(int64_t n_slots, int want);
 cudaError_t as_launch_call_deferred(const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1, const uint8_t* d_ref,
