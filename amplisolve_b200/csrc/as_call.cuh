@@ -1,5 +1,5 @@
-// Device helpers shared by the caller kernels (as_kernels.cu: in-stage caller; as_call_deferred.cu: scan / resolve /
-// series pipeline): the two exact screens, the integer pre-screen of the scan and the survivor entry.
+// Device helpers shared by the caller kernels (as_kernels.cu: in-stage and forward-first callers; as_call_deferred.cu:
+// scan / resolve / series pipeline): the two exact screens, the integer pre-screen of the scan and the survivor entry.
 //   VC = source_codes/AmpliSolveVariantCalling.cpp of the reference.
 #pragma once
 #include "as_device.cuh"
@@ -52,11 +52,12 @@ __device__ __forceinline__ bool strand_can_pass(uint32_t k, uint32_t depth, floa
 //   K = floor(m16/16 + 9/16) when that is <= 64: m >= K - 9/16 >= m*(K)(1 + 1e-9) = AS_MCRIT[K-1] (checked for K = 1..64 in
 //       tests/test_host_cpu.py), the critical-mean screen of strand_can_pass;
 //   K = floor(m16/16) otherwise: m >= k and m > 1, the continued-fraction screen.
+// floor((m16 + 9) / 16) <= 64 exactly when m16 <= 1030, so the two cases are one add under a compare (no overflow: the 9 is
+// only added to small values) -- four instructions per bound, which matters where the scan evaluates one per alt base.
 __device__ __forceinline__ uint32_t prescreen_k(uint32_t depth, uint32_t R) {
     const uint32_t d16 = depth > 0x0FFFFFFFu ? 0xFFFFFFFFu : depth << 4;
     const uint32_t m16 = __umulhi(d16, R);
-    const uint32_t lo = m16 >> 4, hi = lo + (((m16 & 15u) + 9u) >> 4);
-    return hi <= 64u ? hi : lo;
+    return (m16 + (m16 <= 1030u ? 9u : 0u)) >> 4;
 }
 
 // Survivor entry of the staged kernel: 24 bytes (the thresholds are read again from thr_view when the series is

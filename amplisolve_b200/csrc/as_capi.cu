@@ -94,6 +94,7 @@ struct as_ctx {
     int64_t launches = 0;
     int64_t host_tile_slots = 0;  // 0 = automatic
     int64_t defer_cap_override = 0;  // > 0: capacity of the deferred caller's candidate list (tests of the overflow path)
+    int fwd_pending_cap = 0;         // > 0: usable depth of call_forward_kernel's pending ring (tests of its drain path)
     cudaStream_t copy_stream = nullptr, exec_stream = nullptr, aux_stream = nullptr;
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     cudaEvent_t ev_up[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
@@ -272,6 +273,12 @@ int as_set_option(as_ctx* c, const char* name, int64_t value) {
     if (!strcmp(name, "deferred_chunks")) {
         if (value < 1 || value > AS_DEFER_MAX_CHUNKS) return fail(AS_EINVAL, "deferred_chunks must be 1..%d", AS_DEFER_MAX_CHUNKS);
         c->defer_chunks = (int)value;
+        return AS_OK;
+    }
+    if (!strcmp(name, "forward_pending_cap")) {
+        if (value < 0 || value > AS_FWD_PENDING) return fail(AS_EINVAL, "forward_pending_cap must be 0 (automatic) .. %d", AS_FWD_PENDING);
+        c->fwd_pending_cap = (int)value;
+        for (size_t k = 1; k < c->subs.size(); ++k) c->subs[k]->fwd_pending_cap = (int)value;
         return AS_OK;
     }
     if (!strcmp(name, "deferred_capacity")) {
@@ -762,7 +769,7 @@ int as_call_variants_dev(as_ctx* c, const uint32_t* d_counts, int32_t T, int64_t
     if (c->call_variant == AS_DEFERRED_CALL_KERNEL)
         return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_view, 1, P * 8, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
     CU(as_launch_call(c->call_variant, d_counts, T, P, b, e, d_ref, d_thr_view, (uint32_t)cut, d_calls, cap, d_n_calls,
-                      (cudaStream_t)stream));
+                      c->fwd_pending_cap, (cudaStream_t)stream));
     c->launches += 1;
     return AS_OK;
 }
@@ -781,7 +788,7 @@ int as_call_variants_sweep_dev(as_ctx* c, const uint32_t* d_counts, int32_t T, i
     if (c->call_variant == AS_DEFERRED_CALL_KERNEL || (c->call_variant == AS_DEFAULT_CALL_KERNEL && n_c > 1))
         return call_deferred(c, d_counts, T, P, b, e, d_ref, d_thr_views, n_c, P * 8, cut, d_calls, cap, d_n_calls, (cudaStream_t)stream);
     CU(as_launch_call_sweep(c->call_variant, d_counts, T, P, b, e, d_ref, d_thr_views, n_c, P * 8, (uint32_t)cut, d_calls, cap,
-                            d_n_calls, (cudaStream_t)stream));
+                            d_n_calls, c->fwd_pending_cap, (cudaStream_t)stream));
     c->launches += 1;
     return AS_OK;
 }
@@ -844,7 +851,7 @@ static int call_variants_host_range(as_ctx* c, const HostSrc& src, int32_t T, in
                 break;
         } else {
             CUB(as_launch_call_sweep(c->call_variant, d_tile, T, n, 0, n, d_rf_all + (p0 - B), d_tv_all + (p0 - B) * 8, n_c, c_stride,
-                                     (uint32_t)cut, (as_call*)c->calls.p, cap, d_n, c->exec_stream));
+                                     (uint32_t)cut, (as_call*)c->calls.p, cap, d_n, c->fwd_pending_cap, c->exec_stream));
             c->launches += 1;
         }
         if (p0 > 0) {

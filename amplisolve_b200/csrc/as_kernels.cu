@@ -881,6 +881,252 @@ call_staged_kernel(const uint4* __restrict__ counts, int T, int64_t P, int64_t p
     if (n2 > 0) stage2_batch_staged(q2, n2, ref, thr_view, n_c, c_stride, calls, cap, n_calls);
 }
 
+// Forward-first caller.  A record can only become a call if BOTH strand tests pass (VC:898, VC:895-896), and the forward
+// strand alone rules out nearly every record: the ring streams the forward plane only (16 B per record instead of 32).
+// Scan, every record, integer only: present, FW >= cut, and k > prescreen_k(FW, R_min) for some callable base (alt != ref,
+// a threshold on both strands: -1 is never a call, VC:3844-3849), R_min = floor(e * 2^32) of the smallest forward threshold
+// of those bases.  The few records that pass are tested base by base against the base's own bound R_b (what the bound of
+// strand_can_pass is; the minimum is only weaker, and one multiply per record is what keeps the scan lean) before anything
+// is fetched for them.
+// The records with a candidate base are compacted per warp (one prefix sum per stage) into a pending ring in shared
+// memory: the forward word, (sample, column, base mask), and the reverse-strand word, fetched with a 16-byte cp.async that
+// stays in flight while the warp scans the next stages.  The entries of stage i are resolved at stage i + D or later, in
+// batches of at least half a ring, after the stage has been handed back to the producer: BW >= cut, reverse
+// k > prescreen_k(BW, R_b), strand_can_pass on both strands; survivors join the series queue of call_staged_kernel.
+// Nothing in the scan waits on a global read.
+// A ring that cannot take a stage's entries is drained on the spot (wait for every copy, resolve), a slower path that
+// gives the same calls; pend_cap < AS_FWD_PENDING caps the usable depth (tests of that path).
+struct FwdPending {  // per warp; the reverse words are cp.async targets (16-byte aligned)
+    uint4 bw[AS_FWD_PENDING];
+    uint4 fw[AS_FWD_PENDING];
+    uint2 meta[AS_FWD_PENDING];  // sample, tile column | forward candidate base mask << 8
+};
+
+template <int K, int STAGES>
+struct FwdGeom {
+    static constexpr int kSmem = StageRing<K, STAGES, 1>::kStageBytes * STAGES + AS_TILE_SLOTS * (32 + 16 + 8) +
+                                 AS_CONSUMER_WARPS * ((int)sizeof(FwdPending) + AS_Q2_CAP * (int)sizeof(StagedCand));
+    static constexpr int kCtas = (227 * 1024) / (kSmem + 1024) > 8 ? 8 : (227 * 1024) / (kSmem + 1024);
+};
+
+// resolve the n pending entries from ring entry `from` on; full warps, one entry per lane
+__device__ __forceinline__ void fwd_resolve(const FwdPending& pd, uint32_t from, uint32_t n, const float (*thr_s)[8], int64_t tile0,
+                                            uint32_t cut, StagedCand* __restrict__ q2, int& n2, const uint8_t* __restrict__ ref,
+                                            const float* __restrict__ thr_view, as_call* __restrict__ calls, int64_t cap,
+                                            unsigned long long* __restrict__ n_calls) {
+    const int lane = threadIdx.x & 31;
+    for (uint32_t base = 0; base < n; base += 32) {
+        const uint32_t i = base + lane;
+        const uint32_t pos = (from + i) & (AS_FWD_PENDING - 1);
+        uint32_t smask = 0;
+        if (i < n) {
+            const uint4 fw = pd.fw[pos], bw = pd.bw[pos];
+            const uint2 meta = pd.meta[pos];
+            const uint32_t FW = fw.x + fw.y + fw.z + fw.w, BW = bw.x + bw.y + bw.z + bw.w;
+            const uint32_t fm = meta.y >> 8;
+            const float* e = thr_s[meta.y & 255u];
+            if (BW >= cut) {
+#pragma unroll
+                for (int b = 0; b < 4; ++b) {
+                    if ((fm >> b) & 1u) {
+                        const uint32_t kb = comp(bw, b);
+                        const float ee = effective_err(e[2 * b + 1]);
+                        const uint32_t R = (ee > 0.0f && ee < 1.0f) ? __float2uint_rz(ee * 4294967296.0f) : 0u;
+                        if (kb > prescreen_k(BW, R) && strand_can_pass(comp(fw, b), FW, e[2 * b]) && strand_can_pass(kb, BW, e[2 * b + 1]))
+                            smask |= 1u << b;
+                    }
+                }
+            }
+        }
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            const bool surv = (smask >> b) & 1u;
+            const unsigned votes = __ballot_sync(0xffffffffu, surv);
+            if (votes == 0) continue;
+            if (surv) {  // the entry is read again from the ring: nothing of it stays live across the series below
+                const uint4 fw = pd.fw[pos], bw = pd.bw[pos];
+                const uint2 meta = pd.meta[pos];
+                uint2* dst = reinterpret_cast<uint2*>(q2 + n2 + __popc(votes & ((1u << lane) - 1u)));
+                dst[0] = make_uint2(comp(fw, b), fw.x + fw.y + fw.z + fw.w);
+                dst[1] = make_uint2(comp(bw, b), bw.x + bw.y + bw.z + bw.w);
+                dst[2] = make_uint2(meta.x | ((uint32_t)b << 30), (uint32_t)(tile0 + (meta.y & 255u)));
+            }
+            n2 += __popc(votes);
+            __syncwarp();
+            while (n2 >= 16) {
+                stage2_batch_staged(q2 + (n2 - 16), 16, ref, thr_view, 1, 0, calls, cap, n_calls);
+                n2 -= 16;
+                __syncwarp();
+            }
+        }
+    }
+    __syncwarp();  // the entries are read before the ring positions are reused
+}
+
+// entries o in [lo, hi) of this stage (numbered in lane order; this lane's from `first` on) go to ring entry head + o - lo
+__device__ __forceinline__ void fwd_issue(FwdPending& pd, const uint4* st, const uint4* __restrict__ bw_col, int64_t sstride,
+                                          uint32_t mask, uint32_t nz, int first, int lo, int hi, uint32_t head, int t) {
+    const int tid = threadIdx.x;
+    int o = first;
+    while (nz) {
+        const int j = (__ffs(nz) - 1) >> 2;
+        nz &= nz - 1;
+        if (o >= lo && o < hi) {
+            const uint32_t pos = (head + (uint32_t)(o - lo)) & (AS_FWD_PENDING - 1);
+            pd.fw[pos] = st[j * AS_TILE_SLOTS + tid];
+            pd.meta[pos] = make_uint2((uint32_t)(t + j), (uint32_t)tid | (((mask >> (4 * j)) & 15u) << 8));
+            cp_async16(&pd.bw[pos], bw_col + (int64_t)(t + j) * sstride);
+        }
+        ++o;
+    }
+}
+
+template <int K, int STAGES, int D>
+__global__ void __launch_bounds__(AS_CTA_THREADS, (FwdGeom<K, STAGES>::kCtas))
+call_forward_kernel(const uint4* __restrict__ counts, int T, int64_t P, int64_t p0, int64_t p1, int chunk,
+                    const uint8_t* __restrict__ ref, const float* __restrict__ thr_view, uint32_t cut, int pend_cap,
+                    as_call* __restrict__ calls, int64_t cap, unsigned long long* __restrict__ n_calls) {
+    static_assert(K * 4 <= 32, "candidate mask is one 32-bit word per thread and stage");
+    static_assert(D >= 1 && D <= 4, "resolution distance in stages");
+    extern __shared__ __align__(128) uint8_t smem_raw[];
+    __shared__ __align__(8) uint64_t bars[2 * STAGES];
+    __shared__ __align__(16) float thr_s[AS_TILE_SLOTS][8];
+    __shared__ __align__(16) FwdPending pend_all[AS_CONSUMER_WARPS];
+    __shared__ __align__(8) StagedCand q2_all[AS_CONSUMER_WARPS][AS_Q2_CAP];
+    // the scan's per-thread constants, reloaded every stage so that they hold no registers while a warp resolves entries
+    __shared__ __align__(16) uint4 rb_s[AS_TILE_SLOTS];  // floor(e_b * 2^32) of the forward threshold of each base
+    __shared__ __align__(8) uint2 rs_s[AS_TILE_SLOTS];   // (smallest of them over the callable bases, callable-base mask)
+    StageRing<K, STAGES, 1> ring;
+    ring.init(smem_raw, bars);
+    const int64_t tile0 = p0 + (int64_t)blockIdx.x * AS_TILE_SLOTS;
+    const int n_slots = (int)min((int64_t)AS_TILE_SLOTS, p1 - tile0);
+    const int t0 = blockIdx.y * chunk, t1 = min(T, t0 + chunk);
+    const int tid = threadIdx.x;
+    if (tid >= AS_TILE_SLOTS) {  // producer warp
+        if (tid == AS_TILE_SLOTS) ring.produce(counts + tile0, 2 * P, P, t0, t1, n_slots);
+        return;
+    }
+    const int lane = tid & 31, warp = tid >> 5;
+    const int64_t p = tile0 + tid;
+    {
+        uint32_t callable = 0, Rmin = 0xFFFFFFFFu;
+        uint32_t Rf[4] = {0u, 0u, 0u, 0u};  // 0 screens nothing out
+        if (tid < n_slots) {
+            const float4 a = *reinterpret_cast<const float4*>(thr_view + p * 8);
+            const float4 b = *reinterpret_cast<const float4*>(thr_view + p * 8 + 4);
+            *reinterpret_cast<float4*>(&thr_s[tid][0]) = a;
+            *reinterpret_cast<float4*>(&thr_s[tid][4]) = b;
+            const float e[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+            const uint32_t r = ref[p];
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                if (r > 3 || (uint32_t)i == r || e[2 * i] == -1.0f || e[2 * i + 1] == -1.0f) continue;
+                callable |= 1u << i;
+                // e * 2^32 is exact (power-of-two scaling) and < 2^32 for e < 1; anything else (negative, NaN, e >= 1)
+                // switches the pre-screen off for the base: the exact tests decide
+                const float ee = effective_err(e[2 * i]);
+                Rf[i] = (ee > 0.0f && ee < 1.0f) ? __float2uint_rz(ee * 4294967296.0f) : 0u;
+                Rmin = min(Rmin, Rf[i]);
+            }
+        }
+        rb_s[tid] = make_uint4(Rf[0], Rf[1], Rf[2], Rf[3]);
+        rs_s[tid] = make_uint2(Rmin, callable);
+    }
+    __syncwarp();  // a warp resolves only the records of its own 32 slots: their threshold rows are in place
+    FwdPending& pd = pend_all[warp];
+    StagedCand* q2 = q2_all[warp];
+    const uint4* bw_col = counts + P + p;  // reverse word of sample s at bw_col + s * 2P
+    const int cap_pend = (pend_cap > 0 && pend_cap < AS_FWD_PENDING) ? pend_cap : AS_FWD_PENDING;
+    const int batch = min(cap_pend, AS_FWD_PENDING / 2);
+    int n2 = 0;
+    uint32_t head = 0, tail = 0;  // warp-uniform running entry counts; entries [tail, head) are pending (wrap-safe differences)
+    uint32_t ends[D + 1];         // ends[d] = head after the stage d stages back
+#pragma unroll
+    for (int d = 0; d <= D; ++d) ends[d] = 0;
+
+    int it = 0;
+    for (int t = t0; t < t1; t += K, ++it) {
+        const uint4* st = ring.consumer_wait(it);
+        const int k = min(K, t1 - t);
+        // ---- scan, every record: present, FW >= cut, and one pre-screen bound against the smallest forward threshold of
+        // the callable bases (k > K(R_min) for some callable base) -- one multiply per record
+        uint32_t rec = 0;  // one bit per record that passes
+        {
+            const uint2 rs = rs_s[tid];
+            const uint32_t ax = 0u - (rs.y & 1u), ay = 0u - ((rs.y >> 1) & 1u), az = 0u - ((rs.y >> 2) & 1u), aw = 0u - (rs.y >> 3);
+#pragma unroll
+            for (int j = 0; j < K; ++j) {  // records j >= k hold stale words: dropped below
+                const uint4 fw = st[j * AS_TILE_SLOTS + tid];
+                const uint32_t FW = fw.x + fw.y + fw.z + fw.w;
+                const uint32_t kmax = max(max(fw.x & ax, fw.y & ay), max(fw.z & az, fw.w & aw));
+                const bool pass = ((int32_t)fw.x >= 0) & (FW >= cut) & (kmax > prescreen_k(FW, rs.x));  // no branches
+                rec |= pass ? (1u << j) : 0u;
+            }
+            rec &= (1u << k) - 1u;
+        }
+        // ---- the few records that pass: each base against its own bound; 4-bit base mask per record
+        uint32_t mask = 0;
+        if (rec != 0) {
+            const uint4 Rf = rb_s[tid];
+            const uint32_t callable = rs_s[tid].y;
+            do {
+                const int j = __ffs(rec) - 1;
+                rec &= rec - 1;
+                const uint4 fw = st[j * AS_TILE_SLOTS + tid];
+                const uint32_t FW = fw.x + fw.y + fw.z + fw.w;
+                const uint32_t m = (fw.x > prescreen_k(FW, Rf.x) ? 1u : 0u) | (fw.y > prescreen_k(FW, Rf.y) ? 2u : 0u) |
+                                   (fw.z > prescreen_k(FW, Rf.z) ? 4u : 0u) | (fw.w > prescreen_k(FW, Rf.w) ? 8u : 0u);
+                mask |= (m & callable) << (4 * j);
+            } while (rec != 0);
+        }
+        const uint32_t nz = (mask | (mask >> 1) | (mask >> 2) | (mask >> 3)) & 0x11111111u;  // one bit per candidate record
+        if (__ballot_sync(0xffffffffu, nz != 0) != 0) {
+            const int mine = __popc(nz);
+            int incl = mine;
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int up = __shfl_up_sync(0xffffffffu, incl, d);
+                if (lane >= d) incl += up;
+            }
+            const int total = __shfl_sync(0xffffffffu, incl, 31), first = incl - mine;
+            int done = 0;
+            while (total - done > cap_pend - (int)(head - tail)) {  // the ring cannot take the rest of this stage
+                if (head == tail) {  // empty: pass a ring's worth through it at once
+                    fwd_issue(pd, st, bw_col, 2 * P, mask, nz, first, done, done + cap_pend, head, t);
+                    head += (uint32_t)cap_pend;
+                    done += cap_pend;
+                    cp_async_commit();
+                }
+                cp_async_wait<0>();
+                __syncwarp();
+                fwd_resolve(pd, tail, head - tail, thr_s, tile0, cut, q2, n2, ref, thr_view, calls, cap, n_calls);
+                tail = head;
+            }
+            fwd_issue(pd, st, bw_col, 2 * P, mask, nz, first, done, total, head, t);
+            head += (uint32_t)(total - done);
+        }
+        cp_async_commit();
+        ring.consumer_release(it);
+#pragma unroll
+        for (int d = D; d > 0; --d) ends[d] = ends[d - 1];
+        ends[0] = head;
+        // entries of the stages D and more back have landed (every commit group but the D most recent); they are resolved
+        // once there are enough of them to keep the warp's lanes busy, not every stage
+        if ((int)(ends[D] - tail) >= batch) {
+            cp_async_wait<D>();
+            __syncwarp();
+            fwd_resolve(pd, tail, ends[D] - tail, thr_s, tile0, cut, q2, n2, ref, thr_view, calls, cap, n_calls);
+            tail = ends[D];
+        }
+    }
+    if (head != tail) {
+        cp_async_wait<0>();
+        __syncwarp();
+        fwd_resolve(pd, tail, head - tail, thr_s, tile0, cut, q2, n2, ref, thr_view, calls, cap, n_calls);
+    }
+    if (n2 > 0) stage2_batch_staged(q2, n2, ref, thr_view, 1, 0, calls, cap, n_calls);
+}
+
 // ------------------------------------------------------------------------------------------------
 // element-wise evaluators (parity grids)
 // ------------------------------------------------------------------------------------------------
@@ -1148,6 +1394,23 @@ static cudaError_t launch_call_staged_impl(dim3 grid, const uint4* c, int T, int
     return cudaGetLastError();
 }
 
+template <int K, int STAGES, int D>
+static cudaError_t launch_call_forward(dim3 grid, const uint4* c, int T, int64_t P, int64_t p0, int64_t p1, int chunk,
+                                       const uint8_t* ref, const float* tv, uint32_t cut, int pend_cap, as_call* calls, int64_t cap,
+                                       unsigned long long* n, cudaStream_t st) {
+    static bool configured[AS_MAX_DEVICES] = {};  // the attribute is per device
+    const int smem = StageRing<K, STAGES, 1>::kStageBytes * STAGES;
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= AS_MAX_DEVICES || !configured[dev]) {
+        cudaError_t e = cudaFuncSetAttribute(call_forward_kernel<K, STAGES, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e != cudaSuccess) return e;
+        if (dev >= 0 && dev < AS_MAX_DEVICES) configured[dev] = true;
+    }
+    call_forward_kernel<K, STAGES, D><<<grid, AS_CTA_THREADS, smem, st>>>(c, T, P, p0, p1, chunk, ref, tv, cut, pend_cap, calls, cap, n);
+    return cudaGetLastError();
+}
+
 template <int K, int STAGES, bool PRE = false>
 static cudaError_t launch_call_staged(dim3 grid, const uint4* c, int T, int64_t P, int64_t p0, int64_t p1, int chunk,
                                       const uint8_t* ref, const float* tv, int n_c, int64_t c_stride, uint32_t cut,
@@ -1159,29 +1422,34 @@ static cudaError_t launch_call_staged(dim3 grid, const uint4* c, int T, int64_t 
 
 cudaError_t as_launch_call_sweep(int variant, const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1,
                                  const uint8_t* d_ref, const float* d_thr_views, int n_c, int64_t c_stride, uint32_t cut,
-                                 as_call* d_calls, int64_t cap, unsigned long long* d_n_calls, cudaStream_t st) {
+                                 as_call* d_calls, int64_t cap, unsigned long long* d_n_calls, int fwd_pending_cap, cudaStream_t st) {
     if (p1 <= p0 || T <= 0 || n_c <= 0) return cudaSuccess;
     const uint4* c = reinterpret_cast<const uint4*>(d_counts);
     const int chunk = as_call_chunk(T, p1 - p0);
     dim3 grid(cdiv64(p1 - p0, AS_CALL_THREADS), (unsigned)((T + chunk - 1) / chunk));
 #define AS_CALL_ARGS c, T, P, p0, p1, chunk, d_ref, d_thr_views, cut, d_calls, cap, d_n_calls
 #define AS_SWEEP_ARGS c, T, P, p0, p1, chunk, d_ref, d_thr_views, n_c, c_stride, cut, d_calls, cap, d_n_calls
+#define AS_FWD_ARGS c, T, P, p0, p1, chunk, d_ref, d_thr_views, cut, fwd_pending_cap, d_calls, cap, d_n_calls
     switch (variant) {
         case 0: if (n_c != 1) return cudaErrorInvalidValue; call_naive_kernel<<<grid, AS_CALL_THREADS, 0, st>>>(AS_CALL_ARGS); return cudaGetLastError();
         case 1: if (n_c != 1) return cudaErrorInvalidValue; call_queued_kernel<<<grid, AS_CALL_THREADS, 0, st>>>(AS_CALL_ARGS); return cudaGetLastError();
         case 3: return launch_call_staged<4, 2>(grid, AS_SWEEP_ARGS, st);
         case 11: return launch_call_staged<3, 2>(grid, AS_SWEEP_ARGS, st);
         case 14: return launch_call_staged<4, 2, true>(grid, AS_SWEEP_ARGS, st);
-        default: return launch_call_staged<3, 2, true>(grid, AS_SWEEP_ARGS, st);
+        case 15: return launch_call_staged<3, 2, true>(grid, AS_SWEEP_ARGS, st);
+        default: if (n_c != 1) break; return launch_call_forward<6, 2, 2>(grid, AS_FWD_ARGS, st);
     }
+    // a sweep of several tables on a staged variant: the in-stage sweep kernel
+    return launch_call_staged<3, 2, true>(grid, AS_SWEEP_ARGS, st);
 #undef AS_CALL_ARGS
 #undef AS_SWEEP_ARGS
+#undef AS_FWD_ARGS
 }
 
 cudaError_t as_launch_call(int variant, const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1,
                            const uint8_t* d_ref, const float* d_thr_view, uint32_t cut, as_call* d_calls, int64_t cap,
-                           unsigned long long* d_n_calls, cudaStream_t st) {
-    return as_launch_call_sweep(variant, d_counts, T, P, p0, p1, d_ref, d_thr_view, 1, 0, cut, d_calls, cap, d_n_calls, st);
+                           unsigned long long* d_n_calls, int fwd_pending_cap, cudaStream_t st) {
+    return as_launch_call_sweep(variant, d_counts, T, P, p0, p1, d_ref, d_thr_view, 1, 0, cut, d_calls, cap, d_n_calls, fwd_pending_cap, st);
 }
 
 cudaError_t as_launch_poisson_test(const int32_t* k, const int32_t* rd, const float* err, int64_t n, double* p,

@@ -15,7 +15,7 @@
  * thread scans its own rows, the two states are merged exactly after the sample loop (as_noise.cuh pair_merge).
  * 0: every twin group goes to noise_pair_kernel / noise_twin_kernel. */
 #define AS_INTILE_TWINS 1
-#define AS_DEFAULT_CALL_KERNEL 13 /* TMA-staged, 3 samples per stage, 2 stages (7 CTAs/SM), integer pre-screen in the scan: best of the measured sweeps on the c3 and the c5 shape */
+#define AS_DEFAULT_CALL_KERNEL 13 /* forward-first (call_forward_kernel): forward plane streamed, 6 samples per stage, 2 stages, reverse words fetched for forward candidates; 15 = the both-strand staged caller it replaced */
 #define AS_DEFAULT_NOISE_KERNEL 1 /* TMA-staged, 4 samples per stage, 3 stages */
 #define AS_DEFERRED_CALL_KERNEL 20 /* scan -> resolve -> series (as_call_deferred.cu); what a sweep runs by default */
 
@@ -54,9 +54,11 @@ cudaError_t as_launch_patch_wide(const as_wide_record* d_wide, int64_t m, uint32
                                  int n_samples, cudaStream_t st);
 cudaError_t as_launch_thr_view(const float* d_thr, float* d_view, int64_t n, cudaStream_t st);
 int as_call_chunk(int T, int64_t n_slots);
+// fwd_pending_cap: usable depth of call_forward_kernel's per-warp pending ring, 1..AS_FWD_PENDING (else the whole ring)
+#define AS_FWD_PENDING 32
 cudaError_t as_launch_call(int variant, const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1,
                            const uint8_t* d_ref, const float* d_thr_view, uint32_t cut, as_call* d_calls, int64_t cap,
-                           unsigned long long* d_n_calls, cudaStream_t st);
+                           unsigned long long* d_n_calls, int fwd_pending_cap, cudaStream_t st);
 // as_sort.cu: call list housekeeping of the _host caller pipeline
 cudaError_t as_launch_call_slot_offset(as_call* d_calls, const unsigned long long* d_n_prev, const unsigned long long* d_n_now,
                                        int64_t cap, int32_t off, cudaStream_t st);
@@ -68,7 +70,7 @@ cudaError_t as_launch_fisher(const int32_t* d_tables, int64_t n, const double* d
 // n_c threshold tables c_stride floats apart (noise-floor sweep): list ci at d_calls + ci * cap, counter d_n_calls[ci]
 cudaError_t as_launch_call_sweep(int variant, const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1,
                                  const uint8_t* d_ref, const float* d_thr_views, int n_c, int64_t c_stride, uint32_t cut,
-                                 as_call* d_calls, int64_t cap, unsigned long long* d_n_calls, cudaStream_t st);
+                                 as_call* d_calls, int64_t cap, unsigned long long* d_n_calls, int fwd_pending_cap, cudaStream_t st);
 // as_pileup.cu: BAM records -> counts[2][P][4] of one sample (SURVEY.md 8 f4); stats[0] reads used, stats[1] bases counted
 cudaError_t as_launch_pileup(const uint8_t* d_rec, const int64_t* d_rec_off, int64_t n_rec, int64_t n_bytes,
                              const int32_t* d_ref_contig, int32_t n_ref, const int64_t* d_contig_first,

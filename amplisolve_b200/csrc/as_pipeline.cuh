@@ -1,8 +1,8 @@
 // Shared-memory staging of position tiles with the Blackwell bulk-copy engine (TMA, 1-D form).
 //
 // A CTA owns a tile of AS_TILE_SLOTS consecutive panel slots and walks the sample axis.  One elected
-// producer thread streams [K samples][2 strands][tile] blocks of the count tensor into a ring of
-// shared-memory stages with cp.async.bulk (SASS: UBLKCP), one 2 KiB copy per (sample, strand) row, each
+// producer thread streams [K samples][2 strands][tile] blocks (or the forward strand only) of the count tensor into a ring
+// of shared-memory stages with cp.async.bulk (SASS: UBLKCP), one 2 KiB copy per (sample, strand) row, each
 // stage guarded by a "full" mbarrier (transaction-count completion) and an "empty" mbarrier (one arrival
 // per consumer warp).  The consumer warps never touch global memory for counts and hold no in-flight load
 // registers, so the memory system sees up to (stages-1) * K * 4 KiB outstanding per CTA regardless of how
@@ -56,12 +56,24 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
                  : "memory");
 }
 
-// Ring geometry.  A stage holds K samples x 2 strands x AS_TILE_SLOTS uint4 words.
-template <int K, int STAGES>
+// 16-byte asynchronous copy global -> shared through L2 only (SASS: LDGSTS), tracked per thread in commit groups: a thread
+// may read what it copied after cp.async.wait_group, other lanes of its warp after a __syncwarp that follows.
+__device__ __forceinline__ void cp_async16(void* dst_smem, const void* src_gmem) {
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(dst_smem)), "l"(src_gmem) : "memory");
+}
+__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
+// wait until at most N of this thread's most recent commit groups are still in flight
+template <int N>
+__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
+
+// Ring geometry.  A stage holds K samples x STRANDS strands x AS_TILE_SLOTS uint4 words; STRANDS = 1 streams the
+// forward strand only (call_forward_kernel, which fetches reverse-strand words on its own).
+template <int K, int STAGES, int STRANDS = 2>
 struct StageRing {
-    static constexpr int kStageWords = K * 2 * AS_TILE_SLOTS;  // uint4 words
+    static_assert(STRANDS == 1 || STRANDS == 2, "one or both strands per sample");
+    static constexpr int kStageWords = K * STRANDS * AS_TILE_SLOTS;  // uint4 words
     static constexpr int kStageBytes = kStageWords * 16;
-    uint4* data;        // [STAGES][K][2][AS_TILE_SLOTS]
+    uint4* data;        // [STAGES][K][STRANDS][AS_TILE_SLOTS]
     uint64_t* full;     // [STAGES]
     uint64_t* empty;    // [STAGES]
 
@@ -90,12 +102,12 @@ struct StageRing {
             const int s = it % STAGES;
             if (it >= STAGES) mbar_wait(&empty[s], ((it / STAGES) - 1) & 1);
             const int k = min(K, t1 - t);
-            mbar_expect_tx(&full[s], row_bytes * 2u * (uint32_t)k);
+            mbar_expect_tx(&full[s], row_bytes * (uint32_t)STRANDS * (uint32_t)k);
             uint4* dst = data + (size_t)s * kStageWords;
             for (int j = 0; j < k; ++j) {
                 const uint4* g = src + (int64_t)(t + j) * sstride;
-                bulk_g2s(dst + (j * 2 + 0) * AS_TILE_SLOTS, g, row_bytes, &full[s]);
-                bulk_g2s(dst + (j * 2 + 1) * AS_TILE_SLOTS, g + P, row_bytes, &full[s]);
+                bulk_g2s(dst + (j * STRANDS + 0) * AS_TILE_SLOTS, g, row_bytes, &full[s]);
+                if (STRANDS == 2) bulk_g2s(dst + (j * STRANDS + 1) * AS_TILE_SLOTS, g + P, row_bytes, &full[s]);
             }
         }
     }

@@ -99,7 +99,9 @@ int as_host_alloc(void** out, size_t bytes);
 int as_host_free(void* p);
 /* Kernel variants (the tests cross-check them against each other and the oracle; -1 = default):
  *   caller: 0 = straightforward, 1 = per-warp queues over direct loads, TMA-staged with (samples per stage, stages):
- *           3 = (4,2), 11 = (3,2); with the integer pre-screen in the scan: 13 = (3,2) default, 14 = (4,2);
+ *           3 = (4,2), 11 = (3,2); with the integer pre-screen in the scan: 15 = (3,2), 14 = (4,2);
+ *           13 = default: forward-first, the forward strand streamed (6,2) and a record's reverse-strand word fetched
+ *           only when its forward strand can still make a call (single table; a sweep on 13 runs the deferred pipeline);
  *           20 = deferred: scan -> resolve -> series kernels over candidate lists (what a sweep of several tables runs)
  *   noise : 0 = direct loads; TMA-staged 1 = (4,3) default, 4 = (8,2), 6 = (4,2); 7, 8 = shared-pattern accumulators (the
  *           kernel of as_noise_estimate_sweep_dev) with the records of a stage interleaved / walked one by one */
@@ -109,7 +111,9 @@ int as_set_noise_kernel(as_ctx* ctx, int variant);
  * Small values are for tests (tile-boundary handling). */
 int as_set_host_tile_slots(as_ctx* ctx, int64_t slots);
 /* Generic form of the setters above plus "deferred_capacity" (entries of the deferred caller's candidate list; 0 =
- * automatic; the kernels resolve what does not fit on the spot, so results never depend on it -- tests use tiny values). */
+ * automatic; the kernels resolve what does not fit on the spot, so results never depend on it -- tests use tiny values)
+ * and "forward_pending_cap" (usable entries of call kernel 13's per-warp ring of pending reverse-strand fetches, 0 =
+ * automatic, at most 32; a full ring is drained on the spot, so results never depend on it either). */
 int as_set_option(as_ctx* ctx, const char* name, int64_t value);
 /* Number of kernel launches this context has enqueued so far (bench.py's gpu_launches). */
 int64_t as_kernel_launches(const as_ctx* ctx);
