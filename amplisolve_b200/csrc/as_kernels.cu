@@ -883,30 +883,30 @@ call_staged_kernel(const uint4* __restrict__ counts, int T, int64_t P, int64_t p
 
 // Forward-first caller.  A record can only become a call if BOTH strand tests pass (VC:898, VC:895-896), and the forward
 // strand alone rules out nearly every record: the ring streams the forward plane only (16 B per record instead of 32).
-// Scan, every record, integer only: present, FW >= cut, and k > prescreen_k(FW, R_min) for some callable base (alt != ref,
-// a threshold on both strands: -1 is never a call, VC:3844-3849), R_min = floor(e * 2^32) of the smallest forward threshold
-// of those bases.  The few records that pass are tested base by base against the base's own bound R_b (what the bound of
-// strand_can_pass is; the minimum is only weaker, and one multiply per record is what keeps the scan lean) before anything
-// is fetched for them.
-// The records with a candidate base are compacted per warp (one prefix sum per stage) into a pending ring in shared
-// memory: the forward word, (sample, column, base mask), and the reverse-strand word, fetched with a 16-byte cp.async that
-// stays in flight while the warp scans the next stages.  The entries of stage i are resolved at stage i + D or later, in
-// batches of at least half a ring, after the stage has been handed back to the producer: BW >= cut, reverse
-// k > prescreen_k(BW, R_b), strand_can_pass on both strands; survivors join the series queue of call_staged_kernel.
-// Nothing in the scan waits on a global read.
-// A ring that cannot take a stage's entries is drained on the spot (wait for every copy, resolve), a slower path that
-// gives the same calls; pend_cap < AS_FWD_PENDING caps the usable depth (tests of that path).
-struct FwdPending {  // per warp; the reverse words are cp.async targets (16-byte aligned)
+// The CTA's warps have two roles: four scan warps and one control warp per ring stage.
+// Scan warps (warps 0-3, thread per slot), every record, integer only and branch-free: present, FW >= cut, and
+// k > prescreen_k(FW, R_min) for some callable base (alt != ref, a threshold on both strands: -1 is never a call,
+// VC:3844-3849), R_min = floor(e * 2^32) of the smallest forward threshold of those bases.  A thread stores one K-bit pass
+// mask per stage and releases the stage; the arrive on the stage's empty barrier publishes the mask.
+// Control warp c (warp 4 + c) owns stage c.  Each time the scan warps have released it (it is the stage's last reader):
+//   1. the 128 pass masks, one warp prefix sum -> the list of passing (record, column);
+//   2. 32 passers at a time, one per lane: each base against its own bound R_b (what the bound of strand_can_pass is; the
+//      minimum is only weaker, and one multiply per record is what keeps the scan lean);
+//   3. the records with a candidate base, compacted by ballot into the warp's pending ring: the forward word, (sample,
+//      column | base mask), and the reverse-strand word, fetched with a 16-byte cp.async; one commit group per stage;
+//   4. the refill of the stage (bulk copies of the forward rows);
+//   5. then, off the refill path, the pending entries of the warp's stage i are resolved at its stage i + D or later, once
+//      a warp's worth has landed: BW >= cut, reverse k > prescreen_k(BW, R_b), strand_can_pass on both strands; survivors join the series
+//      queue of call_staged_kernel.
+// The per-record candidate work is thus paid once per CTA and stage, on full warps, instead of in every scan warp.  It is
+// still a chain of dependent shared-memory reads, shuffles and fp64 series on one warp; one control warp per stage lets the
+// control work of consecutive stages overlap (one control warp for all stages was slower than the per-warp design it
+// replaces, DESIGN 3.2b).  A ring that cannot take a stage's candidates is drained on the spot (wait for every copy,
+// resolve), a slower path that gives the same calls; pend_cap < AS_FWD_PENDING caps the usable depth (tests of that path).
+struct FwdPending {  // per control warp; the reverse words are cp.async targets (16-byte aligned)
     uint4 bw[AS_FWD_PENDING];
     uint4 fw[AS_FWD_PENDING];
     uint2 meta[AS_FWD_PENDING];  // sample, tile column | forward candidate base mask << 8
-};
-
-template <int K, int STAGES>
-struct FwdGeom {
-    static constexpr int kSmem = StageRing<K, STAGES, 1>::kStageBytes * STAGES + AS_TILE_SLOTS * (32 + 16 + 8) +
-                                 AS_CONSUMER_WARPS * ((int)sizeof(FwdPending) + AS_Q2_CAP * (int)sizeof(StagedCand));
-    static constexpr int kCtas = (227 * 1024) / (kSmem + 1024) > 8 ? 8 : (227 * 1024) / (kSmem + 1024);
 };
 
 // resolve the n pending entries from ring entry `from` on; full warps, one entry per lane
@@ -963,54 +963,32 @@ __device__ __forceinline__ void fwd_resolve(const FwdPending& pd, uint32_t from,
     __syncwarp();  // the entries are read before the ring positions are reused
 }
 
-// entries o in [lo, hi) of this stage (numbered in lane order; this lane's from `first` on) go to ring entry head + o - lo
-__device__ __forceinline__ void fwd_issue(FwdPending& pd, const uint4* st, const uint4* __restrict__ bw_col, int64_t sstride,
-                                          uint32_t mask, uint32_t nz, int first, int lo, int hi, uint32_t head, int t) {
-    const int tid = threadIdx.x;
-    int o = first;
-    while (nz) {
-        const int j = (__ffs(nz) - 1) >> 2;
-        nz &= nz - 1;
-        if (o >= lo && o < hi) {
-            const uint32_t pos = (head + (uint32_t)(o - lo)) & (AS_FWD_PENDING - 1);
-            pd.fw[pos] = st[j * AS_TILE_SLOTS + tid];
-            pd.meta[pos] = make_uint2((uint32_t)(t + j), (uint32_t)tid | (((mask >> (4 * j)) & 15u) << 8));
-            cp_async16(&pd.bw[pos], bw_col + (int64_t)(t + j) * sstride);
-        }
-        ++o;
-    }
-}
-
+// (4, 3): 224 threads, 4 CTAs/SM; registers (one allocation for both roles: 72 per thread, set by the control warps'
+// fp64 series) and shared memory (24 KiB of stages + 28 KiB of tables and per-warp queues) both allow four, neither five.
 template <int K, int STAGES, int D>
-__global__ void __launch_bounds__(AS_CTA_THREADS, (FwdGeom<K, STAGES>::kCtas))
+__global__ void __launch_bounds__(AS_TILE_SLOTS + 32 * STAGES, 4)
 call_forward_kernel(const uint4* __restrict__ counts, int T, int64_t P, int64_t p0, int64_t p1, int chunk,
                     const uint8_t* __restrict__ ref, const float* __restrict__ thr_view, uint32_t cut, int pend_cap,
                     as_call* __restrict__ calls, int64_t cap, unsigned long long* __restrict__ n_calls) {
-    static_assert(K * 4 <= 32, "candidate mask is one 32-bit word per thread and stage");
+    static_assert(K <= 8, "a record's pass bit in one byte per slot and stage");
     static_assert(D >= 1 && D <= 4, "resolution distance in stages");
     extern __shared__ __align__(128) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * STAGES];
     __shared__ __align__(16) float thr_s[AS_TILE_SLOTS][8];
-    __shared__ __align__(16) FwdPending pend_all[AS_CONSUMER_WARPS];
-    __shared__ __align__(8) StagedCand q2_all[AS_CONSUMER_WARPS][AS_Q2_CAP];
-    // the scan's per-thread constants, reloaded every stage so that they hold no registers while a warp resolves entries
-    __shared__ __align__(16) uint4 rb_s[AS_TILE_SLOTS];  // floor(e_b * 2^32) of the forward threshold of each base
-    __shared__ __align__(8) uint2 rs_s[AS_TILE_SLOTS];   // (smallest of them over the callable bases, callable-base mask)
-    StageRing<K, STAGES, 1> ring;
-    ring.init(smem_raw, bars);
+    __shared__ __align__(16) uint4 rb_s[AS_TILE_SLOTS];     // floor(e_b * 2^32) of the forward threshold of each base
+    __shared__ uint32_t callable_s[AS_TILE_SLOTS];           // callable-base mask
+    __shared__ __align__(4) uint8_t pass_s[STAGES][AS_TILE_SLOTS];  // scan -> control: bit j = record j of the stage passes
+    __shared__ uint16_t passers_all[STAGES][K * AS_TILE_SLOTS];  // record << 8 | column, of the stage a control warp reads
+    __shared__ __align__(16) FwdPending pd_all[STAGES];
+    __shared__ __align__(8) StagedCand q2_all[STAGES][AS_Q2_CAP];
     const int64_t tile0 = p0 + (int64_t)blockIdx.x * AS_TILE_SLOTS;
     const int n_slots = (int)min((int64_t)AS_TILE_SLOTS, p1 - tile0);
     const int t0 = blockIdx.y * chunk, t1 = min(T, t0 + chunk);
-    const int tid = threadIdx.x;
-    if (tid >= AS_TILE_SLOTS) {  // producer warp
-        if (tid == AS_TILE_SLOTS) ring.produce(counts + tile0, 2 * P, P, t0, t1, n_slots);
-        return;
-    }
-    const int lane = tid & 31, warp = tid >> 5;
-    const int64_t p = tile0 + tid;
-    {
-        uint32_t callable = 0, Rmin = 0xFFFFFFFFu;
+    const int tid = threadIdx.x, lane = tid & 31;
+    uint32_t Rmin = 0xFFFFFFFFu, callable = 0;
+    if (tid < AS_TILE_SLOTS) {
         uint32_t Rf[4] = {0u, 0u, 0u, 0u};  // 0 screens nothing out
+        const int64_t p = tile0 + tid;
         if (tid < n_slots) {
             const float4 a = *reinterpret_cast<const float4*>(thr_view + p * 8);
             const float4 b = *reinterpret_cast<const float4*>(thr_view + p * 8 + 4);
@@ -1030,88 +1008,123 @@ call_forward_kernel(const uint4* __restrict__ counts, int T, int64_t P, int64_t 
             }
         }
         rb_s[tid] = make_uint4(Rf[0], Rf[1], Rf[2], Rf[3]);
-        rs_s[tid] = make_uint2(Rmin, callable);
+        callable_s[tid] = callable;
     }
-    __syncwarp();  // a warp resolves only the records of its own 32 slots: their threshold rows are in place
-    FwdPending& pd = pend_all[warp];
-    StagedCand* q2 = q2_all[warp];
-    const uint4* bw_col = counts + P + p;  // reverse word of sample s at bw_col + s * 2P
-    const int cap_pend = (pend_cap > 0 && pend_cap < AS_FWD_PENDING) ? pend_cap : AS_FWD_PENDING;
-    const int batch = min(cap_pend, AS_FWD_PENDING / 2);
-    int n2 = 0;
-    uint32_t head = 0, tail = 0;  // warp-uniform running entry counts; entries [tail, head) are pending (wrap-safe differences)
-    uint32_t ends[D + 1];         // ends[d] = head after the stage d stages back
-#pragma unroll
-    for (int d = 0; d <= D; ++d) ends[d] = 0;
+    StageRing<K, STAGES, 1> ring;
+    ring.init(smem_raw, bars);  // its __syncthreads also publishes the tables above to the control warps
+    const int n_it = (t1 - t0 + K - 1) / K;
 
-    int it = 0;
-    for (int t = t0; t < t1; t += K, ++it) {
-        const uint4* st = ring.consumer_wait(it);
-        const int k = min(K, t1 - t);
-        // ---- scan, every record: present, FW >= cut, and one pre-screen bound against the smallest forward threshold of
-        // the callable bases (k > K(R_min) for some callable base) -- one multiply per record
-        uint32_t rec = 0;  // one bit per record that passes
-        {
-            const uint2 rs = rs_s[tid];
-            const uint32_t ax = 0u - (rs.y & 1u), ay = 0u - ((rs.y >> 1) & 1u), az = 0u - ((rs.y >> 2) & 1u), aw = 0u - (rs.y >> 3);
+    if (tid < AS_TILE_SLOTS) {
+        // ---- scan warps: present, FW >= cut, and one pre-screen bound against the smallest forward threshold of the
+        // callable bases (k > K(R_min) for some callable base) -- one multiply per record.  A slot past the tile's end has
+        // no callable base and never passes.
+        const uint32_t ax = 0u - (callable & 1u), ay = 0u - ((callable >> 1) & 1u), az = 0u - ((callable >> 2) & 1u),
+                       aw = 0u - (callable >> 3);
+        for (int it = 0; it < n_it; ++it) {
+            const uint4* st = ring.consumer_wait(it);
+            const int k = min(K, t1 - t0 - it * K);
+            uint32_t rec = 0;  // one bit per record that passes
 #pragma unroll
             for (int j = 0; j < K; ++j) {  // records j >= k hold stale words: dropped below
                 const uint4 fw = st[j * AS_TILE_SLOTS + tid];
                 const uint32_t FW = fw.x + fw.y + fw.z + fw.w;
                 const uint32_t kmax = max(max(fw.x & ax, fw.y & ay), max(fw.z & az, fw.w & aw));
-                const bool pass = ((int32_t)fw.x >= 0) & (FW >= cut) & (kmax > prescreen_k(FW, rs.x));  // no branches
+                const bool pass = ((int32_t)fw.x >= 0) & (FW >= cut) & (kmax > prescreen_k(FW, Rmin));  // no branches
                 rec |= pass ? (1u << j) : 0u;
             }
-            rec &= (1u << k) - 1u;
+            pass_s[it % STAGES][tid] = (uint8_t)(rec & ((1u << k) - 1u));
+            ring.consumer_release(it);
         }
-        // ---- the few records that pass: each base against its own bound; 4-bit base mask per record
-        uint32_t mask = 0;
-        if (rec != 0) {
-            const uint4 Rf = rb_s[tid];
-            const uint32_t callable = rs_s[tid].y;
-            do {
-                const int j = __ffs(rec) - 1;
-                rec &= rec - 1;
-                const uint4 fw = st[j * AS_TILE_SLOTS + tid];
-                const uint32_t FW = fw.x + fw.y + fw.z + fw.w;
-                const uint32_t m = (fw.x > prescreen_k(FW, Rf.x) ? 1u : 0u) | (fw.y > prescreen_k(FW, Rf.y) ? 2u : 0u) |
-                                   (fw.z > prescreen_k(FW, Rf.z) ? 4u : 0u) | (fw.w > prescreen_k(FW, Rf.w) ? 8u : 0u);
-                mask |= (m & callable) << (4 * j);
-            } while (rec != 0);
-        }
-        const uint32_t nz = (mask | (mask >> 1) | (mask >> 2) | (mask >> 3)) & 0x11111111u;  // one bit per candidate record
-        if (__ballot_sync(0xffffffffu, nz != 0) != 0) {
-            const int mine = __popc(nz);
-            int incl = mine;
+        return;
+    }
+
+    // ---- control warps: warp c owns stage c (iterations c, c + STAGES, ...)
+    const int cw = (tid - AS_TILE_SLOTS) >> 5;
+    uint16_t* passers = passers_all[cw];
+    FwdPending& pd = pd_all[cw];
+    StagedCand* q2 = q2_all[cw];
+    const uint4* src = counts + tile0;
+    const int64_t sstride = 2 * P;
+    const uint32_t row_bytes = (uint32_t)n_slots * 16u;
+    if (lane == 0 && cw < n_it) ring.fill(cw, src, sstride, P, t0, t1, row_bytes);
+    const uint4* bw_tile = counts + P + tile0;  // reverse word of (sample s, column c) at bw_tile + s * 2P + c
+    const int cap_pend = (pend_cap > 0 && pend_cap < AS_FWD_PENDING) ? pend_cap : AS_FWD_PENDING;
+    const int batch = min(cap_pend, 32);
+    int n2 = 0;
+    uint32_t head = 0, tail = 0;  // running entry counts; entries [tail, head) are pending (wrap-safe differences)
+    uint32_t ends[D + 1];         // ends[d] = head after the stage d stages back
 #pragma unroll
-            for (int d = 1; d < 32; d <<= 1) {
-                const int up = __shfl_up_sync(0xffffffffu, incl, d);
-                if (lane >= d) incl += up;
+    for (int d = 0; d <= D; ++d) ends[d] = 0;
+
+    for (int it = cw; it < n_it; it += STAGES) {
+        const int s = cw;
+        const uint32_t parity = (it / STAGES) & 1;
+        mbar_wait(&ring.empty[s], parity);  // every scan warp has stored its pass masks and released the stage
+        mbar_wait(&ring.full[s], parity);   // completed long ago; makes the visibility of the bulk-copied words explicit
+        const uint4* st = ring.stage(s);
+        const int t = t0 + it * K;
+        // 1. the passers of the stage: four columns per lane, one prefix sum
+        const uint32_t pm = reinterpret_cast<const uint32_t*>(pass_s[s])[lane];
+        const int mine = __popc(pm);
+        int incl = mine;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int up = __shfl_up_sync(0xffffffffu, incl, d);
+            if (lane >= d) incl += up;
+        }
+        const int total = __shfl_sync(0xffffffffu, incl, 31);
+        for (uint32_t m = pm, o = incl - mine; m != 0; m &= m - 1, ++o) {
+            const int bit = __ffs(m) - 1;
+            passers[o] = (uint16_t)(((bit & 7) << 8) | (lane * 4 + (bit >> 3)));
+        }
+        __syncwarp();
+        // 2.-3. each passer's bases against their own bounds; the candidates into the pending ring
+        for (int base = 0; base < total; base += 32) {
+            const int i = base + lane;
+            uint4 fw = make_uint4(0, 0, 0, 0);
+            uint32_t bm = 0, j = 0, col = 0;
+            if (i < total) {
+                const uint32_t e = passers[i];
+                j = e >> 8;
+                col = e & 255u;
+                fw = st[j * AS_TILE_SLOTS + col];
+                const uint4 Rf = rb_s[col];
+                const uint32_t FW = fw.x + fw.y + fw.z + fw.w;
+                bm = ((fw.x > prescreen_k(FW, Rf.x) ? 1u : 0u) | (fw.y > prescreen_k(FW, Rf.y) ? 2u : 0u) |
+                      (fw.z > prescreen_k(FW, Rf.z) ? 4u : 0u) | (fw.w > prescreen_k(FW, Rf.w) ? 8u : 0u)) & callable_s[col];
             }
-            const int total = __shfl_sync(0xffffffffu, incl, 31), first = incl - mine;
-            int done = 0;
-            while (total - done > cap_pend - (int)(head - tail)) {  // the ring cannot take the rest of this stage
-                if (head == tail) {  // empty: pass a ring's worth through it at once
-                    fwd_issue(pd, st, bw_col, 2 * P, mask, nz, first, done, done + cap_pend, head, t);
-                    head += (uint32_t)cap_pend;
-                    done += cap_pend;
+            unsigned votes = __ballot_sync(0xffffffffu, bm != 0);
+            while (votes != 0) {
+                if ((int)(head - tail) == cap_pend) {  // the ring is full: drain it on the spot
                     cp_async_commit();
+                    cp_async_wait<0>();
+                    __syncwarp();
+                    fwd_resolve(pd, tail, head - tail, thr_s, tile0, cut, q2, n2, ref, thr_view, calls, cap, n_calls);
+                    tail = head;
                 }
-                cp_async_wait<0>();
-                __syncwarp();
-                fwd_resolve(pd, tail, head - tail, thr_s, tile0, cut, q2, n2, ref, thr_view, calls, cap, n_calls);
-                tail = head;
+                const uint32_t room = (uint32_t)cap_pend - (head - tail);
+                const uint32_t rank = __popc(votes & ((1u << lane) - 1u));
+                const bool take = ((votes >> lane) & 1u) && rank < room;
+                if (take) {
+                    const uint32_t pos = (head + rank) & (AS_FWD_PENDING - 1);
+                    pd.fw[pos] = fw;
+                    pd.meta[pos] = make_uint2((uint32_t)t + j, col | (bm << 8));
+                    cp_async16(&pd.bw[pos], bw_tile + (int64_t)(t + (int)j) * sstride + col);
+                }
+                const unsigned taken = __ballot_sync(0xffffffffu, take);
+                head += (uint32_t)__popc(taken);
+                votes &= ~taken;
             }
-            fwd_issue(pd, st, bw_col, 2 * P, mask, nz, first, done, total, head, t);
-            head += (uint32_t)(total - done);
         }
         cp_async_commit();
-        ring.consumer_release(it);
+        // 4. the stage has been read for the last time: refill it
+        __syncwarp();
+        if (lane == 0 && it + STAGES < n_it) ring.fill(it + STAGES, src, sstride, P, t0, t1, row_bytes);
+        // 5. entries of the stages D and more back have landed (every commit group but the D most recent); they are
+        // resolved once there are enough of them to keep the warp's lanes busy, not every stage
 #pragma unroll
         for (int d = D; d > 0; --d) ends[d] = ends[d - 1];
         ends[0] = head;
-        // entries of the stages D and more back have landed (every commit group but the D most recent); they are resolved
-        // once there are enough of them to keep the warp's lanes busy, not every stage
         if ((int)(ends[D] - tail) >= batch) {
             cp_async_wait<D>();
             __syncwarp();
@@ -1407,7 +1420,7 @@ static cudaError_t launch_call_forward(dim3 grid, const uint4* c, int T, int64_t
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < AS_MAX_DEVICES) configured[dev] = true;
     }
-    call_forward_kernel<K, STAGES, D><<<grid, AS_CTA_THREADS, smem, st>>>(c, T, P, p0, p1, chunk, ref, tv, cut, pend_cap, calls, cap, n);
+    call_forward_kernel<K, STAGES, D><<<grid, AS_TILE_SLOTS + 32 * STAGES, smem, st>>>(c, T, P, p0, p1, chunk, ref, tv, cut, pend_cap, calls, cap, n);
     return cudaGetLastError();
 }
 
@@ -1437,7 +1450,7 @@ cudaError_t as_launch_call_sweep(int variant, const uint32_t* d_counts, int T, i
         case 11: return launch_call_staged<3, 2>(grid, AS_SWEEP_ARGS, st);
         case 14: return launch_call_staged<4, 2, true>(grid, AS_SWEEP_ARGS, st);
         case 15: return launch_call_staged<3, 2, true>(grid, AS_SWEEP_ARGS, st);
-        default: if (n_c != 1) break; return launch_call_forward<6, 2, 2>(grid, AS_FWD_ARGS, st);
+        default: if (n_c != 1) break; return launch_call_forward<4, 3, 2>(grid, AS_FWD_ARGS, st);
     }
     // a sweep of several tables on a staged variant: the in-stage sweep kernel
     return launch_call_staged<3, 2, true>(grid, AS_SWEEP_ARGS, st);

@@ -15,7 +15,7 @@
  * thread scans its own rows, the two states are merged exactly after the sample loop (as_noise.cuh pair_merge).
  * 0: every twin group goes to noise_pair_kernel / noise_twin_kernel. */
 #define AS_INTILE_TWINS 1
-#define AS_DEFAULT_CALL_KERNEL 13 /* forward-first (call_forward_kernel): forward plane streamed, 6 samples per stage, 2 stages, reverse words fetched for forward candidates; 15 = the both-strand staged caller it replaced */
+#define AS_DEFAULT_CALL_KERNEL 13 /* forward-first (call_forward_kernel): forward plane streamed, 4 samples per stage, 3 stages; four scan warps and one control warp per stage, which extracts the forward candidates, fetches their reverse words and refills its stage; 15 = the both-strand staged caller it replaced */
 #define AS_DEFAULT_NOISE_KERNEL 1 /* TMA-staged, 4 samples per stage, 3 stages */
 #define AS_DEFERRED_CALL_KERNEL 20 /* scan -> resolve -> series (as_call_deferred.cu); what a sweep runs by default */
 
@@ -54,8 +54,8 @@ cudaError_t as_launch_patch_wide(const as_wide_record* d_wide, int64_t m, uint32
                                  int n_samples, cudaStream_t st);
 cudaError_t as_launch_thr_view(const float* d_thr, float* d_view, int64_t n, cudaStream_t st);
 int as_call_chunk(int T, int64_t n_slots);
-// fwd_pending_cap: usable depth of call_forward_kernel's per-warp pending ring, 1..AS_FWD_PENDING (else the whole ring)
-#define AS_FWD_PENDING 32
+// fwd_pending_cap: usable depth of call_forward_kernel's per-CTA pending ring, 1..AS_FWD_PENDING (else the whole ring)
+#define AS_FWD_PENDING 128
 cudaError_t as_launch_call(int variant, const uint32_t* d_counts, int T, int64_t P, int64_t p0, int64_t p1,
                            const uint8_t* d_ref, const float* d_thr_view, uint32_t cut, as_call* d_calls, int64_t cap,
                            unsigned long long* d_n_calls, int fwd_pending_cap, cudaStream_t st);

@@ -67,7 +67,8 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // Ring geometry.  A stage holds K samples x STRANDS strands x AS_TILE_SLOTS uint4 words; STRANDS = 1 streams the
-// forward strand only (call_forward_kernel, which fetches reverse-strand words on its own).
+// forward strand only (call_forward_kernel, which fetches reverse-strand words on its own and refills stages from its
+// control warp with fill() rather than running produce()).
 template <int K, int STAGES, int STRANDS = 2>
 struct StageRing {
     static_assert(STRANDS == 1 || STRANDS == 2, "one or both strands per sample");
@@ -92,23 +93,28 @@ struct StageRing {
     }
     __device__ __forceinline__ const uint4* stage(int s) const { return data + (size_t)s * kStageWords; }
 
-    // Producer: one thread.  Streams samples [t0, t1) of the tile whose first word is `src` (= counts + p0),
-    // n_slots valid slots in the tile, sample stride `sstride` words, strand stride `P` words.
+    // One thread: bulk-copy iteration `it` (samples t0 + it*K on, at most up to t1) of the tile whose first word is `src`
+    // (= counts + p0) into its stage, which must be free; sample stride `sstride` words, strand stride `P` words,
+    // row_bytes = 16 x the valid slots of the tile.
+    __device__ __forceinline__ void fill(int it, const uint4* __restrict__ src, int64_t sstride, int64_t P, int t0, int t1,
+                                         uint32_t row_bytes) {
+        const int s = it % STAGES, t = t0 + it * K;
+        const int k = min(K, t1 - t);
+        mbar_expect_tx(&full[s], row_bytes * (uint32_t)STRANDS * (uint32_t)k);
+        uint4* dst = data + (size_t)s * kStageWords;
+        for (int j = 0; j < k; ++j) {
+            const uint4* g = src + (int64_t)(t + j) * sstride;
+            bulk_g2s(dst + (j * STRANDS + 0) * AS_TILE_SLOTS, g, row_bytes, &full[s]);
+            if (STRANDS == 2) bulk_g2s(dst + (j * STRANDS + 1) * AS_TILE_SLOTS, g + P, row_bytes, &full[s]);
+        }
+    }
+    // Producer: one thread.  Streams samples [t0, t1) of the tile, n_slots valid slots in the tile.
     __device__ __forceinline__ void produce(const uint4* __restrict__ src, int64_t sstride, int64_t P, int t0, int t1,
                                             int n_slots) {
         const uint32_t row_bytes = (uint32_t)n_slots * 16u;
-        int it = 0;
-        for (int t = t0; t < t1; t += K, ++it) {
-            const int s = it % STAGES;
-            if (it >= STAGES) mbar_wait(&empty[s], ((it / STAGES) - 1) & 1);
-            const int k = min(K, t1 - t);
-            mbar_expect_tx(&full[s], row_bytes * (uint32_t)STRANDS * (uint32_t)k);
-            uint4* dst = data + (size_t)s * kStageWords;
-            for (int j = 0; j < k; ++j) {
-                const uint4* g = src + (int64_t)(t + j) * sstride;
-                bulk_g2s(dst + (j * STRANDS + 0) * AS_TILE_SLOTS, g, row_bytes, &full[s]);
-                if (STRANDS == 2) bulk_g2s(dst + (j * STRANDS + 1) * AS_TILE_SLOTS, g + P, row_bytes, &full[s]);
-            }
+        for (int it = 0; t0 + it * K < t1; ++it) {
+            if (it >= STAGES) mbar_wait(&empty[it % STAGES], ((it / STAGES) - 1) & 1);
+            fill(it, src, sstride, P, t0, t1, row_bytes);
         }
     }
     // Consumer side: wait for iteration `it` to land / hand its stage back (one arrival per warp).

@@ -112,8 +112,8 @@ int as_set_noise_kernel(as_ctx* ctx, int variant);
 int as_set_host_tile_slots(as_ctx* ctx, int64_t slots);
 /* Generic form of the setters above plus "deferred_capacity" (entries of the deferred caller's candidate list; 0 =
  * automatic; the kernels resolve what does not fit on the spot, so results never depend on it -- tests use tiny values)
- * and "forward_pending_cap" (usable entries of call kernel 13's per-warp ring of pending reverse-strand fetches, 0 =
- * automatic, at most 32; a full ring is drained on the spot, so results never depend on it either). */
+ * and "forward_pending_cap" (usable entries of call kernel 13's per-control-warp ring of pending reverse-strand fetches,
+ * 0 = automatic, at most 128; a full ring is drained on the spot, so results never depend on it either). */
 int as_set_option(as_ctx* ctx, const char* name, int64_t value);
 /* Number of kernel launches this context has enqueued so far (bench.py's gpu_launches). */
 int64_t as_kernel_launches(const as_ctx* ctx);
